@@ -17,8 +17,9 @@ For every small scene it writes under tests/golden/:
     <scene>.render1t.npz    single-threaded reference render in exact doubles + the LCG state it started
                             from -> BIT-EXACT pin of the C restatement's whole path loop
     kat.json                unit known answers (LCG stream, reflect/refract/Schlick, tone map)
-The big scenes (raining: 2.2 M quads, millions_lights: 3.1 M spheres) are NOT committed; the
-GPU tests regenerate them on the box with the same bridge binary, which travels with the repo.
+The big scenes (raining: 2.2 M quads, millions_lights: 3.1 M spheres) are NOT committed; where the
+bridge binary is built, the live-reference tests regenerate them with it.  tests/golden/make_big_golden.py
+stores a digest and a ray sample of them for the tests that run without it.
 """
 import gzip
 import json

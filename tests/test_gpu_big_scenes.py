@@ -2,8 +2,9 @@
 2.2 M light quads + 25 k spheres; C5 millions_of_spheres_with_lights: 3.1 M spheres) and on the
 host C++ layer's render call.  The scenes are built by the repo's own host code
 (host/b200rt_scenes, pinned byte-for-byte against reference dumps in test_host_api_cpu.py); the
-expected hits and reference renders come from the compiled reference (oracle/_ref/ref_bridge),
-run live on this box because the fixtures would be hundreds of MB."""
+full comparison runs the compiled reference (oracle/_ref/ref_bridge) live because its fixtures
+would be hundreds of MB; a stored sample of rays with their Scene::hit_by answers
+(tests/golden/<scene>.rays.gz / .hits_brute.gz) checks the ray cast without it."""
 import json
 import os
 import subprocess
@@ -84,6 +85,24 @@ def test_big_scene_raycast_and_render_vs_reference(scenes_bin, ref_bridge, name,
           f"rays/path {st['rays'] / st['paths']:.3f}; {st['paths'] / st['kernel_ms'] / 1e3:.0f} Mpaths/s at {w}x{h}")
     assert got <= 1.25 * floor
     assert lerr <= 0.03 + 3 * abs(lum(tA) - lum(tB)) / lum(tA)
+
+
+@pytest.mark.parametrize("name", ["raining", "millions_lights"])
+def test_big_scene_raycast_matches_stored_scene_hit_by(scenes_bin, golden, name, tmp_path):
+    """Camera rays and one bounce from each camera hit (tests/golden/make_big_golden.py) against Scene::hit_by
+    as the oracle's C restatement answers it: primitive index and t bit-exact on every ray."""
+    import cpp_raytracer_b200 as rt
+    from cpp_raytracer_b200 import scene_io
+    scene_path = str(tmp_path / "s.scene")
+    subprocess.run([scenes_bin, name, "dump", scene_path], check=True, capture_output=True)
+    scene = scene_io.load_scene(scene_path)
+    rays, tmin, tmax = golden.rays(name)
+    want_p, want_t = golden.hits(name, brute=True)
+    with rt.DeviceSceneHandle(scene) as dev:
+        p, t = dev.raycast(rays, tmin, tmax)
+    bad = np.nonzero((p != want_p) | (t != want_t))[0]
+    assert len(bad) == 0, (f"{name}: {len(bad)} of {len(rays)} rays differ from Scene::hit_by; first: ray {bad[0]} "
+                           f"got ({p[bad[0]]}, {t[bad[0]]!r}) want ({want_p[bad[0]]}, {want_t[bad[0]]!r})")
 
 
 def test_host_cpp_render_call_writes_reference_format_ppm(scenes_bin, golden, tmp_path):

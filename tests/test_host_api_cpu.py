@@ -7,6 +7,8 @@ SeedSeqGenerator, rand_int, RGB::random's draw order, Box -> 6 faces in construc
 material sharing by pointer, canonical primitive order, and Camera::init through
 b200rt_camera_init."""
 import gzip
+import hashlib
+import json
 import os
 import subprocess
 
@@ -55,6 +57,18 @@ def test_host_big_scene_builders_match_reference_live(scenes_bin, ref_bridge, na
     subprocess.run([scenes_bin, name, "dump", mine], check=True, capture_output=True)
     subprocess.run([ref_bridge, name, "dump", ref], check=True, capture_output=True)
     assert subprocess.run(["cmp", "-s", mine, ref]).returncode == 0
+
+
+@pytest.mark.parametrize("name", ["raining", "millions_lights"])
+def test_host_big_scene_builders_match_recorded_digest(scenes_bin, name, tmp_path):
+    """The same two scenes against the byte length and SHA-256 of their dumps recorded in
+    tests/golden/big_scenes.json (tests/golden/make_big_golden.py), so a change to the scene code or
+    the flattening shows up without the reference binary."""
+    want = json.load(open(os.path.join(GOLDEN, "big_scenes.json")))[name]
+    out = str(tmp_path / f"{name}.scene")
+    subprocess.run([scenes_bin, name, "dump", out], check=True, capture_output=True)
+    data = open(out, "rb").read()
+    assert len(data) == want["bytes"] and hashlib.sha256(data).hexdigest() == want["sha256"], name
 
 
 def test_reference_style_program_compiles_unchanged(tmp_path):
