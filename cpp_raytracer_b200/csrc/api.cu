@@ -1,10 +1,11 @@
 // api.cu -- implementation of the C ABI declared in include/b200rt.h.
 //
-// Host side of the drop-in boundary: validates and flattens the scene description, computes
-// primitive bounds exactly as the reference's constructors do (sphere.h:112-123,
-// parallelogram.h:269-295), builds the 4-wide BVH (bvh_builder.cpp), lays everything out in
-// leaf order as SoA device arrays and launches the kernels.  There is no CPU compute path:
-// every entry point that produces hits or pixels fails with B200RT_ENODEVICE without a GPU.
+// Host side of the drop-in boundary: validates the scene description's structure, uploads the
+// caller's arrays as they are, has one of the two builders decide the 4-wide BVH and its leaf order
+// (bvh_builder.cpp on the host, with primitive bounds exactly as the reference's constructors
+// compute them, sphere.h:112-123, parallelogram.h:281-295; or lbvh.cu on the device), has
+// scene_layout.cu lay the primitives out in that order and launches the kernels.  There is no CPU
+// compute path: every entry point that produces hits or pixels fails with B200RT_ENODEVICE without a GPU.
 #include <algorithm>
 #include <chrono>
 #include <cmath>
@@ -26,9 +27,12 @@ using namespace b200rt;
 
 namespace b200rt {
 cudaError_t build_lbvh_device(const B200rtSphere *d_sph, uint32_t n_sph, const B200rtQuad *d_quads, uint32_t n_quad,
-                              uint32_t n_materials, double2 *out_sph, uint2 *out_sph_meta, double2 *out_quads, uint2 *out_quad_meta,
-                              float4 **nodes_out, uint32_t *n_nodes_out, uint32_t *depth_out, int *bad_index_out);
-cudaError_t convert_materials_device(const B200rtMaterial *d_raw, uint32_t n, DeviceMaterial *d_out, int *bad_kind_out);
+                              uint32_t *sphere_order, uint32_t *quad_order, float4 **nodes_out, uint32_t *n_nodes_out,
+                              uint32_t *depth_out);
+cudaError_t assemble_scene_device(const B200rtSphere *sph, const uint32_t *sphere_order, uint32_t n_sph, const B200rtQuad *quads,
+                                  const uint32_t *quad_order, uint32_t n_quad, const B200rtMaterial *mats, uint32_t n_mat,
+                                  double2 *out_sph, uint2 *out_sph_meta, double2 *out_quads, uint2 *out_quad_meta,
+                                  DeviceMaterial *out_mats, int bad_out[2]);
 }
 
 namespace {
@@ -186,7 +190,9 @@ int validate_desc(const B200rtSceneDesc *d, bool check_prims = true) {
         return fail(B200RT_EINVAL, "scene description has a count without an array");
     const uint64_t n_prims = d->n_spheres + d->n_quads;
     if (n_prims > 0x7FFFFFFFull) return fail(B200RT_EINVAL, "too many primitives");
-    if (!check_prims) return B200RT_OK;   // the GPU builder checks material kinds and per-primitive indices on the device
+    // scene creation checks material kinds and per-primitive indices on the device (scene_layout.cu); the host loops
+    // below serve b200rt_selftest_bvh, which runs without one
+    if (!check_prims) return B200RT_OK;
     for (uint64_t i = 0; i < d->n_materials; ++i)
         if (d->materials[i].kind > B200RT_MAT_LIGHT)
             return fail(B200RT_EINVAL, "unknown material kind " + std::to_string(d->materials[i].kind) +
@@ -230,17 +236,6 @@ BuildParams build_params(const B200rtBuildOpts *o) {
         if (o->build_threads > 0) p.threads = o->build_threads;
     }
     return p;
-}
-
-template <typename T>
-int upload(SceneImpl *s, int slot, const std::vector<T> &host, const T **dev, uint64_t &bytes) {
-    *dev = nullptr;
-    if (host.empty()) return B200RT_OK;
-    CUDA_TRY(scene_alloc(s, slot, host.size() * sizeof(T)));   // owned by the scene from here on (free_scene releases it on any later failure)
-    CUDA_TRY(staged_upload(s->allocs[slot], host.data(), host.size() * sizeof(T), 0));
-    *dev = static_cast<const T *>(s->allocs[slot]);
-    bytes += host.size() * sizeof(T);
-    return B200RT_OK;
 }
 
 void free_scene(SceneImpl *s) {
@@ -386,176 +381,23 @@ int render_on_device(SceneImpl *s, const B200rtCamera *cam, const B200rtRenderOp
     return B200RT_OK;
 }
 
-std::vector<DeviceMaterial> device_materials(const B200rtSceneDesc *desc) {
-    std::vector<DeviceMaterial> mats(desc->n_materials);
-    for (uint64_t i = 0; i < desc->n_materials; ++i) {
-        const B200rtMaterial &m = desc->materials[i];
-        DeviceMaterial dm{};
-        const double k = m.kind == B200RT_MAT_LIGHT ? m.param : 1.0;   // emit() = intensity * colour (material.h:261-263)
-        dm.r = (float)(k * m.rgb[0]); dm.g = (float)(k * m.rgb[1]); dm.b = (float)(k * m.rgb[2]);
-        dm.kind = m.kind;
-        dm.param = m.kind == B200RT_MAT_METAL ? std::fmin(m.param, 1.0) : m.param;   // Metal ctor clamps fuzz (material.h:150-151)
-        mats[i] = dm;
-    }
-    return mats;
-}
-
-// Host construction: parallel binned-SAH build + 4-wide collapse (bvh_builder.cpp), leaf-ordered SoA
-// arrays assembled on the host, then uploaded.
-int scene_build_host(const B200rtSceneDesc *desc, const B200rtBuildOpts *opts, SceneImpl *s) {
-    const double t0 = now_ms();
-    std::vector<Box3> boxes;
-    compute_boxes(desc, boxes, host_threads(opts));
-    BuiltBVH bvh;
-    const char *err = nullptr;
-    if (!build_bvh4(boxes, desc->n_spheres, desc->n_quads, build_params(opts), bvh, &err))
-        return fail(B200RT_EINVAL, std::string("BVH build failed: ") + (err ? err : "?"));
-    const int need_stack = (int)(3 * bvh.depth);
-    if (need_stack > 128) return fail(B200RT_EINTERNAL, "BVH deeper than the largest traversal stack");
-
-    // ---- leaf-ordered SoA arrays ----
-    std::vector<double2> sph(desc->n_spheres * 2);
-    std::vector<uint2> sph_meta(desc->n_spheres);
-    parallel_ranges(desc->n_spheres, host_threads(opts), [&](uint64_t lo, uint64_t hi) {
-        for (uint64_t i = lo; i < hi; ++i) {
-            const B200rtSphere &s = desc->spheres[bvh.sphere_order[i]];
-            sph[2 * i] = make_double2(s.c[0], s.c[1]);
-            sph[2 * i + 1] = make_double2(s.c[2], s.r);
-            sph_meta[i] = make_uint2(s.prim, s.mat);
-        }
-    });
-    std::vector<double2> quads(desc->n_quads * 8);
-    std::vector<uint2> quad_meta(desc->n_quads);
-    parallel_ranges(desc->n_quads, host_threads(opts), [&](uint64_t lo, uint64_t hi) {
-      for (uint64_t i = lo; i < hi; ++i) {
-        const B200rtQuad &q = desc->quads[bvh.quad_order[i]];
-        const V3 s1 = v3(q.s1), s2 = v3(q.s2);
-        const V3 n = crossv(s1, s2);                 // parallelogram.h:275-279
-        const V3 un = unitv(n);
-        const V3 w = divv(n, mag2(n));
-        const double f[16] = {un.x, un.y, un.z, q.v[0], q.v[1], q.v[2], w.x, w.y, w.z,
-                              s1.x, s1.y, s1.z, s2.x, s2.y, s2.z, 0.0};
-        for (int k = 0; k < 8; ++k) quads[8 * i + k] = make_double2(f[2 * k], f[2 * k + 1]);
-        quad_meta[i] = make_uint2(q.prim, q.mat);
-      }
-    });
-    const std::vector<DeviceMaterial> mats = device_materials(desc);
-    const double t1 = now_ms();
-
-    // ---- upload ----
-    uint64_t bytes = 0;
-    int rc = B200RT_OK;
-    const float4 *d_nodes = nullptr;
-    {
-        std::vector<float4> flat(bvh.nodes.size() * 8);
-        std::memcpy(flat.data(), bvh.nodes.data(), bvh.nodes.size() * sizeof(Node4));
-        rc = upload(s, 0, flat, &d_nodes, bytes);
-    }
-    if (!rc) rc = upload(s, 1, sph, &s->d.spheres, bytes);
-    if (!rc) rc = upload(s, 2, sph_meta, &s->d.sphere_meta, bytes);
-    if (!rc) rc = upload(s, 3, quads, &s->d.quads, bytes);
-    if (!rc) rc = upload(s, 4, quad_meta, &s->d.quad_meta, bytes);
-    if (!rc) rc = upload(s, 5, mats, &s->d.materials, bytes);
-    if (!rc && cudaStreamSynchronize(0) != cudaSuccess) rc = fail(B200RT_ECUDA, "scene upload failed");
-    s->d.nodes = d_nodes;
-    if (rc) return rc;
-    if (reinterpret_cast<uintptr_t>(d_nodes) & 127)   // trav_node_step forms plane addresses with OR / XOR on the low bits
+// Points s->d at the arrays in s->allocs, takes `info`, sizes the traversal stack from the tree depth and creates the
+// per-scene launch state (counters, events, the bounds-check table of the debug build); `s->device` is current.
+int finish_scene(SceneImpl *s, const B200rtSceneInfo &info) {
+    s->d.nodes = static_cast<const float4 *>(s->allocs[0]);
+    s->d.spheres = static_cast<const double2 *>(s->allocs[1]);
+    s->d.sphere_meta = static_cast<const uint2 *>(s->allocs[2]);
+    s->d.quads = static_cast<const double2 *>(s->allocs[3]);
+    s->d.quad_meta = static_cast<const uint2 *>(s->allocs[4]);
+    s->d.materials = static_cast<const DeviceMaterial *>(s->allocs[5]);
+    if (reinterpret_cast<uintptr_t>(s->d.nodes) & 127)   // trav_node_step forms plane addresses with OR / XOR on the low bits
         return fail(B200RT_ECUDA, "node array is not 128-byte aligned");
-    const double t2 = now_ms();
+    s->info = info;
+    const int need_stack = (int)(3 * info.tree_depth);
     s->stack = need_stack <= 32 ? 32 : (need_stack <= 64 ? 64 : 128);
-    s->info.n_nodes = bvh.nodes.size();
-    s->info.device_bytes = bytes;
-    s->info.tree_depth = bvh.depth;
-    s->info.build_ms = t1 - t0;
-    s->info.upload_ms = t2 - t1;
-    return B200RT_OK;
-}
-
-// GPU construction (lbvh.cu): the caller's flat arrays go to the device as they are; bounds, Morton
-// order, tree, 4-wide collapse and the leaf-ordered SoA arrays are all produced there.
-// Returns B200RT_OK, or an error; `too_deep` is set when the tree needs a stack beyond 128 entries
-// (the caller then falls back to the host SAH builder).
-int scene_build_gpu(const B200rtSceneDesc *desc, SceneImpl *s, bool *too_deep) {
-    *too_deep = false;
-    const double t0 = now_ms();
-    const uint32_t n_sph = (uint32_t)desc->n_spheres, n_quad = (uint32_t)desc->n_quads;
-    if (n_sph > kLeafIndexMask || n_quad > kLeafIndexMask || (uint64_t)n_sph + n_quad > (1u << 29))
-        return fail(B200RT_EINVAL, "too many primitives for the leaf encoding (2^26 per type)");
-    if (desc->n_materials > 0xFFFFFFFFull) return fail(B200RT_EINVAL, "too many materials");
-    uint64_t bytes = 0;
-    // The caller's structs go up as they are (pinned staging, pipelined); the scene's own arrays are allocated
-    // straight into s->allocs so that free_scene releases them on every failure path below.
-    B200rtSphere *raw_sph = nullptr;
-    B200rtQuad *raw_quad = nullptr;
-    struct RawGuard {
-        B200rtSphere *&a; B200rtQuad *&b;
-        ~RawGuard() { dev_free(a); dev_free(b); }
-    } raw_guard{raw_sph, raw_quad};
-    CUDA_TRY(dev_alloc_async(&raw_sph, (size_t)n_sph * sizeof(B200rtSphere), 0));
-    CUDA_TRY(dev_alloc_async(&raw_quad, (size_t)n_quad * sizeof(B200rtQuad), 0));
-    const size_t sizes[6] = {0, (size_t)n_sph * 2 * sizeof(double2), (size_t)n_sph * sizeof(uint2),
-                             (size_t)n_quad * 8 * sizeof(double2), (size_t)n_quad * sizeof(uint2), 0};
-    for (int i = 1; i <= 4; ++i) CUDA_TRY(scene_alloc(s, i, sizes[i]));
-    CUDA_TRY(staged_upload(raw_sph, desc->spheres, (size_t)n_sph * sizeof(B200rtSphere), 0));
-    CUDA_TRY(staged_upload(raw_quad, desc->quads, (size_t)n_quad * sizeof(B200rtQuad), 0));
-    double2 *d_sph = static_cast<double2 *>(s->allocs[1]), *d_quads = static_cast<double2 *>(s->allocs[3]);
-    uint2 *d_sph_meta = static_cast<uint2 *>(s->allocs[2]), *d_quad_meta = static_cast<uint2 *>(s->allocs[4]);
-    const bool trace = std::getenv("B200RT_TRACE") != nullptr;
-    if (trace) cudaStreamSynchronize(0);
-    const double t_up = now_ms();
-    float4 *d_nodes = nullptr;
-    uint32_t n_nodes = 0, depth = 0;
-    int bad_index = 0;
-    const cudaError_t e = build_lbvh_device(raw_sph, n_sph, raw_quad, n_quad, (uint32_t)desc->n_materials, d_sph, d_sph_meta, d_quads,
-                                            d_quad_meta, &d_nodes, &n_nodes, &depth, &bad_index);
-    if (e != cudaSuccess) { cudaGetLastError(); return fail(B200RT_ECUDA, std::string("GPU BVH build: ") + cudaGetErrorString(e)); }
-    if (trace) std::fprintf(stderr, "scene_build_gpu: upload %.2f ms, lbvh %.2f ms\n", t_up - t0, now_ms() - t_up);
-    if (bad_index) { dev_free(d_nodes); return fail(B200RT_EINVAL, "a sphere or quad has a material or primitive index out of range"); }
-    if (3 * depth > 128) { dev_free(d_nodes); *too_deep = true; return B200RT_OK; }
-    if (s->peer_visible) {
-        // the builder sized the node array for the worst case (n - 1 nodes) in pool memory; a multi-device scene
-        // keeps an exact-size copy in a peer-visible buffer instead (a device-to-device copy at HBM speed)
-        const cudaError_t e2 = scene_alloc(s, 0, (size_t)n_nodes * sizeof(Node4));
-        if (e2 == cudaSuccess) cudaMemcpyAsync(s->allocs[0], d_nodes, (size_t)n_nodes * sizeof(Node4), cudaMemcpyDeviceToDevice, 0);
-        dev_free(d_nodes);
-        if (e2 != cudaSuccess) { cudaGetLastError(); return fail(B200RT_ENOMEM, "node array copy"); }
-        d_nodes = static_cast<float4 *>(s->allocs[0]);
-    } else {
-        s->allocs[0] = d_nodes;
-        s->alloc_bytes[0] = (size_t)n_nodes * sizeof(Node4);
-    }
-    {   // materials: the caller's records go up as they are and are converted (and their kinds checked) on the device
-        B200rtMaterial *raw_mat = nullptr;
-        CUDA_TRY(dev_alloc_async(&raw_mat, (size_t)desc->n_materials * sizeof(B200rtMaterial), 0));
-        struct MatGuard { B200rtMaterial *&p; ~MatGuard() { dev_free(p); } } mat_guard{raw_mat};
-        CUDA_TRY(scene_alloc(s, 5, (size_t)desc->n_materials * sizeof(DeviceMaterial)));
-        CUDA_TRY(staged_upload(raw_mat, desc->materials, (size_t)desc->n_materials * sizeof(B200rtMaterial), 0));
-        int bad_kind = 0;
-        CUDA_TRY(convert_materials_device(raw_mat, (uint32_t)desc->n_materials, static_cast<DeviceMaterial *>(s->allocs[5]), &bad_kind));
-        if (bad_kind) return fail(B200RT_EINVAL, "unknown material kind (closed set: Lambertian, Metal, Dielectric, DiffuseLight)");
-        s->d.materials = static_cast<const DeviceMaterial *>(s->allocs[5]);
-        bytes += (uint64_t)desc->n_materials * sizeof(DeviceMaterial);
-    }
-    if (reinterpret_cast<uintptr_t>(d_nodes) & 127)   // trav_node_step forms plane addresses with OR / XOR on the low bits
-        return fail(B200RT_ECUDA, "node array is not 128-byte aligned");
-    s->d.nodes = d_nodes;
-    s->d.spheres = d_sph; s->d.sphere_meta = d_sph_meta;
-    s->d.quads = d_quads; s->d.quad_meta = d_quad_meta;
-    CUDA_TRY(cudaStreamSynchronize(0));
-    bytes += (uint64_t)n_nodes * sizeof(Node4) + (uint64_t)n_sph * (2 * sizeof(double2) + sizeof(uint2)) +
-             (uint64_t)n_quad * (8 * sizeof(double2) + sizeof(uint2));
-    const int need_stack = (int)(3 * depth);
-    s->stack = need_stack <= 32 ? 32 : (need_stack <= 64 ? 64 : 128);
-    s->info.n_nodes = n_nodes;
-    s->info.device_bytes = bytes;
-    s->info.tree_depth = depth;
-    s->info.build_ms = now_ms() - t0;
-    s->info.upload_ms = 0;
-    return B200RT_OK;
-}
-
-// Per-scene launch state (counters, events, the bounds-check table of the debug build); `s->device` is current.
-int finish_scene_setup(SceneImpl *s) {
+    s->info.stack_entries = (uint32_t)s->stack;
+    s->info.device_bytes = 0;
+    for (size_t b : s->alloc_bytes) s->info.device_bytes += b;
     cudaError_t e = dev_alloc(&s->d_counters, 4 * sizeof(unsigned long long));
     if (e == cudaSuccess) e = cudaDeviceGetAttribute(&s->sm_count, cudaDevAttrMultiProcessorCount, s->device);
     if (e == cudaSuccess) e = cudaEventCreate(&s->ev0);
@@ -577,7 +419,102 @@ int finish_scene_setup(SceneImpl *s) {
     return B200RT_OK;
 }
 
-// Builds the acceleration structure for `desc` and makes the scene resident on device `dev`.
+// Makes the scene resident on s->device.  The caller's arrays go up as they are; a builder decides the tree and the
+// leaf order -- the GPU LBVH (lbvh.cu) when `gpu_build`, the host SAH builder (bvh_builder.cpp) otherwise or when
+// the LBVH is too deep for the largest traversal stack -- and scene_layout.cu lays the primitives out in that order
+// and checks them, whichever builder ran.  build_ms is the host builder's time when it built the tree, else all of
+// it; upload_ms is the rest.
+int scene_build(const B200rtSceneDesc *desc, const B200rtBuildOpts *opts, bool gpu_build, SceneImpl *s) {
+    const double t0 = now_ms();
+    if (desc->n_spheres > kLeafIndexMask || desc->n_quads > kLeafIndexMask)
+        return fail(B200RT_EINVAL, "too many primitives for the leaf encoding (2^26 per type)");
+    if (desc->n_materials > 0xFFFFFFFFull) return fail(B200RT_EINVAL, "too many materials");
+    const uint32_t n_sph = (uint32_t)desc->n_spheres, n_quad = (uint32_t)desc->n_quads, n_mat = (uint32_t)desc->n_materials;
+    // the caller's records (pinned staging, pipelined) and the leaf order are scratch; the scene's own arrays are
+    // allocated straight into s->allocs so that free_scene releases them on every failure path below
+    struct Raw {
+        B200rtSphere *sph = nullptr;
+        B200rtQuad *quad = nullptr;
+        B200rtMaterial *mat = nullptr;
+        uint32_t *order = nullptr;   // sphere_order[n_sph], then quad_order[n_quad]
+        ~Raw() { dev_free(sph); dev_free(quad); dev_free(mat); dev_free(order); }
+    } raw;
+    CUDA_TRY(dev_alloc_async(&raw.sph, (size_t)n_sph * sizeof(B200rtSphere), 0));
+    CUDA_TRY(dev_alloc_async(&raw.quad, (size_t)n_quad * sizeof(B200rtQuad), 0));
+    // the scene's arrays are sized by the description alone: taken before the tree build's temporaries come and go,
+    // they find the pool as the previous scene left it instead of fragmented by the build
+    const size_t bytes[6] = {0, (size_t)n_sph * 2 * sizeof(double2), (size_t)n_sph * sizeof(uint2), (size_t)n_quad * 8 * sizeof(double2),
+                             (size_t)n_quad * sizeof(uint2), (size_t)n_mat * sizeof(DeviceMaterial)};
+    for (int i = 1; i < 6; ++i)
+        if (bytes[i]) CUDA_TRY(scene_alloc(s, i, bytes[i]));
+    CUDA_TRY(dev_alloc_async(&raw.mat, (size_t)n_mat * sizeof(B200rtMaterial), 0));
+    CUDA_TRY(dev_alloc_async(&raw.order, ((size_t)n_sph + n_quad) * sizeof(uint32_t), 0));
+    CUDA_TRY(staged_upload(raw.sph, desc->spheres, (size_t)n_sph * sizeof(B200rtSphere), 0));
+    CUDA_TRY(staged_upload(raw.quad, desc->quads, (size_t)n_quad * sizeof(B200rtQuad), 0));
+    CUDA_TRY(staged_upload(raw.mat, desc->materials, (size_t)n_mat * sizeof(B200rtMaterial), 0));
+    uint32_t *sphere_order = raw.order, *quad_order = raw.order + n_sph;
+    uint32_t n_nodes = 0, depth = 0;
+    bool have_tree = false;
+    if (gpu_build) {
+        const bool trace = std::getenv("B200RT_TRACE") != nullptr;
+        if (trace) cudaStreamSynchronize(0);
+        const double t_up = now_ms();
+        float4 *d_nodes = nullptr;
+        const cudaError_t e = build_lbvh_device(raw.sph, n_sph, raw.quad, n_quad, sphere_order, quad_order, &d_nodes, &n_nodes, &depth);
+        if (e != cudaSuccess) { cudaGetLastError(); return fail(B200RT_ECUDA, std::string("GPU BVH build: ") + cudaGetErrorString(e)); }
+        if (trace) std::fprintf(stderr, "scene_build: upload %.2f ms, lbvh %.2f ms, depth %u\n", t_up - t0, now_ms() - t_up, depth);
+        have_tree = 3 * depth <= 128;
+        if (!have_tree) {
+            dev_free(d_nodes);   // pathological depth: the depth-capped host builder below takes over
+        } else if (s->peer_visible) {
+            // the builder sized the node array for the worst case (n - 1 nodes) in pool memory; a multi-device scene
+            // keeps an exact-size copy in a peer-visible buffer instead (a device-to-device copy at HBM speed)
+            const cudaError_t e2 = scene_alloc(s, 0, (size_t)n_nodes * sizeof(Node4));
+            if (e2 == cudaSuccess) cudaMemcpyAsync(s->allocs[0], d_nodes, (size_t)n_nodes * sizeof(Node4), cudaMemcpyDeviceToDevice, 0);
+            dev_free(d_nodes);
+            if (e2 != cudaSuccess) { cudaGetLastError(); return fail(B200RT_ENOMEM, "node array copy"); }
+        } else {
+            s->allocs[0] = d_nodes;
+            s->alloc_bytes[0] = (size_t)n_nodes * sizeof(Node4);
+        }
+    }
+    double host_ms = -1;
+    if (!have_tree) {   // parallel binned SAH + 4-wide collapse on the host; the nodes and the leaf order go up
+        const double t1 = now_ms();
+        std::vector<Box3> boxes;
+        compute_boxes(desc, boxes, host_threads(opts));
+        BuiltBVH bvh;
+        const char *err = nullptr;
+        if (!build_bvh4(boxes, desc->n_spheres, desc->n_quads, build_params(opts), bvh, &err))
+            return fail(B200RT_EINVAL, std::string("BVH build failed: ") + (err ? err : "?"));
+        host_ms = now_ms() - t1;
+        n_nodes = (uint32_t)bvh.nodes.size();
+        depth = bvh.depth;
+        if (3 * depth > 128) return fail(B200RT_EINTERNAL, "BVH deeper than the largest traversal stack");
+        CUDA_TRY(scene_alloc(s, 0, (size_t)n_nodes * sizeof(Node4)));
+        CUDA_TRY(staged_upload(s->allocs[0], bvh.nodes.data(), (size_t)n_nodes * sizeof(Node4), 0));
+        CUDA_TRY(staged_upload(sphere_order, bvh.sphere_order.data(), (size_t)n_sph * sizeof(uint32_t), 0));
+        CUDA_TRY(staged_upload(quad_order, bvh.quad_order.data(), (size_t)n_quad * sizeof(uint32_t), 0));
+    }
+    int bad[2] = {0, 0};
+    CUDA_TRY(assemble_scene_device(raw.sph, sphere_order, n_sph, raw.quad, quad_order, n_quad, raw.mat, n_mat,
+                                   static_cast<double2 *>(s->allocs[1]), static_cast<uint2 *>(s->allocs[2]),
+                                   static_cast<double2 *>(s->allocs[3]), static_cast<uint2 *>(s->allocs[4]),
+                                   static_cast<DeviceMaterial *>(s->allocs[5]), bad));
+    if (bad[1]) return fail(B200RT_EINVAL, "unknown material kind (closed set: Lambertian, Metal, Dielectric, DiffuseLight)");
+    if (bad[0]) return fail(B200RT_EINVAL, "a sphere or quad has a material or primitive index out of range");
+    B200rtSceneInfo info{};
+    info.n_prims = (uint64_t)n_sph + n_quad;
+    info.n_spheres = n_sph; info.n_quads = n_quad; info.n_materials = n_mat;
+    info.n_nodes = n_nodes;
+    info.tree_depth = depth;
+    const double total = now_ms() - t0;
+    info.build_ms = host_ms >= 0 ? host_ms : total;
+    info.upload_ms = total - info.build_ms;
+    return finish_scene(s, info);
+}
+
+// Builds the acceleration structure for `desc` (structure already validated) and makes the scene resident on device `dev`.
 int create_scene_on(const B200rtSceneDesc *desc, const B200rtBuildOpts *opts, int dev, bool peer_visible, SceneImpl **out) {
     *out = nullptr;
     SceneImpl *s = new SceneImpl();
@@ -591,26 +528,7 @@ int create_scene_on(const B200rtSceneDesc *desc, const B200rtBuildOpts *opts, in
     // 4 k-sphere scene), Morton LBVH on the GPU from 64 k primitives up (2.2 M / 3.1 M primitives:
     // tens of ms incl. the upload vs 0.8 / 1.0 s, with equal or better render rates)
     if (builder == B200RT_BUILDER_AUTO) builder = n_prims >= 65536 ? B200RT_BUILDER_GPU_LBVH : B200RT_BUILDER_HOST_SAH;
-    bool built = false;
-    const bool gpu_build = builder == B200RT_BUILDER_GPU_LBVH && n_prims >= 2;
-    if (int rc = validate_desc(desc, !gpu_build)) { delete s; return rc; }
-    if (gpu_build) {
-        bool too_deep = false;
-        if (int rc = scene_build_gpu(desc, s, &too_deep)) { free_scene(s); return rc; }
-        if (too_deep) {   // pathological depth: start over with the depth-capped host builder
-            scene_free_arrays(s);
-        } else {
-            built = true;
-        }
-    }
-    if (!built) {
-        if (gpu_build) { if (int rc = validate_desc(desc, true)) { free_scene(s); return rc; } }
-        if (int rc = scene_build_host(desc, opts, s)) { free_scene(s); return rc; }
-    }
-    s->info.n_prims = n_prims;
-    s->info.n_spheres = desc->n_spheres; s->info.n_quads = desc->n_quads; s->info.n_materials = desc->n_materials;
-    s->info.stack_entries = (uint32_t)s->stack;
-    if (int rc = finish_scene_setup(s)) { free_scene(s); return rc; }
+    if (int rc = scene_build(desc, opts, builder == B200RT_BUILDER_GPU_LBVH && n_prims >= 2, s)) { free_scene(s); return rc; }
     *out = s;
     return B200RT_OK;
 }
@@ -634,16 +552,7 @@ int replicate_scene_on(const SceneImpl *src, int dev, SceneImpl **out) {
             return fail(e == cudaErrorMemoryAllocation ? B200RT_ENOMEM : B200RT_ECUDA, std::string("scene copy to a peer device: ") + cudaGetErrorString(e));
         }
     }
-    s->d.nodes = static_cast<const float4 *>(s->allocs[0]);
-    s->d.spheres = static_cast<const double2 *>(s->allocs[1]);
-    s->d.sphere_meta = static_cast<const uint2 *>(s->allocs[2]);
-    s->d.quads = static_cast<const double2 *>(s->allocs[3]);
-    s->d.quad_meta = static_cast<const uint2 *>(s->allocs[4]);
-    s->d.materials = static_cast<const DeviceMaterial *>(s->allocs[5]);
-    if (reinterpret_cast<uintptr_t>(s->d.nodes) & 127) { free_scene(s); return fail(B200RT_ECUDA, "node array is not 128-byte aligned"); }
-    s->info = src->info;
-    s->stack = src->stack;
-    if (int rc = finish_scene_setup(s)) { free_scene(s); return rc; }
+    if (int rc = finish_scene(s, src->info)) { free_scene(s); return rc; }
     *out = s;
     return B200RT_OK;
 }

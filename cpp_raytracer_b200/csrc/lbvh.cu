@@ -5,8 +5,9 @@
 // time-to-first-pixel matters more than tree quality -- the multi-million-primitive scenes, where
 // even the parallel host SAH builder (bvh_builder.cpp, ~0.8 s) costs more than the render at 8 GPUs.
 //
-// Pipeline, all device-side (the host only uploads the caller's flat arrays as they are):
-//   1. prim_setup      index validation of the description; primitive bounds exactly as the reference's constructors compute them
+// Builds the tree and the leaf order only, all device-side from the caller's flat arrays as they are; the
+// primitive records are laid out in that order by scene_layout.cu, as for the host builder:
+//   1. prim_setup      primitive bounds exactly as the reference's constructors compute them
 //                      (sphere.h:112-123, parallelogram.h:281-295) in double, rounded outward to FP32;
 //                      centroid bounds by warp shuffle + ordered-int atomics
 //   2. morton_codes    63-bit Morton code of the centroid (21 bits per axis)
@@ -14,11 +15,10 @@
 //   4. radix_tree      Karras 2012, "Maximizing parallelism in the construction of BVHs, octrees and
 //                      k-d trees": one thread per internal node, duplicates broken by index
 //   5. fit_boxes       bottom-up union of child boxes, second arrival continues (atomic counters)
-//   6. collapse_level  binary -> 4-wide, breadth first, one launch per level: each task pulls up the
+//   6. leaf_order      leaf (= Morton) position -> per-type position: sphere_order / quad_order
+//   7. collapse_level  binary -> 4-wide, breadth first, one launch per level: each task pulls up the
 //                      larger-area grandchildren until four slots are used, reserves its Node4 with an
 //                      atomic counter, patches its parent's child slot and queues its interior children
-//   7. reorder         spheres / quads / meta into leaf (= Morton) order; the quad constants
-//                      (unit normal, n/|n|^2) are computed in double exactly as on the host path
 // Closest-hit results do not depend on the tree, so the parity tests run against this builder too.
 #include <cstdio>
 #include <cub/cub.cuh>
@@ -26,7 +26,6 @@
 #include "../../include/b200rt.h"
 #include "bvh_builder.h"
 #include "devmem.h"
-#include "kernels.h"
 
 namespace b200rt {
 
@@ -46,17 +45,13 @@ struct PrimBoxes {
 };
 
 __global__ void prim_setup(const B200rtSphere *sph, uint32_t n_sph, const B200rtQuad *quads, uint32_t n_quad, PrimBoxes B,
-                           int *cbounds /* [6]: ordered-int min xyz, max xyz; [6]: bad-index flag */, uint32_t n_materials) {
+                           int *cbounds /* [6]: ordered-int min xyz, max xyz */) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     const uint32_t n = n_sph + n_quad;
     float c[3] = {0.f, 0.f, 0.f};
     const bool valid = i < n;
     if (valid) {
         double lo[3], hi[3];
-        // the scene description's index checks (material / canonical primitive index in range) happen here for the
-        // multi-million-primitive scenes instead of in a serial host loop over the caller's arrays
-        const uint32_t mat = i < n_sph ? sph[i].mat : quads[i - n_sph].mat, prim = i < n_sph ? sph[i].prim : quads[i - n_sph].prim;
-        if (mat >= n_materials || prim >= n) cbounds[6] = 1;
         if (i < n_sph) {                                   // sphere.h:112-123
             const B200rtSphere s = sph[i];
             for (int a = 0; a < 3; ++a) {
@@ -270,49 +265,14 @@ __global__ void collapse_level(BinTree T, PrimBoxes B, const uint32_t *vals, con
     }
 }
 
-// spheres / quads / meta into leaf (Morton) order
-__global__ void reorder_prims(const B200rtSphere *sph, uint32_t n_sph, const B200rtQuad *quads, const uint32_t *vals,
-                              const uint32_t *quad_rank, uint32_t n, double2 *out_sph, uint2 *out_sph_meta, double2 *out_quads,
-                              uint2 *out_quad_meta) {
+// the caller's index of the primitive at each leaf (Morton) position, per type
+__global__ void leaf_order(const uint32_t *vals, const uint32_t *quad_rank, uint32_t n, uint32_t n_sph, uint32_t *sphere_order,
+                           uint32_t *quad_order) {
     const uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= n) return;
     const uint32_t prim = vals[p];
-    if (prim < n_sph) {
-        const B200rtSphere s = sph[prim];
-        const uint32_t i = p - quad_rank[p];
-        out_sph[2 * (size_t)i] = make_double2(s.c[0], s.c[1]);
-        out_sph[2 * (size_t)i + 1] = make_double2(s.c[2], s.r);
-        out_sph_meta[i] = make_uint2(s.prim, s.mat);
-    } else {
-        const B200rtQuad q = quads[prim - n_sph];
-        const uint32_t i = quad_rank[p];
-        // parallelogram.h:275-279: n = cross(s1, s2); unit = n * (1 / |n|); w = n * (1 / |n|^2)
-        const double nx = q.s1[1] * q.s2[2] - q.s1[2] * q.s2[1], ny = q.s1[2] * q.s2[0] - q.s1[0] * q.s2[2],
-                     nz = q.s1[0] * q.s2[1] - q.s1[1] * q.s2[0];
-        const double m2 = nx * nx + ny * ny + nz * nz;
-        const double im = 1 / sqrt(m2), im2 = 1 / m2;
-        const double f[16] = {nx * im, ny * im, nz * im, q.v[0], q.v[1], q.v[2], nx * im2, ny * im2, nz * im2,
-                              q.s1[0], q.s1[1], q.s1[2], q.s2[0], q.s2[1], q.s2[2], 0.0};
-        for (int k = 0; k < 8; ++k) out_quads[8 * (size_t)i + k] = make_double2(f[2 * k], f[2 * k + 1]);
-        out_quad_meta[i] = make_uint2(q.prim, q.mat);
-    }
-}
-
-// B200rtMaterial (the caller's 40-byte records) -> DeviceMaterial, as api.cu's device_materials() does on the host for
-// small scenes: lights pre-multiplied by their intensity (material.h:261-263), metal fuzz clamped to 1
-// (material.h:150-151).  The reference's big scenes carry one material PER PRIMITIVE (millions), so this runs here.
-__global__ void convert_materials(const B200rtMaterial *__restrict__ raw, uint32_t n, DeviceMaterial *__restrict__ out, int *bad_kind) {
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    const B200rtMaterial m = raw[i];
-    if (m.kind > B200RT_MAT_LIGHT) *bad_kind = 1;
-    DeviceMaterial dm;
-    const double k = m.kind == B200RT_MAT_LIGHT ? m.param : 1.0;
-    dm.r = (float)(k * m.rgb[0]); dm.g = (float)(k * m.rgb[1]); dm.b = (float)(k * m.rgb[2]);
-    dm.kind = m.kind;
-    dm.param = m.kind == B200RT_MAT_METAL ? fmin(m.param, 1.0) : m.param;
-    dm.pad = 0.0;
-    out[i] = dm;
+    if (prim < n_sph) sphere_order[p - quad_rank[p]] = prim;
+    else quad_order[quad_rank[p]] = prim - n_sph;
 }
 
 template <typename T>
@@ -327,29 +287,12 @@ cudaError_t tmp_alloc(std::vector<void *> &owned, T **p, size_t count) {
 
 }  // namespace
 
-cudaError_t convert_materials_device(const B200rtMaterial *d_raw, uint32_t n, DeviceMaterial *d_out, int *bad_kind_out) {
-    *bad_kind_out = 0;
-    if (n == 0) return cudaSuccess;
-    int *flag = nullptr;
-    cudaError_t e = dev_alloc_async(&flag, sizeof(int), 0);
-    if (e != cudaSuccess) return e;
-    e = cudaMemsetAsync(flag, 0, sizeof(int), 0);
-    if (e == cudaSuccess) {
-        convert_materials<<<(n + 255) / 256, 256>>>(d_raw, n, d_out, flag);
-        e = cudaMemcpyAsync(bad_kind_out, flag, sizeof(int), cudaMemcpyDeviceToHost, 0);
-    }
-    if (e == cudaSuccess) e = cudaStreamSynchronize(0);
-    dev_free(flag);
-    return e;
-}
-
-// Builds the scene's device arrays on the GPU.  d_sph / d_quads are the caller's flat structs already
-// on the device.  Outputs (allocated by the caller with the sizes known up front): leaf-ordered
-// sphere / quad / meta arrays; the Node4 array is allocated here (its size is only known at the end)
-// with cudaMallocAsync and handed back through nodes_out.
+// Builds the 4-wide tree on the GPU.  d_sph / d_quads are the caller's flat structs already on the device.
+// Outputs: the leaf order, sphere_order[n_sph] / quad_order[n_quad] (allocated by the caller); the Node4 array
+// is allocated here (its size is only known at the end) with cudaMallocAsync and handed back through nodes_out.
 cudaError_t build_lbvh_device(const B200rtSphere *d_sph, uint32_t n_sph, const B200rtQuad *d_quads, uint32_t n_quad,
-                              uint32_t n_materials, double2 *out_sph, uint2 *out_sph_meta, double2 *out_quads, uint2 *out_quad_meta,
-                              float4 **nodes_out, uint32_t *n_nodes_out, uint32_t *depth_out, int *bad_index_out) {
+                              uint32_t *sphere_order, uint32_t *quad_order, float4 **nodes_out, uint32_t *n_nodes_out,
+                              uint32_t *depth_out) {
     const uint32_t n = n_sph + n_quad;
     // Encoding limits: a leaf reference holds a 26-bit index into its per-type array (bvh_builder.h), and the radix
     // tree's index arithmetic ((n - 1) + ~child, lmax * d) must stay inside int.  The host builder rejects the same
@@ -367,12 +310,10 @@ cudaError_t build_lbvh_device(const B200rtSphere *d_sph, uint32_t n_sph, const B
     LB(tmp_alloc(owned, &pb.hix, n)); LB(tmp_alloc(owned, &pb.hiy, n)); LB(tmp_alloc(owned, &pb.hiz, n));
     LB(tmp_alloc(owned, &pb.cx, n)); LB(tmp_alloc(owned, &pb.cy, n)); LB(tmp_alloc(owned, &pb.cz, n));
     int *cbounds;
-    LB(tmp_alloc(owned, &cbounds, 7));
-    const int init[7] = {0x7fffffff, 0x7fffffff, 0x7fffffff, (int)0x80000000, (int)0x80000000, (int)0x80000000, 0};
+    LB(tmp_alloc(owned, &cbounds, 6));
+    const int init[6] = {0x7fffffff, 0x7fffffff, 0x7fffffff, (int)0x80000000, (int)0x80000000, (int)0x80000000};
     LB(cudaMemcpyAsync(cbounds, init, sizeof init, cudaMemcpyHostToDevice, 0));
-    prim_setup<<<gn, B>>>(d_sph, n_sph, d_quads, n_quad, pb, cbounds, n_materials);
-    int bad_index = 0;
-    LB(cudaMemcpyAsync(&bad_index, cbounds + 6, sizeof(int), cudaMemcpyDeviceToHost, 0));   // read at the first sync below
+    prim_setup<<<gn, B>>>(d_sph, n_sph, d_quads, n_quad, pb, cbounds);
     unsigned long long *keys, *keys_alt;
     uint32_t *vals, *vals_alt;
     LB(tmp_alloc(owned, &keys, n)); LB(tmp_alloc(owned, &keys_alt, n));
@@ -408,7 +349,7 @@ cudaError_t build_lbvh_device(const B200rtSphere *d_sph, uint32_t n_sph, const B
         LB(tmp_alloc(owned, &tmp, tmp_bytes));
         LB(cub::DeviceScan::ExclusiveSum(tmp, tmp_bytes, flags, quad_rank, (int)n));
     }
-    reorder_prims<<<gn, B>>>(d_sph, n_sph, d_quads, vals, quad_rank, n, out_sph, out_sph_meta, out_quads, out_quad_meta);
+    leaf_order<<<gn, B>>>(vals, quad_rank, n, n_sph, sphere_order, quad_order);
     // breadth-first collapse to 4-wide nodes (at most n - 1 of them)
     LB(dev_alloc_async(&nodes4, (size_t)(n - 1) * sizeof(Node4), 0));
     CollapseTask *qa, *qb;
@@ -432,7 +373,6 @@ cudaError_t build_lbvh_device(const B200rtSphere *d_sph, uint32_t n_sph, const B
     LB(cudaStreamSynchronize(0));
     LB(cudaGetLastError());
     cleanup();
-    *bad_index_out = bad_index;
     *nodes_out = reinterpret_cast<float4 *>(nodes4);
     *n_nodes_out = n_nodes;
     *depth_out = depth;

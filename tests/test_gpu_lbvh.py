@@ -82,25 +82,18 @@ def test_lbvh_tiny_and_degenerate_inputs(n):
         assert np.array_equal(p, want_p) and np.array_equal(t, want_t), (n, layout)
 
 
-@pytest.mark.parametrize("field,value", [("mat", 1 << 30), ("prim", 1 << 30)])
+@pytest.mark.parametrize("field,value", [("mat", 1 << 30), ("prim", 1 << 30), ("kind", 9)])
 def test_gpu_builder_rejects_out_of_range_indices(golden, field, value):
-    """With the GPU builder the per-primitive index checks of the scene description run on the device (prim_setup);
-    a bad material or canonical index is still B200RT_EINVAL, exactly as on the host path."""
+    """Scene creation checks the description's per-primitive indices and material kinds on the device
+    (scene_layout.cu) whichever builder made the tree: a bad material or canonical index on a sphere or a quad, or an
+    unknown material kind, is B200RT_EINVAL under both builders."""
     import cpp_raytracer_b200 as rt
     from cpp_raytracer_b200 import capi
-    scene = golden.scene("rtow_final")
-    for prims in ("spheres",):
+    for name, prims, i in (("rtow_final", "spheres", 7), ("cornell", "quads", 3)):
+        scene = golden.scene(name)
         bad = capi.HostScene(scene.materials.copy(), scene.spheres.copy(), scene.quads.copy(), scene.camera)
-        getattr(bad, prims)[field][7] = value
-        with pytest.raises(rt.B200rtError) as e:
-            rt.DeviceSceneHandle(bad, builder=capi.BUILDER_GPU_LBVH)
-        assert e.value.code == capi.EINVAL
-        with pytest.raises(rt.B200rtError) as e:
-            rt.DeviceSceneHandle(bad, builder=capi.BUILDER_HOST_SAH)
-        assert e.value.code == capi.EINVAL
-    quads = golden.scene("cornell")
-    bad = capi.HostScene(quads.materials.copy(), quads.spheres.copy(), quads.quads.copy(), quads.camera)
-    bad.quads[field][3] = value
-    with pytest.raises(rt.B200rtError) as e:
-        rt.DeviceSceneHandle(bad, builder=capi.BUILDER_GPU_LBVH)
-    assert e.value.code == capi.EINVAL
+        (bad.materials if field == "kind" else getattr(bad, prims))[field][i] = value
+        for builder in (capi.BUILDER_GPU_LBVH, capi.BUILDER_HOST_SAH):
+            with pytest.raises(rt.B200rtError) as e:
+                rt.DeviceSceneHandle(bad, builder=builder)
+            assert e.value.code == capi.EINVAL, (name, prims, builder)
