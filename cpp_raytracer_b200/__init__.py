@@ -9,8 +9,8 @@ Layout:
     dist.py       sample-split multi-GPU render + NCCL reduce (one process per GPU)
 """
 from .capi import (B200rtError, DeviceSceneHandle, HostScene, camera_init, camera_with, device_count,  # noqa: F401
-                   lib, render_scene, selftest_bvh, tonemap)
+                   lib, render_scene, sample_variance, selftest_bvh, tonemap)
 from .scene_io import load_scene, save_scene  # noqa: F401
 
 __all__ = ["B200rtError", "DeviceSceneHandle", "HostScene", "camera_init", "camera_with", "device_count",
-           "lib", "render_scene", "selftest_bvh", "tonemap", "load_scene", "save_scene"]
+           "lib", "render_scene", "sample_variance", "selftest_bvh", "tonemap", "load_scene", "save_scene"]

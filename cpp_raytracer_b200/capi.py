@@ -97,6 +97,7 @@ EXPORTS = {
     "b200rt_raycast": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_double, C.c_double, C.c_void_p, C.c_void_p]),
     "b200rt_render": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(RenderOpts), C.c_void_p, C.POINTER(Stats)]),
     "b200rt_render_device": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(RenderOpts), C.c_void_p, C.c_void_p, C.POINTER(Stats)]),
+    "b200rt_render_moments": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(RenderOpts), C.c_void_p, C.c_void_p, C.POINTER(Stats)]),
     "b200rt_render_scene": (C.c_int, [C.POINTER(SceneDesc), C.c_void_p, C.POINTER(RenderOpts), C.POINTER(BuildOpts),
                                       C.c_void_p, C.POINTER(Stats), C.POINTER(SceneInfo)]),
     "b200rt_tonemap": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int]),
@@ -260,6 +261,20 @@ class DeviceSceneHandle:
         _check(lib().b200rt_render(self._h, cam.ctypes.data, C.byref(opts), out.ctypes.data, C.byref(st)))
         return out, st.as_dict()
 
+    def render_moments(self, cam: np.ndarray, seed: int = 0xB200, sample_offset: int = 0, sample_count: int = 0, flags: int = 0):
+        """render() plus each pixel's second moment (b200rt_render_moments): returns (mean, m2, stats), where m2 is the
+        mean over the samples of x^2 per channel (both planes are sums with FLAG_SUM).  sample_variance(mean, m2, n) turns
+        them into the per-pixel sample variance.  Default kernel only: the wavefront variant, FLAG_THREAD_PIXELS and
+        FLAG_COUNTERS are EINVAL."""
+        cam = np.ascontiguousarray(cam, dtype=CAMERA_DTYPE).reshape(1)
+        h, w = int(cam["image_h"][0]), int(cam["image_w"][0])
+        mean = np.empty((h, w, 3), dtype=np.float32)
+        m2 = np.empty((h, w, 3), dtype=np.float32)
+        opts = RenderOpts(seed, sample_offset, sample_count, VARIANT_MEGAKERNEL, flags)
+        st = Stats()
+        _check(lib().b200rt_render_moments(self._h, cam.ctypes.data, C.byref(opts), mean.ctypes.data, m2.ctypes.data, C.byref(st)))
+        return mean, m2, st.as_dict()
+
     def bounds_violations(self) -> np.ndarray:
         """[stack, node index, primitive / material index, pixel] violations counted by a -DB200RT_DEBUG_BOUNDS build."""
         out = np.zeros(4, dtype=np.uint64)
@@ -304,6 +319,17 @@ def render_scene(scene: HostScene, cam: np.ndarray, seed: int = 0xB200, sample_o
         _check(lib().b200rt_render_scene(C.byref(desc), cam.ctypes.data, C.byref(opts), None, out.ctypes.data,
                                          C.byref(st), C.byref(info)))
     return out, st.as_dict(), info.as_dict()
+
+
+def sample_variance(mean, m2, n: int) -> np.ndarray:
+    """Per-pixel, per-channel sample variance s^2 = n/(n-1) * (m2 - mean^2) from render_moments' MEAN planes over n
+    samples, in float64, clamped at 0 (FP32 rounding can push m2 - mean^2 slightly below 0); inf where n < 2.  The
+    standard error of the pixel mean is sqrt(s^2 / n)."""
+    mean = np.asarray(mean, dtype=np.float64)
+    m2 = np.asarray(m2, dtype=np.float64)
+    if n < 2:
+        return np.full(np.broadcast(mean, m2).shape, np.inf)
+    return np.maximum(n / (n - 1) * (m2 - mean * mean), 0.0)
 
 
 def debug_philox(counters_keys: np.ndarray, device: int = 0) -> np.ndarray:

@@ -302,19 +302,23 @@ int sample_range_of(const B200rtCamera *cam, const B200rtRenderOpts &o, uint64_t
 }
 
 // Enqueues the path kernel(s) of one render call on `st` (the caller holds s->mu and has made s->device current).
+// d_m2 (optional): the second-moment plane, written by the moments instantiation of the default kernel.
 int render_on_device(SceneImpl *s, const B200rtCamera *cam, const B200rtRenderOpts *opts, float *d_out,
-                     cudaStream_t st, B200rtStats *stats, bool sync_for_stats) {
+                     cudaStream_t st, B200rtStats *stats, bool sync_for_stats, float *d_m2 = nullptr) {
     RenderParams P{};
     if (int rc = fill_camera(cam, P.cam)) return rc;
     B200rtRenderOpts o{};
     if (opts) o = *opts;
     uint64_t count = 0;
     if (int rc = sample_range_of(cam, o, &count)) return rc;
+    if (d_m2 && (o.variant == B200RT_VARIANT_WAVEFRONT || (o.flags & (B200RT_FLAG_THREAD_PIXELS | B200RT_FLAG_COUNTERS))))
+        return fail(B200RT_EINVAL, "moments are rendered by the default kernel only: no wavefront variant, B200RT_FLAG_THREAD_PIXELS or B200RT_FLAG_COUNTERS");
     P.scene = s->d;
     P.seed = o.seed;
     P.sample_begin = (uint32_t)o.sample_offset;
     P.sample_count = (uint32_t)count;
     P.out = d_out;
+    P.out_m2 = d_m2;
     P.flags = o.flags;
     P.scale = (o.flags & B200RT_FLAG_SUM) || count == 0 ? 1.0f : (float)(1.0 / (double)count);
     P.counters = s->d_counters;
@@ -327,8 +331,10 @@ int render_on_device(SceneImpl *s, const B200rtCamera *cam, const B200rtRenderOp
     if (count == 0) {
         // an empty share of a sample split: no samples, so the sum is zero (nothing to add under ACCUMULATE)
         launches = 0;
-        if (!(o.flags & B200RT_FLAG_ACCUMULATE))
+        if (!(o.flags & B200RT_FLAG_ACCUMULATE)) {
             CUDA_TRY(cudaMemsetAsync(d_out, 0, (size_t)cam->image_w * cam->image_h * 3 * sizeof(float), st));
+            if (d_m2) CUDA_TRY(cudaMemsetAsync(d_m2, 0, (size_t)cam->image_w * cam->image_h * 3 * sizeof(float), st));
+        }
     } else if (o.variant == B200RT_VARIANT_WAVEFRONT) {
         // pool of path slots: 2^21 by default (B200RT_WF_SLOTS overrides, for experiments).  Renders of one scene
         // share the pool: each waits (on the device) for the previous one to be done with it.
@@ -352,13 +358,15 @@ int render_on_device(SceneImpl *s, const B200rtCamera *cam, const B200rtRenderOp
         bool leaf_first = s->info.n_quads > s->info.n_spheres;
         if (const char *lf = std::getenv("B200RT_LEAF_FIRST")) leaf_first = lf[0] == '1';   // experiments
         // the tile work pool counts (pixel, sample) items in 32 bits: more than 2^22 samples per pixel go in several launches
+        // (2^16 with moments: the range of the x^2 accumulator, kernels.h)
+        const uint64_t per_launch = d_m2 ? kMaxSamplesPerLaunchMoments : kMaxSamplesPerLaunch;
         launches = 0;
-        for (uint64_t done = 0; done < count; done += kMaxSamplesPerLaunch) {
+        for (uint64_t done = 0; done < count; done += per_launch) {
             RenderParams Q = P;
             Q.sample_begin = (uint32_t)(o.sample_offset + done);
-            Q.sample_count = (uint32_t)std::min<uint64_t>(kMaxSamplesPerLaunch, count - done);
+            Q.sample_count = (uint32_t)std::min<uint64_t>(per_launch, count - done);
             if (done) Q.flags |= kRenderAccumulate;
-            CUDA_TRY(launch_path_megakernel(s->stack, Q, (o.flags & B200RT_FLAG_COUNTERS) != 0, leaf_first, st));
+            CUDA_TRY(launch_path_megakernel(s->stack, Q, (o.flags & B200RT_FLAG_COUNTERS) != 0, leaf_first, st, d_m2 != nullptr));
             ++launches;
         }
     }
@@ -566,8 +574,10 @@ void collect_stats(SceneImpl *s, B200rtStats *st) {   // after the stream that r
     st->rays = c[0]; st->node_visits = c[1]; st->prim_tests = c[2]; st->quad_tests = c[3];
 }
 
-// One frame on all devices of `m` into the caller's host buffer: sample split, exchange, scale, read back.
-int render_multi(MultiImpl *m, const B200rtCamera *cam, const B200rtRenderOpts *opts, float *out_rgb, B200rtStats *stats) {
+// One frame on all devices of `m` into the caller's host buffer(s): sample split, exchange, scale, read back.  With
+// out_m2 every device's frame holds [image | second moment] and both planes go through the same per-float exchange.
+int render_multi(MultiImpl *m, const B200rtCamera *cam, const B200rtRenderOpts *opts, float *out_rgb, float *out_m2,
+                 B200rtStats *stats) {
     std::lock_guard<std::mutex> lk(m->mu);
     const double t0 = now_ms();
     CameraParams C{};
@@ -578,17 +588,19 @@ int render_multi(MultiImpl *m, const B200rtCamera *cam, const B200rtRenderOpts *
     if (int rc = sample_range_of(cam, o, &count)) return rc;
     const int n = (int)m->dev.size();
     const long long n_pixels = (long long)cam->image_w * cam->image_h;
-    const size_t floats = (size_t)n_pixels * 3;
-    if (floats > m->frame_floats) {
+    const size_t floats = (size_t)n_pixels * 3;               // one plane
+    const int planes = out_m2 ? 2 : 1;
+    const size_t all_floats = floats * planes;
+    if (all_floats > m->frame_floats) {
         for (int d = 0; d < n; ++d) {
             DeviceGuard g(m->dev[d]->device);
             peer_buffer_release(m->dev[d]->device, m->frame[d]); m->frame[d] = nullptr;
             if (d == 0) { dev_free(m->scratch); m->scratch = nullptr; }
             m->frame_floats = 0;
-            CUDA_TRY(peer_buffer_acquire(m->dev[d]->device, floats * sizeof(float), reinterpret_cast<void **>(&m->frame[d])));
-            if (d == 0 && !m->peers) CUDA_TRY(dev_alloc(&m->scratch, floats * sizeof(float)));
+            CUDA_TRY(peer_buffer_acquire(m->dev[d]->device, all_floats * sizeof(float), reinterpret_cast<void **>(&m->frame[d])));
+            if (d == 0 && !m->peers) CUDA_TRY(dev_alloc(&m->scratch, all_floats * sizeof(float)));
         }
-        m->frame_floats = floats;
+        m->frame_floats = all_floats;
     }
     std::vector<B200rtStats> st(n);
     for (int d = 0; d < n; ++d) {   // rank d of n: samples [count*d/n, count*(d+1)/n) of the requested range, as a SUM
@@ -598,7 +610,8 @@ int render_multi(MultiImpl *m, const B200rtCamera *cam, const B200rtRenderOpts *
         od.sample_offset = o.sample_offset + lo;
         od.sample_count = hi - lo;
         od.flags = (o.flags & (B200RT_FLAG_COUNTERS | B200RT_FLAG_THREAD_PIXELS)) | B200RT_FLAG_SUM | B200RT_FLAG_EXACT_COUNT;
-        if (int rc = render_on_device(m->dev[d], cam, &od, m->frame[d], m->stream[d], &st[d], false)) return rc;
+        if (int rc = render_on_device(m->dev[d], cam, &od, m->frame[d], m->stream[d], &st[d], false, out_m2 ? m->frame[d] + floats : nullptr))
+            return rc;
         CUDA_TRY(cudaEventRecord(m->ev_render[d], m->stream[d]));
     }
     const float scale = (o.flags & B200RT_FLAG_SUM) || count == 0 ? 1.0f : (float)(1.0 / (double)count);
@@ -620,7 +633,7 @@ int render_multi(MultiImpl *m, const B200rtCamera *cam, const B200rtRenderOpts *
             for (int r = 0; r < n; ++r)
                 if (r != d) CUDA_TRY(cudaStreamWaitEvent(m->stream[d], m->ev_render[r], 0));
             if (d == 0) CUDA_TRY(cudaEventRecord(x0, m->stream[0]));
-            CUDA_TRY(launch_reduce_finalize_peers(in, n, d, n_pixels, scale, m->frame[0], nullptr, 0, m->stream[d]));
+            CUDA_TRY(launch_reduce_finalize_peers(in, n, d, n_pixels * planes, scale, m->frame[0], nullptr, 0, m->stream[d]));
             CUDA_TRY(cudaEventRecord(m->ev_xchg[d], m->stream[d]));
             ++xchg_launches;
         }
@@ -633,11 +646,11 @@ int render_multi(MultiImpl *m, const B200rtCamera *cam, const B200rtRenderOpts *
         CUDA_TRY(cudaEventRecord(x0, m->stream[0]));
         for (int r = 1; r < n; ++r) {
             CUDA_TRY(cudaStreamWaitEvent(m->stream[0], m->ev_render[r], 0));
-            CUDA_TRY(cudaMemcpyPeerAsync(m->scratch, m->dev[0]->device, m->frame[r], m->dev[r]->device, floats * sizeof(float), m->stream[0]));
-            CUDA_TRY(launch_add_frame(m->frame[0], m->scratch, (long long)floats, m->stream[0]));
+            CUDA_TRY(cudaMemcpyPeerAsync(m->scratch, m->dev[0]->device, m->frame[r], m->dev[r]->device, all_floats * sizeof(float), m->stream[0]));
+            CUDA_TRY(launch_add_frame(m->frame[0], m->scratch, (long long)all_floats, m->stream[0]));
             ++xchg_launches;
         }
-        CUDA_TRY(launch_finalize(m->frame[0], n_pixels, scale, nullptr, 0, m->stream[0]));
+        CUDA_TRY(launch_finalize(m->frame[0], n_pixels * planes, scale, nullptr, 0, m->stream[0]));
         ++xchg_launches;
         CUDA_TRY(cudaEventRecord(x1, m->stream[0]));
     }
@@ -647,6 +660,7 @@ int render_multi(MultiImpl *m, const B200rtCamera *cam, const B200rtRenderOpts *
         CUDA_TRY(cudaStreamSynchronize(m->stream[0]));
         const double t1 = now_ms();
         CUDA_TRY(staged_download(out_rgb, m->frame[0], floats * sizeof(float), m->stream[0]));
+        if (out_m2) CUDA_TRY(staged_download(out_m2, m->frame[0] + floats, floats * sizeof(float), m->stream[0]));
         d2h_ms = now_ms() - t1;
     }
     B200rtStats total{};
@@ -668,10 +682,46 @@ int render_multi(MultiImpl *m, const B200rtCamera *cam, const B200rtRenderOpts *
     }
     total.kernel_launches += xchg_launches;
     total.d2h_ms = d2h_ms;
-    total.d2h_bytes = floats * sizeof(float);
+    total.d2h_bytes = all_floats * sizeof(float);
     total.replicate_ms = m->replicate_ms;
     total.total_ms = now_ms() - t0;
     if (stats) *stats = total;
+    return B200RT_OK;
+}
+
+// b200rt_render and b200rt_render_moments: one frame into the caller's host buffer(s).  out_m2 may be NULL (image only);
+// otherwise the scene's frame holds [image | second moment] and both planes are read back.
+int render_host(void *scene, const B200rtCamera *cam, const B200rtRenderOpts *opts, float *out_rgb, float *out_m2, B200rtStats *stats) {
+    if (MultiImpl *m = as_multi(scene)) return render_multi(m, cam, opts, out_rgb, out_m2, stats);
+    SceneImpl *s = as_scene(scene);
+    if (!s) return fail(B200RT_EINVAL, "bad scene handle");
+    {
+        CameraParams C{};
+        if (int rc = fill_camera(cam, C)) return rc;   // range-checks the dimensions BEFORE anything is sized by them
+    }
+    std::lock_guard<std::mutex> lk(s->mu);
+    DeviceGuard g(s->device);
+    const double t0 = now_ms();
+    const size_t floats = (size_t)cam->image_w * cam->image_h * 3;   // one plane
+    const size_t all_floats = floats * (out_m2 ? 2 : 1);
+    if (all_floats > s->frame_floats) {
+        if (s->d_frame) { dev_free(s->d_frame); s->d_frame = nullptr; s->frame_floats = 0; }
+        CUDA_TRY(dev_alloc(&s->d_frame, all_floats * sizeof(float)));
+        s->frame_floats = all_floats;
+    }
+    B200rtRenderOpts o{};
+    if (opts) o = *opts;
+    o.flags &= ~(uint32_t)B200RT_FLAG_ACCUMULATE;   // host entry always overwrites
+    B200rtStats local{};
+    if (int rc = render_on_device(s, cam, &o, s->d_frame, 0, &local, true, out_m2 ? s->d_frame + floats : nullptr)) return rc;
+    const double t1 = now_ms();
+    CUDA_TRY(staged_download(out_rgb, s->d_frame, floats * sizeof(float), 0));
+    if (out_m2) CUDA_TRY(staged_download(out_m2, s->d_frame + floats, floats * sizeof(float), 0));
+    const double t2 = now_ms();
+    local.d2h_ms = t2 - t1;
+    local.d2h_bytes = all_floats * sizeof(float);
+    local.total_ms = t2 - t0;
+    if (stats) *stats = local;
     return B200RT_OK;
 }
 
@@ -981,35 +1031,13 @@ int b200rt_render_device(void *scene, const B200rtCamera *cam, const B200rtRende
 
 int b200rt_render(void *scene, const B200rtCamera *cam, const B200rtRenderOpts *opts, float *out_rgb, B200rtStats *stats) {
     if (!cam || !out_rgb) return fail(B200RT_EINVAL, "camera or output pointer is NULL");
-    if (MultiImpl *m = as_multi(scene)) return render_multi(m, cam, opts, out_rgb, stats);
-    SceneImpl *s = as_scene(scene);
-    if (!s) return fail(B200RT_EINVAL, "bad scene handle");
-    {
-        CameraParams C{};
-        if (int rc = fill_camera(cam, C)) return rc;   // range-checks the dimensions BEFORE anything is sized by them
-    }
-    std::lock_guard<std::mutex> lk(s->mu);
-    DeviceGuard g(s->device);
-    const double t0 = now_ms();
-    const size_t floats = (size_t)cam->image_w * cam->image_h * 3;
-    if (floats > s->frame_floats) {
-        if (s->d_frame) { dev_free(s->d_frame); s->d_frame = nullptr; s->frame_floats = 0; }
-        CUDA_TRY(dev_alloc(&s->d_frame, floats * sizeof(float)));
-        s->frame_floats = floats;
-    }
-    B200rtRenderOpts o{};
-    if (opts) o = *opts;
-    o.flags &= ~(uint32_t)B200RT_FLAG_ACCUMULATE;   // host entry always overwrites
-    B200rtStats local{};
-    if (int rc = render_on_device(s, cam, &o, s->d_frame, 0, &local, true)) return rc;
-    const double t1 = now_ms();
-    CUDA_TRY(staged_download(out_rgb, s->d_frame, floats * sizeof(float), 0));
-    const double t2 = now_ms();
-    local.d2h_ms = t2 - t1;
-    local.d2h_bytes = floats * sizeof(float);
-    local.total_ms = t2 - t0;
-    if (stats) *stats = local;
-    return B200RT_OK;
+    return render_host(scene, cam, opts, out_rgb, nullptr, stats);
+}
+
+int b200rt_render_moments(void *scene, const B200rtCamera *cam, const B200rtRenderOpts *opts, float *out_rgb, float *out_m2,
+                          B200rtStats *stats) {
+    if (!cam || !out_rgb || !out_m2) return fail(B200RT_EINVAL, "camera or output pointer is NULL");
+    return render_host(scene, cam, opts, out_rgb, out_m2, stats);
 }
 
 int b200rt_render_scene_multi(const B200rtSceneDesc *desc, const B200rtCamera *cam, const B200rtRenderOpts *opts,

@@ -7,6 +7,8 @@
 //                         a lane whose path ended starts its next sample right away
 //                         [Camera::render<T> + ray_color, reference camera.h:205-297]
 //   tonemap_kernel        Reinhard + gamma 2 + int(255.999999 v)   [RGB::as_string, rgb.h:90-113]
+#include <type_traits>
+
 #include "kernels.h"
 #include "shade.cuh"
 
@@ -203,8 +205,16 @@ struct TilePool {
     unsigned int next;                 // next (pixel, sample) item of this tile
     long long acc[kPathBlock * 3];     // per tile pixel: sum of radiance x 2^30
 };
+// The moments instantiation's pool: the same, plus the sum of x^2 per pixel and channel in 2^-24 units (range: kernels.h).
+struct TilePoolMoments : TilePool {
+    long long acc2[kPathBlock * 3];    // per tile pixel: sum of radiance^2 x 2^24
+};
+template <bool MOMENTS>
+using TilePoolOf = std::conditional_t<MOMENTS, TilePoolMoments, TilePool>;
 constexpr float kFixScale = 1073741824.0f;            // 2^30
 constexpr double kFixInv = 1.0 / 1073741824.0;
+constexpr float kFix2Scale = 16777216.0f;             // 2^24
+constexpr double kFix2Inv = 1.0 / 16777216.0;
 
 struct TileMap {
     uint32_t x0, y0, vw, n_valid;      // tile origin, valid width, valid pixel count (edge tiles are ragged)
@@ -230,10 +240,20 @@ struct PoolLane {
 // (The 64-bit shared-memory atomicAdd compiles to a compare-and-swap loop, ATOMS.CAST.SPIN.64.  Splitting it into two native
 //  32-bit atomics with an exact carry -- the thread whose addition wrapped the low word carries into the high one -- was
 //  measured 2-5 % SLOWER on all six scenes in a same-box A/B, so the plain form stays.)
-__device__ __forceinline__ void pool_contribute(TilePool &tp, uint32_t lp, float r, float g, float b) {
+//   MOMENTS also sums x^2 per channel.  x^2 of a path is the square of its single non-zero contribution: a path adds
+// radiance at exactly one interaction -- the light it hits (DiffuseLight emits and never scatters, so the path ends there,
+// material.h:248-263) or the background on a miss -- and zero at every other one.  So squaring each contribution here is
+// the square of the path's sample radiance, with no per-lane state.
+template <bool MOMENTS = false>
+__device__ __forceinline__ void pool_contribute(TilePoolOf<MOMENTS> &tp, uint32_t lp, float r, float g, float b) {
     if (r != 0.0f) atomicAdd(reinterpret_cast<unsigned long long *>(&tp.acc[lp * 3 + 0]), (unsigned long long)__float2ll_rn(r * kFixScale));
     if (g != 0.0f) atomicAdd(reinterpret_cast<unsigned long long *>(&tp.acc[lp * 3 + 1]), (unsigned long long)__float2ll_rn(g * kFixScale));
     if (b != 0.0f) atomicAdd(reinterpret_cast<unsigned long long *>(&tp.acc[lp * 3 + 2]), (unsigned long long)__float2ll_rn(b * kFixScale));
+    if constexpr (MOMENTS) {
+        if (r != 0.0f) atomicAdd(reinterpret_cast<unsigned long long *>(&tp.acc2[lp * 3 + 0]), (unsigned long long)__float2ll_rn(r * r * kFix2Scale));
+        if (g != 0.0f) atomicAdd(reinterpret_cast<unsigned long long *>(&tp.acc2[lp * 3 + 1]), (unsigned long long)__float2ll_rn(g * g * kFix2Scale));
+        if (b != 0.0f) atomicAdd(reinterpret_cast<unsigned long long *>(&tp.acc2[lp * 3 + 2]), (unsigned long long)__float2ll_rn(b * b * kFix2Scale));
+    }
 }
 
 // Takes the tile's next (pixel, sample) item into L (false: none left).  Item order: group_shift = 0: sample-major
@@ -274,8 +294,9 @@ __device__ __forceinline__ bool pool_fetch(const RenderParams &P, const TileMap 
 }
 
 // shade_and_advance with the tile pool: same path semantics, same Philox keys (pixel, sample, bounce).
-__device__ __forceinline__ bool pool_shade_and_advance(const RenderParams &P, const TileMap &tm, TilePool &tp, uint32_t total_items,
-                                                       const Hit &best, PoolLane &L, Ray &ray) {
+template <bool MOMENTS = false>
+__device__ __forceinline__ bool pool_shade_and_advance(const RenderParams &P, const TileMap &tm, TilePoolOf<MOMENTS> &tp,
+                                                       uint32_t total_items, const Hit &best, PoolLane &L, Ray &ray) {
     const CameraParams &C = P.cam;
     const uint32_t k0 = (uint32_t)P.seed, k1 = (uint32_t)(P.seed >> 32);
     if (L.has_path) {
@@ -291,7 +312,7 @@ __device__ __forceinline__ bool pool_shade_and_advance(const RenderParams &P, co
             // ray_color(scattered, depth_left - 1): contributes nothing once depth_left hits 0 (camera.h:211-213)
             if (cont && ++L.bounce == C.max_depth) cont = false;
         }
-        pool_contribute(tp, L.lp, er, eg, eb);
+        pool_contribute<MOMENTS>(tp, L.lp, er, eg, eb);   // the path's only non-zero contribution, if any (see pool_contribute)
         if (!cont) L.has_path = false;
     }
     if (!L.has_path) {
@@ -304,14 +325,18 @@ __device__ __forceinline__ bool pool_shade_and_advance(const RenderParams &P, co
     return true;
 }
 
-__device__ __forceinline__ void pool_init(TilePool &tp) {
+template <bool MOMENTS = false>
+__device__ __forceinline__ void pool_init(TilePoolOf<MOMENTS> &tp) {
     if (threadIdx.x == 0) tp.next = 0u;
     for (int i = threadIdx.x; i < kPathBlock * 3; i += kPathBlock) tp.acc[i] = 0;
+    if constexpr (MOMENTS)
+        for (int i = threadIdx.x; i < kPathBlock * 3; i += kPathBlock) tp.acc2[i] = 0;
     __syncthreads();
 }
 
-// After the block's last path: thread t writes tile pixel t.
-__device__ __forceinline__ void pool_write_tile(const RenderParams &P, const TileMap &tm, TilePool &tp) {
+// After the block's last path: thread t writes tile pixel t (and, with MOMENTS, its x^2 sums, scaled the same way).
+template <bool MOMENTS = false>
+__device__ __forceinline__ void pool_write_tile(const RenderParams &P, const TileMap &tm, TilePoolOf<MOMENTS> &tp) {
     __syncthreads();
     const uint32_t lp = threadIdx.x;
     if (lp < tm.n_valid) {
@@ -324,6 +349,13 @@ __device__ __forceinline__ void pool_write_tile(const RenderParams &P, const Til
             const float k = P.scale;
             if (P.flags & kRenderAccumulate) { o[0] += sum_r * k; o[1] += sum_g * k; o[2] += sum_b * k; }
             else { o[0] = sum_r * k; o[1] = sum_g * k; o[2] = sum_b * k; }
+            if constexpr (MOMENTS) {
+                const float q_r = (float)((double)tp.acc2[lp * 3 + 0] * kFix2Inv), q_g = (float)((double)tp.acc2[lp * 3 + 1] * kFix2Inv),
+                            q_b = (float)((double)tp.acc2[lp * 3 + 2] * kFix2Inv);
+                float *o2 = P.out_m2 + (size_t)pixel * 3;
+                if (P.flags & kRenderAccumulate) { o2[0] += q_r * k; o2[1] += q_g * k; o2[2] += q_b * k; }
+                else { o2[0] = q_r * k; o2[1] = q_g * k; o2[2] = q_b * k; }
+            }
         }
     }
 }
@@ -344,24 +376,24 @@ __device__ __forceinline__ void write_counters(const RenderParams &P, uint32_t l
 }
 
 // path_megakernel_pool (variant 0, default): every lane runs traverse-then-shade in a loop and takes the tile's next
-// (pixel, sample) item as soon as its path ends.
-template <int STACK, bool COUNT, bool LEAF_FIRST = false, int MINB = kPathMinBlocks>
+// (pixel, sample) item as soon as its path ends.  MOMENTS: also the per-pixel sum of x^2 into P.out_m2 (b200rt_render_moments).
+template <int STACK, bool COUNT, bool LEAF_FIRST = false, int MINB = kPathMinBlocks, bool MOMENTS = false>
 __global__ void __launch_bounds__(kPathBlock, MINB) path_megakernel_pool(const __grid_constant__ RenderParams P) {
-    __shared__ TilePool tp;
+    __shared__ TilePoolOf<MOMENTS> tp;
     const CameraParams &C = P.cam;
     const TileMap tm = map_tile(C);
-    pool_init(tp);
+    pool_init<MOMENTS>(tp);
     const uint32_t total_items = C.max_depth > 0 ? tm.n_valid * P.sample_count : 0u;
     PoolLane L;
     Ray ray;
     TraversalCounters ctr;
     Hit best{0.0, kNoHit};
-    while (pool_shade_and_advance(P, tm, tp, total_items, best, L, ray)) {
+    while (pool_shade_and_advance<MOMENTS>(P, tm, tp, total_items, best, L, ray)) {
         // world.hit_by(ray, Interval::with_min(0.00001))  (camera.h:217)
         best = closest_hit<STACK, COUNT, LEAF_FIRST>(P.scene, ray.ox, ray.oy, ray.oz, ray.dx, ray.dy, ray.dz, 0.00001,
                                                   __longlong_as_double(0x7ff0000000000000LL), &ctr);
     }
-    pool_write_tile(P, tm, tp);
+    pool_write_tile<MOMENTS>(P, tm, tp);
     write_counters(P, L.rays, COUNT, ctr);
 }
 
@@ -624,9 +656,14 @@ cudaError_t launch_debug_shade(int stack, const DeviceScene &S, const double *ra
 }
 
 template <int STACK>
-static cudaError_t launch_path_t(const RenderParams &P, bool count, bool leaf_first, cudaStream_t st) {
+static cudaError_t launch_path_t(const RenderParams &P, bool count, bool leaf_first, cudaStream_t st, bool moments) {
     const uint32_t tiles = ((P.cam.w + (uint32_t)kPathTileW - 1u) / (uint32_t)kPathTileW) * ((P.cam.h + (uint32_t)kPathTileH - 1u) / (uint32_t)kPathTileH);
     if (tiles == 0) return cudaSuccess;
+    if (moments) {   // tile pool, no counters (the caller has rejected kRenderThreadPixels and the counters flag)
+        if (leaf_first) path_megakernel_pool<STACK, false, true, kPathMinBlocks, true><<<tiles, kPathBlock, 0, st>>>(P);
+        else path_megakernel_pool<STACK, false, false, kPathMinBlocks, true><<<tiles, kPathBlock, 0, st>>>(P);
+        return cudaGetLastError();
+    }
     if (!(P.flags & kRenderThreadPixels)) {
         if (leaf_first) {
             if (count) path_megakernel_pool<STACK, true, true><<<tiles, kPathBlock, 0, st>>>(P);
@@ -640,10 +677,10 @@ static cudaError_t launch_path_t(const RenderParams &P, bool count, bool leaf_fi
     return cudaGetLastError();
 }
 
-cudaError_t launch_path_megakernel(int stack, const RenderParams &P, bool count, bool leaf_first, cudaStream_t st) {
-    if (stack <= 32) return launch_path_t<32>(P, count, leaf_first, st);
-    if (stack <= 64) return launch_path_t<64>(P, count, leaf_first, st);
-    return launch_path_t<128>(P, count, leaf_first, st);
+cudaError_t launch_path_megakernel(int stack, const RenderParams &P, bool count, bool leaf_first, cudaStream_t st, bool moments) {
+    if (stack <= 32) return launch_path_t<32>(P, count, leaf_first, st, moments);
+    if (stack <= 64) return launch_path_t<64>(P, count, leaf_first, st, moments);
+    return launch_path_t<128>(P, count, leaf_first, st, moments);
 }
 
 cudaError_t launch_path_lanes(int stack, const RenderParams &P, unsigned long long *acc, bool leaf_first, cudaStream_t st) {

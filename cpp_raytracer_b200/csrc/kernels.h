@@ -29,6 +29,11 @@ constexpr int kPathMinBlocks = 1024 / kPathBlock;   // 1024 threads = 32 warps p
 constexpr uint32_t kRenderAccumulate = 2u;    // == B200RT_FLAG_ACCUMULATE
 constexpr uint32_t kRenderThreadPixels = 16u; // == B200RT_FLAG_THREAD_PIXELS
 constexpr uint32_t kMaxSamplesPerLaunch = 1u << 22;   // tile items (up to 1024 pixels x samples, + one group) are counted in 32 bits
+// Second-moment plane (path_megakernel_pool<..., MOMENTS = true>): the sum of x^2 per pixel and channel is kept in 64-bit
+// fixed point of 2^-24 units -- per-sample resolution 6.0e-8, range +-5.5e11 per pixel per launch.  At most 2^16 samples
+// per launch, so a mean x^2 of up to 8.4e6 per sample (x up to about 2900) fits; the brightest emitter of the scene
+// set (500 x 0.8) gives x^2 <= 1.6e5.
+constexpr uint32_t kMaxSamplesPerLaunchMoments = 1u << 16;
 
 struct RenderParams {
     DeviceScene scene;
@@ -40,6 +45,8 @@ struct RenderParams {
     uint32_t flags;
     unsigned long long *counters;      // [0] rays, [1] node visits, [2] primitive tests, [3] of which quad tests
     uint32_t group_shift;              // work-pool item order: 2^group_shift consecutive items are samples of one pixel
+    float *out_m2;                     // moments launches only: image_h x image_w x 3, mean (or sum) of x^2; last, so that
+                                       // the fields above keep their parameter offsets
 };
 
 // Path-slot pool of the wavefront variant (wavefront.cu); all pointers are device memory.
@@ -75,8 +82,10 @@ cudaError_t run_wavefront(int stack, const RenderParams &P, const WavefrontPool 
 // launchers pick the smallest instantiation that fits (32 / 64 / 128).
 cudaError_t launch_raycast(int stack, const DeviceScene &S, const double *rays, long long n, double tmin, double tmax,
                            int32_t *prim, double *t, cudaStream_t st);
-// leaf_first: order of the two steps inside one iteration of the traversal loop (see closest_hit)
-cudaError_t launch_path_megakernel(int stack, const RenderParams &P, bool count, bool leaf_first, cudaStream_t st);
+// leaf_first: order of the two steps inside one iteration of the traversal loop (see closest_hit).  moments: the tile-pool
+// kernel that also writes P.out_m2 (not with count, not with kRenderThreadPixels; at most kMaxSamplesPerLaunchMoments samples)
+cudaError_t launch_path_megakernel(int stack, const RenderParams &P, bool count, bool leaf_first, cudaStream_t st,
+                                   bool moments = false);
 // measurement only: 16 lane-accounting counters (see path_lanes_kernel)
 cudaError_t launch_path_lanes(int stack, const RenderParams &P, unsigned long long *acc, bool leaf_first, cudaStream_t st);
 cudaError_t launch_finalize(float *frame, long long n_pixels, float scale, int32_t *ldr, int clamp, cudaStream_t st);

@@ -36,7 +36,9 @@
 #include <thread>
 #include <type_traits>
 #include <typeinfo>
+#include <limits>
 #include <unordered_map>
+#include <utility>
 #include <vector>
 
 #include "../../../../include/b200rt.h"
@@ -853,13 +855,14 @@ public:
         return c;
     }
 
-    static Image to_image(const std::vector<float> &hdr, size_t w, size_t h, double scale = 1.0) {
+    template <typename V>
+    static Image to_image(const std::vector<V> &hdr, size_t w, size_t h, double scale = 1.0) {
         Image img = Image::with_dimensions(w, h);
         const unsigned T = w * h < (1u << 20) ? 1u : std::min(16u, std::max(1u, std::thread::hardware_concurrency()));
         b200rt_host::for_chunks(h, T, [&](unsigned, size_t lo, size_t hi) {          // rows are independent
             for (size_t r = lo; r < hi; ++r)
                 for (size_t c = 0; c < w; ++c) {
-                    const float *p = &hdr[(r * w + c) * 3];
+                    const V *p = &hdr[(r * w + c) * 3];
                     img[r][c] = RGB::from_mag(p[0] * scale, p[1] * scale, p[2] * scale);
                 }
         });
@@ -920,6 +923,88 @@ public:
         last_stats = total;
         last_info = bvh.info();
         return to_image(sum, image_w, image_h, 1.0 / (double)std::max<size_t>(1, done));
+    }
+
+    // Sample variance of one pixel channel from the mean of x and the mean of x^2 over n samples: n/(n-1) (m2 - mean^2),
+    // in double; +inf when n < 2.  Both planes come from FP32 frames (and x^2 is summed in 2^-24 units), so a difference
+    // within their resolution -- 2^-20 of m2, plus 2^-24 -- is no evidence of noise and counts as 0: a pixel whose
+    // samples are all equal (one that sees only the background) reports exactly 0.
+    static double sample_variance(double mean, double m2, size_t n) {
+        if (n < 2) return std::numeric_limits<double>::infinity();
+        const double d = m2 - mean * mean;
+        if (d <= std::ldexp(m2, -20) + std::ldexp(1.0, -24)) return 0.0;
+        return (double)n / (double)(n - 1) * d;
+    }
+
+    // Extension: render(bvh) and, per pixel and channel, the standard error of that mean, sqrt(s^2 / n) with s^2 the
+    // sample variance of the pixel's n = samples_per_pixel samples (b200rt_render_moments).  The first image is the one
+    // render(bvh) returns, bit for bit, up to 2^16 samples per pixel.
+    std::pair<Image, Image> render_with_noise(const BVH &bvh) {
+        const B200rtCamera cam = to_abi();
+        B200rtRenderOpts opts{};
+        opts.seed = rng_seed;
+        std::vector<float> hdr(image_w * image_h * 3), m2(image_w * image_h * 3);
+        if (b200rt_render_moments(bvh.handle(), &cam, &opts, hdr.data(), m2.data(), &last_stats) != B200RT_OK) {
+            std::cout << "Error: In Camera::render_with_noise(), " << b200rt_last_error() << std::endl;
+            std::exit(-1);
+        }
+        last_info = bvh.info();
+        std::vector<double> se(hdr.size());
+        for (size_t i = 0; i < hdr.size(); ++i) se[i] = std::sqrt(sample_variance(hdr[i], m2[i], samples_per_pixel) / (double)samples_per_pixel);
+        return {to_image(hdr, image_w, image_h), to_image(se, image_w, image_h)};
+    }
+
+    // Extension: renders until the frame is as clean as asked.  Passes of `samples_per_pass` samples over the resident
+    // scene, as render_progressive, each through b200rt_render_moments as SUM planes that are added on the host in
+    // double; stops after the first pass whose frame relative noise is <= rel_noise, or when samples_per_pixel samples
+    // are done.  Returns the mean image; stats().paths / (width * height) is the number of samples it used.
+    //   Frame relative noise = sqrt(mean over all pixels and channels of se^2) / (mean over all pixels and channels of
+    // the image), where se^2 = s^2 / n is the squared standard error of a pixel channel's mean (s^2: sample_variance).
+    // Channels, not luminance, because the moments are per channel.  +inf while fewer than 2 samples are done; 0 for a
+    // black, noise-free frame.
+    Image render_to_noise(const BVH &bvh, double rel_noise, size_t samples_per_pass) {
+        const B200rtCamera cam = to_abi();
+        const size_t n_fl = image_w * image_h * 3;
+        std::vector<double> sum(n_fl, 0.0), sum2(n_fl, 0.0);
+        std::vector<float> pass(n_fl), pass2(n_fl);
+        B200rtStats total{};
+        size_t done = 0;
+        samples_per_pass = std::max<size_t>(1, samples_per_pass);
+        while (done < samples_per_pixel) {
+            B200rtRenderOpts opts{};
+            opts.seed = rng_seed;
+            opts.sample_offset = done;
+            opts.sample_count = std::min(samples_per_pass, samples_per_pixel - done);
+            opts.flags = B200RT_FLAG_SUM;
+            B200rtStats st{};
+            if (b200rt_render_moments(bvh.handle(), &cam, &opts, pass.data(), pass2.data(), &st) != B200RT_OK) {
+                std::cout << "Error: In Camera::render_to_noise(), " << b200rt_last_error() << std::endl;
+                std::exit(-1);
+            }
+            for (size_t i = 0; i < n_fl; ++i) { sum[i] += pass[i]; sum2[i] += pass2[i]; }
+            done += opts.sample_count;
+            total.kernel_ms += st.kernel_ms; total.total_ms += st.total_ms; total.paths += st.paths; total.rays += st.rays;
+            total.kernel_launches += st.kernel_launches; total.d2h_bytes += st.d2h_bytes;
+            if (frame_relative_noise(sum, sum2, done) <= rel_noise) break;
+        }
+        last_stats = total;
+        last_info = bvh.info();
+        return to_image(sum, image_w, image_h, 1.0 / (double)std::max<size_t>(1, done));
+    }
+
+    // The frame relative noise (see render_to_noise) of SUM planes over n samples.
+    static double frame_relative_noise(const std::vector<double> &sum, const std::vector<double> &sum2, size_t n) {
+        if (n < 2 || sum.empty()) return std::numeric_limits<double>::infinity();
+        double se2 = 0, img = 0;
+        for (size_t i = 0; i < sum.size(); ++i) {
+            const double mean = sum[i] / (double)n;
+            se2 += sample_variance(mean, sum2[i] / (double)n, n) / (double)n;
+            img += mean;
+        }
+        se2 /= (double)sum.size();
+        img /= (double)sum.size();
+        if (!(img > 0)) return se2 > 0 ? std::numeric_limits<double>::infinity() : 0.0;
+        return std::sqrt(se2) / img;
     }
 
     // camera.h:301-303.  Builds the acceleration structure, uploads, renders on the GPU and

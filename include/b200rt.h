@@ -263,6 +263,19 @@ int b200rt_render(void *scene, const B200rtCamera *cam, const B200rtRenderOpts *
 int b200rt_render_device(void *scene, const B200rtCamera *cam, const B200rtRenderOpts *opts,
                          float *out_rgb_device, void *stream, B200rtStats *stats);
 
+/* b200rt_render plus, for every pixel and channel, the second moment of the sample radiance:
+ * out_m2 (image_h x image_w x 3 floats, same layout as out_rgb) = mean over the requested samples of x^2
+ * (the SUM of x^2 with B200RT_FLAG_SUM).  out_rgb is the same bits b200rt_render returns for the same
+ * arguments (up to FP32 summation order above 2^16 samples per pixel, where both planes are summed
+ * over several launches).  SUM frames of both planes add across sample ranges and devices, so the
+ * sample variance of a pixel is n/(n-1) * (m2 - mean^2).  Single- and multi-device scenes.
+ * The per-pixel sums of x^2 are accumulated in 64-bit fixed point (2^-24 units) over at most 2^16 samples per
+ * launch, so they are as independent of the GPU's work distribution as the image; one launch's sum of x^2 of one
+ * pixel must stay below 5.5e11 (a mean x^2 of 8.4e6 per sample, x up to about 2900).
+ * B200RT_EINVAL with the wavefront variant, B200RT_FLAG_THREAD_PIXELS or B200RT_FLAG_COUNTERS. */
+int b200rt_render_moments(void *scene, const B200rtCamera *cam, const B200rtRenderOpts *opts,
+                          float *out_rgb, float *out_m2, B200rtStats *stats);
+
 /* Replaces: Camera::render(const Scene &) end to end (camera.h:301-303): build + upload +
  * render + read back + free, all inside one call on host buffers. */
 int b200rt_render_scene(const B200rtSceneDesc *desc, const B200rtCamera *cam,
