@@ -91,6 +91,9 @@ struct SceneImpl {
     cudaEvent_t ev_pool = nullptr;   // wavefront: the path-slot pool is free again (renders of one scene share it)
     void *d_pool = nullptr;          // wavefront path-slot pool
     uint32_t pool_slots = 0;
+    cudaEvent_t ev_tail = nullptr;   // the tail scratch is free again (renders of one scene share it)
+    void *d_tail = nullptr;          // chunked tail tiles of the path kernel: partial sums and arrival counters, zero between launches
+    size_t tail_bytes = 0;
     int sm_count = 148;
 };
 
@@ -250,9 +253,11 @@ void free_scene(SceneImpl *s) {
     dev_free(s->d_prim);
     dev_free(s->d_t);
     dev_free(s->d_pool);
+    dev_free(s->d_tail);
     if (s->ev0) cudaEventDestroy(s->ev0);
     if (s->ev1) cudaEventDestroy(s->ev1);
     if (s->ev_pool) cudaEventDestroy(s->ev_pool);
+    if (s->ev_tail) cudaEventDestroy(s->ev_tail);
     s->magic = 0;
     delete s;
 }
@@ -299,6 +304,64 @@ int sample_range_of(const B200rtCamera *cam, const B200rtRenderOpts &o, uint64_t
         return fail(B200RT_EINVAL, "unknown kernel variant");
     *count_out = count;
     return B200RT_OK;
+}
+
+// The chunked tail of the tile-pool grid (RenderParams::tail_first): the last `tiles` tiles of the image are rendered by
+// blocks of about 1/`chunks` of their samples each, so that short blocks fill the SMs while the last whole tiles drain.
+// Default: twice the blocks the GPU holds at once, 8 chunks of at least 8 samples.  B200RT_TAIL_TILES=R[,K] forces R tail
+// tiles and K chunks per tile (R = 0: whole tiles only), for A/B measurements and tests.
+struct TailPlan {
+    uint32_t tiles = 0, chunks = 8, min_chunk = 8;
+    bool forced = false;
+};
+int plan_tail(SceneImpl *s, const CameraParams &C, bool count, bool leaf_first, bool moments, TailPlan *t) {
+    const uint32_t tiles = ((C.w + (uint32_t)kPathTileW - 1u) / (uint32_t)kPathTileW) * ((C.h + (uint32_t)kPathTileH - 1u) / (uint32_t)kPathTileH);
+    if (const char *e = std::getenv("B200RT_TAIL_TILES")) {
+        long long r = 0, k = 0;
+        const int n = std::sscanf(e, "%lld,%lld", &r, &k);
+        t->tiles = (uint32_t)std::min<long long>(tiles, std::max(0ll, r));
+        if (n == 2) { t->chunks = (uint32_t)std::max(1ll, std::min(k, 1ll << 22)); t->min_chunk = 1; }
+        t->forced = true;
+        return B200RT_OK;
+    }
+    int resident = 0;
+    if (cudaError_t e = path_resident_blocks(s->stack, count, leaf_first, moments, s->sm_count, &resident); e != cudaSuccess) {
+        cudaGetLastError();
+        return fail(B200RT_ECUDA, std::string("path kernel occupancy: ") + cudaGetErrorString(e));
+    }
+    t->tiles = (uint32_t)std::min<uint64_t>(tiles, 2ull * (uint64_t)std::max(0, resident));
+    return B200RT_OK;
+}
+
+// Points P at the scene's tail scratch for `tail_tiles` tiles, growing it if needed.  Renders of one scene share the
+// scratch: the caller's stream waits (on the device) until the previous render is done with it.  Every launch leaves it zero.
+cudaError_t tail_scratch(SceneImpl *s, uint32_t tail_tiles, bool moments, cudaStream_t st, RenderParams *P) {
+    const size_t bytes = tail_scratch_bytes(tail_tiles, moments);
+    if (bytes > s->tail_bytes) {
+        if (s->d_tail) { cudaEventSynchronize(s->ev_tail); dev_free(s->d_tail); s->d_tail = nullptr; s->tail_bytes = 0; }
+        if (cudaError_t e = dev_alloc(&s->d_tail, bytes); e != cudaSuccess) return e;
+        s->tail_bytes = bytes;
+        if (cudaError_t e = cudaMemsetAsync(s->d_tail, 0, bytes, st); e != cudaSuccess) return e;
+    }
+    if (cudaError_t e = cudaStreamWaitEvent(st, s->ev_tail, 0); e != cudaSuccess) return e;
+    P->tail_acc = static_cast<long long *>(s->d_tail);
+    P->tail_arrivals = reinterpret_cast<uint32_t *>(static_cast<char *>(s->d_tail) + bytes - (size_t)tail_tiles * sizeof(uint32_t));
+    return cudaSuccess;
+}
+
+// One launch's chunking of its tail tiles: the chunk is a multiple of 2^group_shift samples (so same-pixel item groups
+// stay whole and chunks partition the tile's items, kernels.cu block_items).  A launch whose samples make one chunk keeps
+// whole tiles, unless the chunk count was forced.
+void chunk_tail(const TailPlan &t, RenderParams &Q) {
+    const uint32_t n = Q.sample_count, group = 1u << Q.group_shift;
+    uint32_t chunk = std::max(t.min_chunk, (uint32_t)(((uint64_t)n + t.chunks - 1) / t.chunks));
+    chunk = (uint32_t)(((uint64_t)chunk + group - 1) / group * group);
+    const uint32_t k = (uint32_t)(((uint64_t)n + chunk - 1) / chunk);
+    if (k <= 1 && !t.forced) return;
+    const uint32_t tiles = ((Q.cam.w + (uint32_t)kPathTileW - 1u) / (uint32_t)kPathTileW) * ((Q.cam.h + (uint32_t)kPathTileH - 1u) / (uint32_t)kPathTileH);
+    Q.tail_first = tiles - t.tiles;
+    Q.tail_chunks = k;
+    Q.tail_chunk_samples = chunk;
 }
 
 // Enqueues the path kernel(s) of one render call on `st` (the caller holds s->mu and has made s->device current).
@@ -357,6 +420,12 @@ int render_on_device(SceneImpl *s, const B200rtCamera *cam, const B200rtRenderOp
         // order of the node and the leaf step inside a traversal iteration (traverse.cuh): leaf first when quads dominate
         bool leaf_first = s->info.n_quads > s->info.n_spheres;
         if (const char *lf = std::getenv("B200RT_LEAF_FIRST")) leaf_first = lf[0] == '1';   // experiments
+        const bool count_flag = (o.flags & B200RT_FLAG_COUNTERS) != 0;
+        TailPlan tail;
+        if (!(o.flags & B200RT_FLAG_THREAD_PIXELS)) {
+            if (int rc = plan_tail(s, P.cam, count_flag, leaf_first, d_m2 != nullptr, &tail)) return rc;
+            if (tail.tiles) CUDA_TRY(tail_scratch(s, tail.tiles, d_m2 != nullptr, st, &P));
+        }
         // the tile work pool counts (pixel, sample) items in 32 bits: more than 2^22 samples per pixel go in several launches
         // (2^16 with moments: the range of the x^2 accumulator, kernels.h)
         const uint64_t per_launch = d_m2 ? kMaxSamplesPerLaunchMoments : kMaxSamplesPerLaunch;
@@ -366,9 +435,11 @@ int render_on_device(SceneImpl *s, const B200rtCamera *cam, const B200rtRenderOp
             Q.sample_begin = (uint32_t)(o.sample_offset + done);
             Q.sample_count = (uint32_t)std::min<uint64_t>(per_launch, count - done);
             if (done) Q.flags |= kRenderAccumulate;
-            CUDA_TRY(launch_path_megakernel(s->stack, Q, (o.flags & B200RT_FLAG_COUNTERS) != 0, leaf_first, st, d_m2 != nullptr));
+            if (tail.tiles) chunk_tail(tail, Q);
+            CUDA_TRY(launch_path_megakernel(s->stack, Q, count_flag, leaf_first, st, d_m2 != nullptr));
             ++launches;
         }
+        if (tail.tiles) CUDA_TRY(cudaEventRecord(s->ev_tail, st));
     }
     CUDA_TRY(cudaEventRecord(s->ev1, st));
     if (stats) {
@@ -411,6 +482,7 @@ int finish_scene(SceneImpl *s, const B200rtSceneInfo &info) {
     if (e == cudaSuccess) e = cudaEventCreate(&s->ev0);
     if (e == cudaSuccess) e = cudaEventCreate(&s->ev1);
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&s->ev_pool, cudaEventDisableTiming);
+    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&s->ev_tail, cudaEventDisableTiming);
 #ifdef B200RT_DEBUG_BOUNDS
     if (e == cudaSuccess) e = dev_alloc(&s->d_viol, 4 * sizeof(unsigned long long));
     if (e == cudaSuccess) e = cudaMemsetAsync(s->d_viol, 0, 4 * sizeof(unsigned long long), 0);
@@ -1017,6 +1089,19 @@ int b200rt_debug_lane_accounting(void *scene, const B200rtCamera *cam, const B20
     if (e != cudaSuccess) { cudaGetLastError(); return fail(B200RT_ECUDA, std::string("lane accounting: ") + cudaGetErrorString(e)); }
     return B200RT_OK;
 }
+
+#ifdef B200RT_BLOCK_TIMES
+// Diagnostic build only (-DB200RT_BLOCK_TIMES, scripts/tail_profile.py): from now on every path_megakernel_pool launch on the
+// current device writes {start ns, end ns, SM} of block b to device_buf[3 b .. 3 b + 2], for b < n_blocks.  NULL disarms.
+int b200rt_debug_block_times(uint64_t *device_buf, uint64_t n_blocks) {
+    if (cudaError_t e = set_block_times(reinterpret_cast<unsigned long long *>(device_buf), (uint32_t)std::min<uint64_t>(n_blocks, 0xFFFFFFFFu));
+        e != cudaSuccess) {
+        cudaGetLastError();
+        return fail(B200RT_ECUDA, std::string("block times: ") + cudaGetErrorString(e));
+    }
+    return B200RT_OK;
+}
+#endif
 
 int b200rt_render_device(void *scene, const B200rtCamera *cam, const B200rtRenderOpts *opts, float *out_rgb_device,
                          void *stream, B200rtStats *stats) {

@@ -203,6 +203,8 @@ __device__ __forceinline__ bool shade_and_advance(const RenderParams &P, const P
 // miss), so three atomics per path at most.  Resolution 9.3e-10, range +-8.6e9 per pixel per launch.
 struct TilePool {
     unsigned int next;                 // next (pixel, sample) item of this tile
+    unsigned int slot;                 // BlockWork::slot (kept here rather than in a register through the path loop)
+    unsigned int last;                 // chunk blocks: this block arrived last and writes the tile
     long long acc[kPathBlock * 3];     // per tile pixel: sum of radiance x 2^30
 };
 // The moments instantiation's pool: the same, plus the sum of x^2 per pixel and channel in 2^-24 units (range: kernels.h).
@@ -219,15 +221,48 @@ constexpr double kFix2Inv = 1.0 / 16777216.0;
 struct TileMap {
     uint32_t x0, y0, vw, n_valid;      // tile origin, valid width, valid pixel count (edge tiles are ragged)
 };
-__device__ __forceinline__ TileMap map_tile(const CameraParams &C) {
+__device__ __forceinline__ TileMap map_tile(const CameraParams &C, uint32_t tile) {
     const uint32_t tiles_x = (C.w + (uint32_t)kPathTileW - 1u) / (uint32_t)kPathTileW;
-    const uint32_t tile_x = blockIdx.x % tiles_x, tile_y = blockIdx.x / tiles_x;
+    const uint32_t tile_x = tile % tiles_x, tile_y = tile / tiles_x;
     TileMap t;
     t.x0 = tile_x * (uint32_t)kPathTileW;
     t.y0 = tile_y * (uint32_t)kPathTileH;
     t.vw = min((uint32_t)kPathTileW, C.w - t.x0);
     t.n_valid = t.vw * min((uint32_t)kPathTileH, C.h - t.y0);
     return t;
+}
+
+// What one block of path_megakernel_pool renders: all samples of a tile, or -- in the tail of the grid -- one chunk
+// [s_begin, s_end) of a tail tile's samples.  The last whole tiles drain while the short chunk blocks that follow them
+// in the grid keep the SMs full, so a frame no longer ends on a partly idle GPU.  Nothing depends on the order in which
+// the hardware starts blocks.
+struct BlockWork {
+    uint32_t tile, s_begin, s_end;
+    uint32_t slot;                     // tail-tile ordinal, or kWholeTile
+};
+constexpr uint32_t kWholeTile = 0xFFFFFFFFu;
+__device__ __forceinline__ BlockWork block_work(const RenderParams &P) {
+    BlockWork w{blockIdx.x, 0u, P.sample_count, kWholeTile};
+    if (P.tail_chunks && blockIdx.x >= P.tail_first) {
+        const uint32_t j = blockIdx.x - P.tail_first;
+        w.slot = j / P.tail_chunks;
+        w.tile = P.tail_first + w.slot;
+        w.s_begin = (j - w.slot * P.tail_chunks) * P.tail_chunk_samples;
+        w.s_end = min(w.s_begin + P.tail_chunk_samples, P.sample_count);
+    }
+    return w;
+}
+
+// The block's (pixel, sample) items in pool_fetch's numbering: [*first, return value).  A chunk starts, and unless it is
+// the last one also ends, on a multiple of 2^group_shift samples (the host rounds the chunk size), so the item ranges of a
+// tile's chunks partition the items of the whole tile and every chunk sees the same (pixel, sample) pairs it would there.
+__device__ __forceinline__ uint32_t block_items(const RenderParams &P, const TileMap &tm, const BlockWork &w, uint32_t &first) {
+    const uint32_t gs = P.group_shift;
+    if (P.cam.max_depth == 0) { first = 0u; return 0u; }
+    if (gs == 0u) { first = tm.n_valid * w.s_begin; return tm.n_valid * w.s_end; }
+    const uint32_t per_block = tm.n_valid << gs;
+    first = per_block * (w.s_begin >> gs);
+    return per_block * ((w.s_end + (1u << gs) - 1u) >> gs);
 }
 
 struct PoolLane {
@@ -262,7 +297,7 @@ __device__ __forceinline__ void pool_contribute(TilePoolOf<MOMENTS> &tp, uint32_
 // C4b +15 %, C5 +5 % -- when the background is black.  With a bright background every escaping path adds to its pixel's
 // accumulator and lanes on the same pixel serialise on it (C1 -3 %; warp-aggregating the sums first costs more than it
 // saves), so the host picks g = 3 for a black background and 0 otherwise (profiles/r2_tile_shape.md).  The image is the same
-// bit for bit under every order.
+// bit for bit under every order.  The items run from pool_init's start to total_items (block_items).
 __device__ __forceinline__ bool pool_fetch(const RenderParams &P, const TileMap &tm, TilePool &tp, uint32_t total_items, PoolLane &L,
                                            uint32_t &px, uint32_t &py) {
     if (total_items == 0u) return false;
@@ -274,10 +309,9 @@ __device__ __forceinline__ bool pool_fetch(const RenderParams &P, const TileMap 
         else { L.s = item / tm.n_valid; L.lp = item - L.s * tm.n_valid; }
     } else {
         const uint32_t per_block = tm.n_valid << gs;                             // items per block of 2^g samples
-        const uint32_t limit = per_block * ((P.sample_count + (1u << gs) - 1u) >> gs);
         while (true) {
             const uint32_t item = atomicAdd(&tp.next, 1u);
-            if (item >= limit) return false;
+            if (item >= total_items) return false;
             const uint32_t s_hi = item / per_block, rem = item - s_hi * per_block;
             L.lp = rem >> gs;
             L.s = (s_hi << gs) + (rem & ((1u << gs) - 1u));
@@ -326,38 +360,75 @@ __device__ __forceinline__ bool pool_shade_and_advance(const RenderParams &P, co
 }
 
 template <bool MOMENTS = false>
-__device__ __forceinline__ void pool_init(TilePoolOf<MOMENTS> &tp) {
-    if (threadIdx.x == 0) tp.next = 0u;
+__device__ __forceinline__ void pool_init(TilePoolOf<MOMENTS> &tp, uint32_t first_item, uint32_t slot = kWholeTile) {
+    if (threadIdx.x == 0) { tp.next = first_item; tp.slot = slot; }
     for (int i = threadIdx.x; i < kPathBlock * 3; i += kPathBlock) tp.acc[i] = 0;
     if constexpr (MOMENTS)
         for (int i = threadIdx.x; i < kPathBlock * 3; i += kPathBlock) tp.acc2[i] = 0;
     __syncthreads();
 }
 
-// After the block's last path: thread t writes tile pixel t (and, with MOMENTS, its x^2 sums, scaled the same way).
+// Tile pixel lp's fixed-point sums a (and, with MOMENTS, its x^2 sums q, scaled the same way) -> the image.
+template <bool MOMENTS = false>
+__device__ __forceinline__ void store_tile_pixel(const RenderParams &P, const TileMap &tm, uint32_t lp, const long long (&a)[3],
+                                                 const long long (&q)[3]) {
+    const uint32_t px = tm.x0 + lp % tm.vw, py = tm.y0 + lp / tm.vw;
+    const uint32_t pixel = py * P.cam.w + px;
+    if (B200RT_CHECK(P.scene, pixel < P.cam.w * P.cam.h, 3)) {
+        const float sum_r = (float)((double)a[0] * kFixInv), sum_g = (float)((double)a[1] * kFixInv), sum_b = (float)((double)a[2] * kFixInv);
+        float *o = P.out + (size_t)pixel * 3;
+        const float k = P.scale;
+        if (P.flags & kRenderAccumulate) { o[0] += sum_r * k; o[1] += sum_g * k; o[2] += sum_b * k; }
+        else { o[0] = sum_r * k; o[1] = sum_g * k; o[2] = sum_b * k; }
+        if constexpr (MOMENTS) {
+            const float q_r = (float)((double)q[0] * kFix2Inv), q_g = (float)((double)q[1] * kFix2Inv), q_b = (float)((double)q[2] * kFix2Inv);
+            float *o2 = P.out_m2 + (size_t)pixel * 3;
+            if (P.flags & kRenderAccumulate) { o2[0] += q_r * k; o2[1] += q_g * k; o2[2] += q_b * k; }
+            else { o2[0] = q_r * k; o2[1] = q_g * k; o2[2] = q_b * k; }
+        }
+    }
+}
+
+// After the block's last path: thread t writes tile pixel t.
 template <bool MOMENTS = false>
 __device__ __forceinline__ void pool_write_tile(const RenderParams &P, const TileMap &tm, TilePoolOf<MOMENTS> &tp) {
     __syncthreads();
     const uint32_t lp = threadIdx.x;
     if (lp < tm.n_valid) {
-        const uint32_t px = tm.x0 + lp % tm.vw, py = tm.y0 + lp / tm.vw;
-        const uint32_t pixel = py * P.cam.w + px;
-        if (B200RT_CHECK(P.scene, pixel < P.cam.w * P.cam.h, 3)) {
-            const float sum_r = (float)((double)tp.acc[lp * 3 + 0] * kFixInv), sum_g = (float)((double)tp.acc[lp * 3 + 1] * kFixInv),
-                        sum_b = (float)((double)tp.acc[lp * 3 + 2] * kFixInv);
-            float *o = P.out + (size_t)pixel * 3;
-            const float k = P.scale;
-            if (P.flags & kRenderAccumulate) { o[0] += sum_r * k; o[1] += sum_g * k; o[2] += sum_b * k; }
-            else { o[0] = sum_r * k; o[1] = sum_g * k; o[2] = sum_b * k; }
-            if constexpr (MOMENTS) {
-                const float q_r = (float)((double)tp.acc2[lp * 3 + 0] * kFix2Inv), q_g = (float)((double)tp.acc2[lp * 3 + 1] * kFix2Inv),
-                            q_b = (float)((double)tp.acc2[lp * 3 + 2] * kFix2Inv);
-                float *o2 = P.out_m2 + (size_t)pixel * 3;
-                if (P.flags & kRenderAccumulate) { o2[0] += q_r * k; o2[1] += q_g * k; o2[2] += q_b * k; }
-                else { o2[0] = q_r * k; o2[1] = q_g * k; o2[2] = q_b * k; }
-            }
-        }
+        const long long a[3] = {tp.acc[lp * 3 + 0], tp.acc[lp * 3 + 1], tp.acc[lp * 3 + 2]};
+        long long q[3] = {0, 0, 0};
+        if constexpr (MOMENTS) { q[0] = tp.acc2[lp * 3 + 0]; q[1] = tp.acc2[lp * 3 + 1]; q[2] = tp.acc2[lp * 3 + 2]; }
+        store_tile_pixel<MOMENTS>(P, tm, lp, a, q);
     }
+}
+
+// After a chunk block's last path: add its sums into the tail tile's slot of P.tail_acc with 64-bit integer atomics (so the
+// total does not depend on how the samples were split or in which order the chunks finish), then count the block in.
+// The chunk that arrives last takes the totals -- leaving the slot and its counter zero for the next launch -- and writes
+// the pixels exactly as pool_write_tile does.  No block waits for another.
+template <bool MOMENTS = false>
+__device__ __forceinline__ void pool_merge_chunk(const RenderParams &P, const TileMap &tm, TilePoolOf<MOMENTS> &tp, uint32_t slot) {
+    constexpr uint32_t kPlane = (uint32_t)kPathBlock * 3u;
+    unsigned long long *part = reinterpret_cast<unsigned long long *>(P.tail_acc) + (size_t)slot * kPlane * (MOMENTS ? 2u : 1u);
+    for (uint32_t i = threadIdx.x; i < kPlane; i += kPathBlock) {
+        if (tp.acc[i]) atomicAdd(&part[i], (unsigned long long)tp.acc[i]);
+        if constexpr (MOMENTS)
+            if (tp.acc2[i]) atomicAdd(&part[kPlane + i], (unsigned long long)tp.acc2[i]);
+    }
+    __threadfence();
+    __syncthreads();
+    if (threadIdx.x == 0) tp.last = atomicAdd(&P.tail_arrivals[slot], 1u) == P.tail_chunks - 1u;
+    __syncthreads();
+    if (!tp.last) return;
+    __threadfence();
+    const uint32_t lp = threadIdx.x;
+    long long a[3], q[3] = {0, 0, 0};
+    for (int c = 0; c < 3; ++c) {
+        a[c] = (long long)atomicExch(&part[lp * 3 + c], 0ull);
+        if constexpr (MOMENTS) q[c] = (long long)atomicExch(&part[kPlane + lp * 3 + c], 0ull);
+    }
+    if (lp == 0) P.tail_arrivals[slot] = 0u;
+    if (lp < tm.n_valid) store_tile_pixel<MOMENTS>(P, tm, lp, a, q);
 }
 
 __device__ __forceinline__ void write_counters(const RenderParams &P, uint32_t lane_rays, bool count, const TraversalCounters &ctr) {
@@ -375,15 +446,44 @@ __device__ __forceinline__ void write_counters(const RenderParams &P, uint32_t l
     }
 }
 
+#ifdef B200RT_BLOCK_TIMES
+// Diagnostic build (-DB200RT_BLOCK_TIMES, scripts/tail_profile.py): thread 0 of every path_megakernel_pool block records
+// {start ns, end ns, SM} of %globaltimer into g_block_times[blockIdx.x] (armed by b200rt_debug_block_times).
+__device__ unsigned long long *g_block_times;
+__device__ uint32_t g_block_times_n;
+__device__ __forceinline__ unsigned long long globaltimer_ns() {
+    unsigned long long t;
+    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+    return t;
+}
+__device__ __forceinline__ void record_block_time(unsigned long long t_start) {
+    if (threadIdx.x != 0 || !g_block_times || blockIdx.x >= g_block_times_n) return;
+    uint32_t sm;
+    asm volatile("mov.u32 %0, %%smid;" : "=r"(sm));
+    unsigned long long *r = g_block_times + (size_t)blockIdx.x * 3;
+    r[0] = t_start; r[1] = globaltimer_ns(); r[2] = sm;
+}
+cudaError_t set_block_times(unsigned long long *buf, uint32_t n_blocks) {
+    cudaError_t e = cudaMemcpyToSymbol(g_block_times, &buf, sizeof buf);
+    if (e == cudaSuccess) e = cudaMemcpyToSymbol(g_block_times_n, &n_blocks, sizeof n_blocks);
+    return e;
+}
+#endif
+
 // path_megakernel_pool (variant 0, default): every lane runs traverse-then-shade in a loop and takes the tile's next
 // (pixel, sample) item as soon as its path ends.  MOMENTS: also the per-pixel sum of x^2 into P.out_m2 (b200rt_render_moments).
 template <int STACK, bool COUNT, bool LEAF_FIRST = false, int MINB = kPathMinBlocks, bool MOMENTS = false>
 __global__ void __launch_bounds__(kPathBlock, MINB) path_megakernel_pool(const __grid_constant__ RenderParams P) {
     __shared__ TilePoolOf<MOMENTS> tp;
+#ifdef B200RT_BLOCK_TIMES
+    const unsigned long long t_start = globaltimer_ns();
+#endif
     const CameraParams &C = P.cam;
-    const TileMap tm = map_tile(C);
-    pool_init<MOMENTS>(tp);
-    const uint32_t total_items = C.max_depth > 0 ? tm.n_valid * P.sample_count : 0u;
+    const BlockWork w = block_work(P);
+    const TileMap tm = map_tile(C, w.tile);
+    uint32_t first_item;
+    const uint32_t total_items = block_items(P, tm, w, first_item);
+    pool_init<MOMENTS>(tp, first_item, w.slot);
     PoolLane L;
     Ray ray;
     TraversalCounters ctr;
@@ -393,8 +493,14 @@ __global__ void __launch_bounds__(kPathBlock, MINB) path_megakernel_pool(const _
         best = closest_hit<STACK, COUNT, LEAF_FIRST>(P.scene, ray.ox, ray.oy, ray.oz, ray.dx, ray.dy, ray.dz, 0.00001,
                                                   __longlong_as_double(0x7ff0000000000000LL), &ctr);
     }
-    pool_write_tile<MOMENTS>(P, tm, tp);
+    __syncthreads();
+    const uint32_t slot = tp.slot;
+    if (slot == kWholeTile) pool_write_tile<MOMENTS>(P, tm, tp);
+    else pool_merge_chunk<MOMENTS>(P, tm, tp, slot);
     write_counters(P, L.rays, COUNT, ctr);
+#ifdef B200RT_BLOCK_TIMES
+    record_block_time(t_start);
+#endif
 }
 
 // ------------------------------------------------------------------------------------------
@@ -435,9 +541,11 @@ __global__ void __launch_bounds__(kPathBlock) path_lanes_kernel(const __grid_con
     __shared__ TilePool tp;
     const CameraParams &C = P.cam;
     const PixelMap m = map_pixel(C);
-    const TileMap tm = map_tile(C);
-    if (POOL) pool_init(tp);
-    const uint32_t total_items = C.max_depth > 0 ? tm.n_valid * P.sample_count : 0u;
+    const BlockWork w = block_work(P);   // whole tiles: the measurement launch has no chunked tail
+    const TileMap tm = map_tile(C, w.tile);
+    uint32_t first_item;
+    const uint32_t total_items = block_items(P, tm, w, first_item);
+    if (POOL) pool_init(tp, first_item);
     LaneState L;
     PoolLane Lp;
     Trav T;
@@ -659,17 +767,19 @@ template <int STACK>
 static cudaError_t launch_path_t(const RenderParams &P, bool count, bool leaf_first, cudaStream_t st, bool moments) {
     const uint32_t tiles = ((P.cam.w + (uint32_t)kPathTileW - 1u) / (uint32_t)kPathTileW) * ((P.cam.h + (uint32_t)kPathTileH - 1u) / (uint32_t)kPathTileH);
     if (tiles == 0) return cudaSuccess;
+    // tile pool: whole-tile blocks, then tail_chunks chunk blocks for each tile from tail_first on
+    const uint32_t blocks = P.tail_chunks ? P.tail_first + (tiles - P.tail_first) * P.tail_chunks : tiles;
     if (moments) {   // tile pool, no counters (the caller has rejected kRenderThreadPixels and the counters flag)
-        if (leaf_first) path_megakernel_pool<STACK, false, true, kPathMinBlocks, true><<<tiles, kPathBlock, 0, st>>>(P);
-        else path_megakernel_pool<STACK, false, false, kPathMinBlocks, true><<<tiles, kPathBlock, 0, st>>>(P);
+        if (leaf_first) path_megakernel_pool<STACK, false, true, kPathMinBlocks, true><<<blocks, kPathBlock, 0, st>>>(P);
+        else path_megakernel_pool<STACK, false, false, kPathMinBlocks, true><<<blocks, kPathBlock, 0, st>>>(P);
         return cudaGetLastError();
     }
     if (!(P.flags & kRenderThreadPixels)) {
         if (leaf_first) {
-            if (count) path_megakernel_pool<STACK, true, true><<<tiles, kPathBlock, 0, st>>>(P);
-            else path_megakernel_pool<STACK, false, true><<<tiles, kPathBlock, 0, st>>>(P);
-        } else if (count) path_megakernel_pool<STACK, true><<<tiles, kPathBlock, 0, st>>>(P);
-        else path_megakernel_pool<STACK, false><<<tiles, kPathBlock, 0, st>>>(P);
+            if (count) path_megakernel_pool<STACK, true, true><<<blocks, kPathBlock, 0, st>>>(P);
+            else path_megakernel_pool<STACK, false, true><<<blocks, kPathBlock, 0, st>>>(P);
+        } else if (count) path_megakernel_pool<STACK, true><<<blocks, kPathBlock, 0, st>>>(P);
+        else path_megakernel_pool<STACK, false><<<blocks, kPathBlock, 0, st>>>(P);
         return cudaGetLastError();
     }
     if (count) path_megakernel<STACK, true><<<tiles, kPathBlock, 0, st>>>(P);      // round-1 work distribution: node-then-leaf only
@@ -681,6 +791,31 @@ cudaError_t launch_path_megakernel(int stack, const RenderParams &P, bool count,
     if (stack <= 32) return launch_path_t<32>(P, count, leaf_first, st, moments);
     if (stack <= 64) return launch_path_t<64>(P, count, leaf_first, st, moments);
     return launch_path_t<128>(P, count, leaf_first, st, moments);
+}
+
+size_t tail_scratch_bytes(uint32_t tail_tiles, bool moments) {
+    return (size_t)tail_tiles * ((size_t)kPathBlock * 3 * sizeof(long long) * (moments ? 2 : 1) + sizeof(uint32_t));
+}
+
+template <int STACK>
+static cudaError_t path_blocks_per_sm(bool count, bool leaf_first, bool moments, int &n) {
+    cudaError_t e;
+    if (moments) e = leaf_first ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, path_megakernel_pool<STACK, false, true, kPathMinBlocks, true>, kPathBlock, 0)
+                                : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, path_megakernel_pool<STACK, false, false, kPathMinBlocks, true>, kPathBlock, 0);
+    else if (leaf_first) e = count ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, path_megakernel_pool<STACK, true, true>, kPathBlock, 0)
+                                   : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, path_megakernel_pool<STACK, false, true>, kPathBlock, 0);
+    else e = count ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, path_megakernel_pool<STACK, true>, kPathBlock, 0)
+                   : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, path_megakernel_pool<STACK, false>, kPathBlock, 0);
+    return e;
+}
+
+cudaError_t path_resident_blocks(int stack, bool count, bool leaf_first, bool moments, int sm_count, int *blocks) {
+    int n = 0;
+    const cudaError_t e = stack <= 32   ? path_blocks_per_sm<32>(count, leaf_first, moments, n)
+                          : stack <= 64 ? path_blocks_per_sm<64>(count, leaf_first, moments, n)
+                                        : path_blocks_per_sm<128>(count, leaf_first, moments, n);
+    *blocks = n * sm_count;
+    return e;
 }
 
 cudaError_t launch_path_lanes(int stack, const RenderParams &P, unsigned long long *acc, bool leaf_first, cudaStream_t st) {

@@ -47,7 +47,20 @@ struct RenderParams {
     uint32_t group_shift;              // work-pool item order: 2^group_shift consecutive items are samples of one pixel
     float *out_m2;                     // moments launches only: image_h x image_w x 3, mean (or sum) of x^2; last, so that
                                        // the fields above keep their parameter offsets
+    // Tail of the tile-pool grid (path_megakernel_pool): blocks [0, tail_first) render whole tiles; with tail_chunks > 0,
+    // each of the remaining tiles is split into tail_chunks blocks of tail_chunk_samples samples (the last one ragged),
+    // which sum into tail_acc and let the last of them to arrive write the pixels.  tail_chunks = 0: whole tiles only.
+    uint32_t tail_first, tail_chunks, tail_chunk_samples;
+    long long *tail_acc;               // per tail tile: kPathBlock x 3 sums (x 2 with moments), zero between launches
+    uint32_t *tail_arrivals;           // per tail tile: chunk blocks done, zero between launches
 };
+// Scratch of a launch with `tail_tiles` chunked tail tiles: tail_acc, then tail_arrivals.
+size_t tail_scratch_bytes(uint32_t tail_tiles, bool moments);
+// Path blocks of the tile-pool kernel resident on the current device at once (occupancy x SM count).
+cudaError_t path_resident_blocks(int stack, bool count, bool leaf_first, bool moments, int sm_count, int *blocks);
+#ifdef B200RT_BLOCK_TIMES
+cudaError_t set_block_times(unsigned long long *buf, uint32_t n_blocks);   // diagnostic build: see kernels.cu
+#endif
 
 // Path-slot pool of the wavefront variant (wavefront.cu); all pointers are device memory.
 // One slot = one 128-byte line, read and written with 16-byte vector accesses.
