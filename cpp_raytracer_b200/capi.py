@@ -62,6 +62,10 @@ class RenderOpts(C.Structure):
                 ("variant", C.c_int32), ("flags", C.c_uint32)]
 
 
+class AdaptiveOpts(C.Structure):
+    _fields_ = [("min_spp", C.c_uint32), ("step_spp", C.c_uint32), ("rel_noise", C.c_double), ("abs_noise", C.c_double)]
+
+
 class Stats(C.Structure):
     _fields_ = [("kernel_ms", C.c_double), ("h2d_ms", C.c_double), ("d2h_ms", C.c_double), ("total_ms", C.c_double),
                 ("paths", C.c_uint64), ("rays", C.c_uint64), ("node_visits", C.c_uint64), ("prim_tests", C.c_uint64),
@@ -98,6 +102,8 @@ EXPORTS = {
     "b200rt_render": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(RenderOpts), C.c_void_p, C.POINTER(Stats)]),
     "b200rt_render_device": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(RenderOpts), C.c_void_p, C.c_void_p, C.POINTER(Stats)]),
     "b200rt_render_moments": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(RenderOpts), C.c_void_p, C.c_void_p, C.POINTER(Stats)]),
+    "b200rt_render_adaptive": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(RenderOpts), C.POINTER(AdaptiveOpts), C.c_void_p,
+                                         C.c_void_p, C.c_void_p, C.POINTER(Stats)]),
     "b200rt_render_scene": (C.c_int, [C.POINTER(SceneDesc), C.c_void_p, C.POINTER(RenderOpts), C.POINTER(BuildOpts),
                                       C.c_void_p, C.POINTER(Stats), C.POINTER(SceneInfo)]),
     "b200rt_tonemap": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int]),
@@ -274,6 +280,25 @@ class DeviceSceneHandle:
         st = Stats()
         _check(lib().b200rt_render_moments(self._h, cam.ctypes.data, C.byref(opts), mean.ctypes.data, m2.ctypes.data, C.byref(st)))
         return mean, m2, st.as_dict()
+
+    def render_adaptive(self, cam: np.ndarray, rel_noise: float, abs_noise: float = 0.0, min_spp: int = 16, step_spp: int = 16,
+                        seed: int = 0xB200, sample_offset: int = 0, sample_count: int = 0, flags: int = 0):
+        """Adaptive sampling (b200rt_render_adaptive): each pixel gets samples, min_spp first and then step_spp per pass,
+        until its own standard error is <= rel_noise x its mean radiance + abs_noise (judged over its 3 x 3 neighbourhood),
+        or it reaches the render's sample count (sample_count, else the camera's spp; at most 2^16).  Returns
+        (mean, m2, spp, stats): each pixel's planes are the bits render_moments returns for a uniform render of spp[y, x]
+        samples (sums with FLAG_SUM); spp is uint32."""
+        cam = np.ascontiguousarray(cam, dtype=CAMERA_DTYPE).reshape(1)
+        h, w = int(cam["image_h"][0]), int(cam["image_w"][0])
+        mean = np.empty((h, w, 3), dtype=np.float32)
+        m2 = np.empty((h, w, 3), dtype=np.float32)
+        spp = np.empty((h, w), dtype=np.uint32)
+        opts = RenderOpts(seed, sample_offset, sample_count, VARIANT_MEGAKERNEL, flags)
+        aopts = AdaptiveOpts(min_spp, step_spp, rel_noise, abs_noise)
+        st = Stats()
+        _check(lib().b200rt_render_adaptive(self._h, cam.ctypes.data, C.byref(opts), C.byref(aopts), mean.ctypes.data,
+                                            m2.ctypes.data, spp.ctypes.data, C.byref(st)))
+        return mean, m2, spp, st.as_dict()
 
     def bounds_violations(self) -> np.ndarray:
         """[stack, node index, primitive / material index, pixel] violations counted by a -DB200RT_DEBUG_BOUNDS build."""

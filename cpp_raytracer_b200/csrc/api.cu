@@ -94,6 +94,8 @@ struct SceneImpl {
     cudaEvent_t ev_tail = nullptr;   // the tail scratch is free again (renders of one scene share it)
     void *d_tail = nullptr;          // chunked tail tiles of the path kernel: partial sums and arrival counters, zero between launches
     size_t tail_bytes = 0;
+    void *d_adapt = nullptr;         // adaptive sampling: int64 planes, counts, masks and tile lists (AdaptiveBuffers)
+    size_t adapt_bytes = 0;
     int sm_count = 148;
 };
 
@@ -254,6 +256,7 @@ void free_scene(SceneImpl *s) {
     dev_free(s->d_t);
     dev_free(s->d_pool);
     dev_free(s->d_tail);
+    dev_free(s->d_adapt);
     if (s->ev0) cudaEventDestroy(s->ev0);
     if (s->ev1) cudaEventDestroy(s->ev1);
     if (s->ev_pool) cudaEventDestroy(s->ev_pool);
@@ -296,6 +299,10 @@ int fill_camera(const B200rtCamera *cam, CameraParams &C) {
     return B200RT_OK;
 }
 
+uint32_t image_tiles(const CameraParams &C) {
+    return ((C.w + (uint32_t)kPathTileW - 1u) / (uint32_t)kPathTileW) * ((C.h + (uint32_t)kPathTileH - 1u) / (uint32_t)kPathTileH);
+}
+
 // Resolves the sample range of a render call: count 0 means camera.spp unless B200RT_FLAG_EXACT_COUNT is set.
 int sample_range_of(const B200rtCamera *cam, const B200rtRenderOpts &o, uint64_t *count_out) {
     const uint64_t count = (o.sample_count || (o.flags & B200RT_FLAG_EXACT_COUNT)) ? o.sample_count : cam->spp;
@@ -314,7 +321,7 @@ struct TailPlan {
     uint32_t tiles = 0, chunks = 8, min_chunk = 8;
     bool forced = false;
 };
-int plan_tail(SceneImpl *s, const CameraParams &C, bool count, bool leaf_first, bool moments, TailPlan *t) {
+int plan_tail(SceneImpl *s, const CameraParams &C, bool count, bool leaf_first, bool moments, TailPlan *t, bool adaptive = false) {
     const uint32_t tiles = ((C.w + (uint32_t)kPathTileW - 1u) / (uint32_t)kPathTileW) * ((C.h + (uint32_t)kPathTileH - 1u) / (uint32_t)kPathTileH);
     if (const char *e = std::getenv("B200RT_TAIL_TILES")) {
         long long r = 0, k = 0;
@@ -325,7 +332,7 @@ int plan_tail(SceneImpl *s, const CameraParams &C, bool count, bool leaf_first, 
         return B200RT_OK;
     }
     int resident = 0;
-    if (cudaError_t e = path_resident_blocks(s->stack, count, leaf_first, moments, s->sm_count, &resident); e != cudaSuccess) {
+    if (cudaError_t e = path_resident_blocks(s->stack, count, leaf_first, moments, s->sm_count, &resident, adaptive); e != cudaSuccess) {
         cudaGetLastError();
         return fail(B200RT_ECUDA, std::string("path kernel occupancy: ") + cudaGetErrorString(e));
     }
@@ -351,15 +358,14 @@ cudaError_t tail_scratch(SceneImpl *s, uint32_t tail_tiles, bool moments, cudaSt
 
 // One launch's chunking of its tail tiles: the chunk is a multiple of 2^group_shift samples (so same-pixel item groups
 // stay whole and chunks partition the tile's items, kernels.cu block_items).  A launch whose samples make one chunk keeps
-// whole tiles, unless the chunk count was forced.
-void chunk_tail(const TailPlan &t, RenderParams &Q) {
+// whole tiles, unless the chunk count was forced.  `tiles`: the tiles the launch renders (the last of them are chunked).
+void chunk_tail(const TailPlan &t, uint32_t tiles, RenderParams &Q) {
     const uint32_t n = Q.sample_count, group = 1u << Q.group_shift;
     uint32_t chunk = std::max(t.min_chunk, (uint32_t)(((uint64_t)n + t.chunks - 1) / t.chunks));
     chunk = (uint32_t)(((uint64_t)chunk + group - 1) / group * group);
     const uint32_t k = (uint32_t)(((uint64_t)n + chunk - 1) / chunk);
     if (k <= 1 && !t.forced) return;
-    const uint32_t tiles = ((Q.cam.w + (uint32_t)kPathTileW - 1u) / (uint32_t)kPathTileW) * ((Q.cam.h + (uint32_t)kPathTileH - 1u) / (uint32_t)kPathTileH);
-    Q.tail_first = tiles - t.tiles;
+    Q.tail_first = tiles - std::min(t.tiles, tiles);
     Q.tail_chunks = k;
     Q.tail_chunk_samples = chunk;
 }
@@ -435,7 +441,7 @@ int render_on_device(SceneImpl *s, const B200rtCamera *cam, const B200rtRenderOp
             Q.sample_begin = (uint32_t)(o.sample_offset + done);
             Q.sample_count = (uint32_t)std::min<uint64_t>(per_launch, count - done);
             if (done) Q.flags |= kRenderAccumulate;
-            if (tail.tiles) chunk_tail(tail, Q);
+            if (tail.tiles) chunk_tail(tail, image_tiles(P.cam), Q);
             CUDA_TRY(launch_path_megakernel(s->stack, Q, count_flag, leaf_first, st, d_m2 != nullptr));
             ++launches;
         }
@@ -797,6 +803,154 @@ int render_host(void *scene, const B200rtCamera *cam, const B200rtRenderOpts *op
     return B200RT_OK;
 }
 
+// The scene's adaptive-sampling state for one image, carved out of s->d_adapt (grown on first use, like d_frame):
+// per pixel 6 int64 sums and a count, per tile two 256-bit masks (active, unconverged) and two tile lists, and the
+// two totals the host reads after each pass.
+struct AdaptiveBuffers {
+    long long *planes;
+    uint32_t *counts, *mask, *unconv, *list_a, *list_b, *totals;
+};
+size_t adaptive_layout(char *base, size_t pixels, size_t tiles, AdaptiveBuffers *b) {
+    size_t off = 0;
+    auto take = [&](size_t bytes) { char *p = base ? base + off : nullptr; off += (bytes + 255) / 256 * 256; return p; };
+    b->planes = reinterpret_cast<long long *>(take(pixels * kAdaptivePlanes * sizeof(long long)));
+    b->counts = reinterpret_cast<uint32_t *>(take(pixels * sizeof(uint32_t)));
+    b->mask = reinterpret_cast<uint32_t *>(take(tiles * kAdaptiveMaskWords * sizeof(uint32_t)));
+    b->unconv = reinterpret_cast<uint32_t *>(take(tiles * kAdaptiveMaskWords * sizeof(uint32_t)));
+    b->list_a = reinterpret_cast<uint32_t *>(take(tiles * sizeof(uint32_t)));
+    b->list_b = reinterpret_cast<uint32_t *>(take(tiles * sizeof(uint32_t)));
+    b->totals = reinterpret_cast<uint32_t *>(take(2 * sizeof(uint32_t)));
+    return off;
+}
+
+// b200rt_render_adaptive on a single-device scene.  Pass 1 renders min(min_spp, max) samples of every pixel; each later
+// pass renders the next min(step_spp, max - n) samples of the pixels still active, all of which have n samples.  Between
+// passes two kernels judge the pass's pixels and dilate the result into the next active set and tile list; the host reads
+// the next pass's tile and pixel counts, which size its grid or end the loop.
+int render_adaptive_host(void *scene, const B200rtCamera *cam, const B200rtRenderOpts *opts, const B200rtAdaptiveOpts *aopts,
+                         float *out_rgb, float *out_m2, uint32_t *out_spp, B200rtStats *stats) {
+    if (as_multi(scene)) return fail(B200RT_EINVAL, "b200rt_render_adaptive takes a single-device scene");
+    SceneImpl *s = as_scene(scene);
+    if (!s) return fail(B200RT_EINVAL, "bad scene handle");
+    if (!cam || !aopts || !out_rgb) return fail(B200RT_EINVAL, "camera, adaptive options or output pointer is NULL");
+    RenderParams P{};
+    if (int rc = fill_camera(cam, P.cam)) return rc;
+    B200rtRenderOpts o{};
+    if (opts) o = *opts;
+    o.flags &= ~(uint32_t)B200RT_FLAG_ACCUMULATE;   // host entry always overwrites
+    uint64_t max_spp = 0;
+    if (int rc = sample_range_of(cam, o, &max_spp)) return rc;
+    if (o.variant == B200RT_VARIANT_WAVEFRONT || (o.flags & (B200RT_FLAG_THREAD_PIXELS | B200RT_FLAG_COUNTERS)))
+        return fail(B200RT_EINVAL, "adaptive renders use the default kernel only: no wavefront variant, B200RT_FLAG_THREAD_PIXELS or B200RT_FLAG_COUNTERS");
+    const B200rtAdaptiveOpts a = *aopts;
+    if (a.min_spp < 2 || a.step_spp == 0) return fail(B200RT_EINVAL, "adaptive options need min_spp >= 2 and step_spp >= 1");
+    if (max_spp > kMaxSamplesPerLaunchMoments) return fail(B200RT_EINVAL, "an adaptive render takes at most 2^16 samples per pixel");
+    if (!std::isfinite(a.rel_noise) || !std::isfinite(a.abs_noise) || a.rel_noise < 0 || a.abs_noise < 0)
+        return fail(B200RT_EINVAL, "rel_noise and abs_noise must be finite and >= 0");
+    std::lock_guard<std::mutex> lk(s->mu);
+    DeviceGuard g(s->device);
+    const double t0 = now_ms();
+    const cudaStream_t st = 0;
+    const size_t pixels = (size_t)cam->image_w * cam->image_h, floats = pixels * 3;
+    const uint32_t tiles = image_tiles(P.cam);
+    if (2 * floats > s->frame_floats) {
+        if (s->d_frame) { dev_free(s->d_frame); s->d_frame = nullptr; s->frame_floats = 0; }
+        CUDA_TRY(dev_alloc(&s->d_frame, 2 * floats * sizeof(float)));
+        s->frame_floats = 2 * floats;
+    }
+    AdaptiveBuffers b{};
+    const size_t bytes = adaptive_layout(nullptr, pixels, tiles, &b);
+    if (bytes > s->adapt_bytes) {
+        if (s->d_adapt) { dev_free(s->d_adapt); s->d_adapt = nullptr; s->adapt_bytes = 0; }
+        CUDA_TRY(dev_alloc(&s->d_adapt, bytes));
+        s->adapt_bytes = bytes;
+    }
+    adaptive_layout(static_cast<char *>(s->d_adapt), pixels, tiles, &b);
+
+    P.scene = s->d;
+    P.seed = o.seed;
+    P.flags = o.flags;
+    P.counters = s->d_counters;
+    P.group_shift = (cam->background[0] == 0.0 && cam->background[1] == 0.0 && cam->background[2] == 0.0) ? 3u : 0u;   // as render_on_device
+    if (const char *gs = std::getenv("B200RT_GROUP_SHIFT")) P.group_shift = (uint32_t)std::min(5, std::max(0, std::atoi(gs)));
+    P.ad_mask = b.mask;
+    P.ad_planes = b.planes;
+    bool leaf_first = s->info.n_quads > s->info.n_spheres;
+    if (const char *lf = std::getenv("B200RT_LEAF_FIRST")) leaf_first = lf[0] == '1';
+    TailPlan tail;
+    if (int rc = plan_tail(s, P.cam, false, leaf_first, true, &tail, true)) return rc;
+    tail.tiles = std::min(tail.tiles, tiles);
+
+    AdaptiveState A{};
+    A.w = P.cam.w; A.h = P.cam.h;
+    A.list = b.list_a; A.next_list = b.list_b;
+    A.mask = b.mask; A.unconv = b.unconv; A.planes = b.planes; A.counts = b.counts; A.totals = b.totals;
+    A.rel_noise = a.rel_noise; A.abs_noise = a.abs_noise;
+
+    CUDA_TRY(cudaMemsetAsync(s->d_counters, 0, 4 * sizeof(unsigned long long), st));
+    CUDA_TRY(cudaEventRecord(s->ev0, st));
+    if (tail.tiles) CUDA_TRY(tail_scratch(s, tail.tiles, true, st, &P));
+    CUDA_TRY(cudaMemsetAsync(b.planes, 0, pixels * kAdaptivePlanes * sizeof(long long), st));
+    CUDA_TRY(cudaMemsetAsync(b.counts, 0, pixels * sizeof(uint32_t), st));
+    CUDA_TRY(launch_adaptive_init(A, tiles, st));
+    unsigned long long launches = 1, paths = 0;
+    uint64_t n = 0, active_pixels = pixels;
+    uint32_t n_list = tiles;
+    while (n < max_spp) {
+        const uint64_t k = n == 0 ? std::min<uint64_t>(a.min_spp, max_spp) : std::min<uint64_t>(a.step_spp, max_spp - n);
+        RenderParams Q = P;
+        Q.sample_begin = (uint32_t)(o.sample_offset + n);
+        Q.sample_count = (uint32_t)k;
+        Q.ad_list = A.list;
+        Q.ad_n_list = n_list;
+        if (tail.tiles) chunk_tail(tail, n_list, Q);
+        CUDA_TRY(launch_path_adaptive(s->stack, Q, leaf_first, st));
+        paths += active_pixels * k;
+        n += k;
+        A.n_list = n_list;
+        CUDA_TRY(launch_adaptive_judge(A, (uint32_t)n, n < max_spp, s->d, st));
+        launches += 2;
+        if (n == max_spp) break;
+        CUDA_TRY(cudaMemsetAsync(b.totals, 0, 2 * sizeof(uint32_t), st));
+        CUDA_TRY(launch_adaptive_decide(A, s->d, st));
+        ++launches;
+        uint32_t next[2];
+        CUDA_TRY(cudaMemcpyAsync(next, b.totals, sizeof next, cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaStreamSynchronize(st));
+        if (next[0] == 0) break;
+        std::swap(A.list, A.next_list);
+        n_list = next[0];
+        active_pixels = next[1];
+    }
+    CUDA_TRY(launch_adaptive_finish(A, (o.flags & B200RT_FLAG_SUM) != 0, s->d_frame, s->d_frame + floats, st));
+    ++launches;
+    if (tail.tiles) CUDA_TRY(cudaEventRecord(s->ev_tail, st));
+    CUDA_TRY(cudaEventRecord(s->ev1, st));
+    unsigned long long c[4];
+    CUDA_TRY(cudaMemcpyAsync(c, s->d_counters, sizeof c, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    const double t1 = now_ms();
+    CUDA_TRY(staged_download(out_rgb, s->d_frame, floats * sizeof(float), st));
+    if (out_m2) CUDA_TRY(staged_download(out_m2, s->d_frame + floats, floats * sizeof(float), st));
+    if (out_spp) CUDA_TRY(staged_download(out_spp, b.counts, pixels * sizeof(uint32_t), st));
+    const double t2 = now_ms();
+    if (stats) {
+        B200rtStats local{};
+        float ms = 0;
+        CUDA_TRY(cudaEventElapsedTime(&ms, s->ev0, s->ev1));
+        local.kernel_ms = ms;
+        local.paths = paths;
+        local.rays = c[0];
+        local.kernel_launches = launches;
+        local.n_devices = 1;
+        local.d2h_ms = t2 - t1;
+        local.d2h_bytes = (floats * ((out_m2 ? 2 : 1)) + (out_spp ? pixels : 0)) * sizeof(float);
+        local.total_ms = t2 - t0;
+        *stats = local;
+    }
+    return B200RT_OK;
+}
+
 }  // namespace
 
 // ==========================================================================================
@@ -1123,6 +1277,11 @@ int b200rt_render_moments(void *scene, const B200rtCamera *cam, const B200rtRend
                           B200rtStats *stats) {
     if (!cam || !out_rgb || !out_m2) return fail(B200RT_EINVAL, "camera or output pointer is NULL");
     return render_host(scene, cam, opts, out_rgb, out_m2, stats);
+}
+
+int b200rt_render_adaptive(void *scene, const B200rtCamera *cam, const B200rtRenderOpts *opts, const B200rtAdaptiveOpts *aopts,
+                           float *out_rgb, float *out_m2_or_null, uint32_t *out_spp_or_null, B200rtStats *stats) {
+    return render_adaptive_host(scene, cam, opts, aopts, out_rgb, out_m2_or_null, out_spp_or_null, stats);
 }
 
 int b200rt_render_scene_multi(const B200rtSceneDesc *desc, const B200rtCamera *cam, const B200rtRenderOpts *opts,

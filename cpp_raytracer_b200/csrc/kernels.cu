@@ -211,8 +211,15 @@ struct TilePool {
 struct TilePoolMoments : TilePool {
     long long acc2[kPathBlock * 3];    // per tile pixel: sum of radiance^2 x 2^24
 };
-template <bool MOMENTS>
-using TilePoolOf = std::conditional_t<MOMENTS, TilePoolMoments, TilePool>;
+// The adaptive instantiation's pool: the moments pool, plus the tile pixels the block renders.  Its items and its
+// accumulators are numbered over that list instead of over the tile's valid pixels.
+struct TilePoolAdaptive : TilePoolMoments {
+    unsigned char act[kPathBlock];     // active tile pixels, ascending
+    unsigned int warp_act[kAdaptiveMaskWords];
+};
+static_assert(kPathBlock <= 256, "TilePoolAdaptive::act holds tile pixels in bytes");
+template <bool MOMENTS, bool ADAPTIVE = false>
+using TilePoolOf = std::conditional_t<ADAPTIVE, TilePoolAdaptive, std::conditional_t<MOMENTS, TilePoolMoments, TilePool>>;
 constexpr float kFixScale = 1073741824.0f;            // 2^30
 constexpr double kFixInv = 1.0 / 1073741824.0;
 constexpr float kFix2Scale = 16777216.0f;             // 2^24
@@ -297,7 +304,9 @@ __device__ __forceinline__ void pool_contribute(TilePoolOf<MOMENTS> &tp, uint32_
 // C4b +15 %, C5 +5 % -- when the background is black.  With a bright background every escaping path adds to its pixel's
 // accumulator and lanes on the same pixel serialise on it (C1 -3 %; warp-aggregating the sums first costs more than it
 // saves), so the host picks g = 3 for a black background and 0 otherwise (profiles/r2_tile_shape.md).  The image is the same
-// bit for bit under every order.  The items run from pool_init's start to total_items (block_items).
+// bit for bit under every order.  The items run from pool_init's start to total_items (block_items).  ADAPTIVE: L.lp
+// numbers the block's active pixels (tm.n_valid of them); tp.act maps it to the tile pixel.
+template <bool ADAPTIVE = false>
 __device__ __forceinline__ bool pool_fetch(const RenderParams &P, const TileMap &tm, TilePool &tp, uint32_t total_items, PoolLane &L,
                                            uint32_t &px, uint32_t &py) {
     if (total_items == 0u) return false;
@@ -318,8 +327,10 @@ __device__ __forceinline__ bool pool_fetch(const RenderParams &P, const TileMap 
             if (L.s < P.sample_count) break;                                      // ragged last block of samples
         }
     }
-    const uint32_t lx = tm.vw == (uint32_t)kPathTileW ? L.lp % (uint32_t)kPathTileW : L.lp % tm.vw;
-    const uint32_t ly = tm.vw == (uint32_t)kPathTileW ? L.lp / (uint32_t)kPathTileW : L.lp / tm.vw;
+    uint32_t lt = L.lp;
+    if constexpr (ADAPTIVE) lt = static_cast<TilePoolAdaptive &>(tp).act[L.lp];
+    const uint32_t lx = tm.vw == (uint32_t)kPathTileW ? lt % (uint32_t)kPathTileW : lt % tm.vw;
+    const uint32_t ly = tm.vw == (uint32_t)kPathTileW ? lt / (uint32_t)kPathTileW : lt / tm.vw;
     px = tm.x0 + lx;
     py = tm.y0 + ly;
     L.pixel = py * P.cam.w + px;
@@ -328,8 +339,8 @@ __device__ __forceinline__ bool pool_fetch(const RenderParams &P, const TileMap 
 }
 
 // shade_and_advance with the tile pool: same path semantics, same Philox keys (pixel, sample, bounce).
-template <bool MOMENTS = false>
-__device__ __forceinline__ bool pool_shade_and_advance(const RenderParams &P, const TileMap &tm, TilePoolOf<MOMENTS> &tp,
+template <bool MOMENTS = false, bool ADAPTIVE = false>
+__device__ __forceinline__ bool pool_shade_and_advance(const RenderParams &P, const TileMap &tm, TilePoolOf<MOMENTS, ADAPTIVE> &tp,
                                                        uint32_t total_items, const Hit &best, PoolLane &L, Ray &ray) {
     const CameraParams &C = P.cam;
     const uint32_t k0 = (uint32_t)P.seed, k1 = (uint32_t)(P.seed >> 32);
@@ -351,7 +362,7 @@ __device__ __forceinline__ bool pool_shade_and_advance(const RenderParams &P, co
     }
     if (!L.has_path) {
         uint32_t px, py;
-        if (!pool_fetch(P, tm, tp, total_items, L, px, py)) return false;
+        if (!pool_fetch<ADAPTIVE>(P, tm, tp, total_items, L, px, py)) return false;
         const Philox4 rnd = philox4x32_10(L.pixel, P.sample_begin + L.s, 0u, 0u, k0, k1);
         camera_ray(C, px, py, rnd, ray, L.p);
         L.has_path = true;
@@ -389,16 +400,37 @@ __device__ __forceinline__ void store_tile_pixel(const RenderParams &P, const Ti
     }
 }
 
+// ADAPTIVE: active pixel lp's sums of this pass are added to its int64 planes.  A pixel has one writer per pass (the
+// block of a whole tile, or the last chunk of a tail tile to arrive), so a plain add is exact; the conversion to floats
+// happens once, after the last pass (adaptive_finish_kernel), with the expression store_tile_pixel uses.
+__device__ __forceinline__ void add_tile_pixel(const RenderParams &P, const TileMap &tm, const TilePoolAdaptive &tp, uint32_t lp,
+                                               const long long (&a)[3], const long long (&q)[3]) {
+    const uint32_t lt = tp.act[lp];
+    const uint32_t pixel = (tm.y0 + lt / tm.vw) * P.cam.w + tm.x0 + lt % tm.vw;
+    if (B200RT_CHECK(P.scene, lt < kPathBlock && pixel < P.cam.w * P.cam.h, 3)) {
+        long long *o = P.ad_planes + (size_t)pixel * kAdaptivePlanes;
+        o[0] += a[0]; o[1] += a[1]; o[2] += a[2];
+        o[3] += q[0]; o[4] += q[1]; o[5] += q[2];
+    }
+}
+
+template <bool MOMENTS, bool ADAPTIVE>
+__device__ __forceinline__ void finish_tile_pixel(const RenderParams &P, const TileMap &tm, const TilePoolOf<MOMENTS, ADAPTIVE> &tp,
+                                                  uint32_t lp, const long long (&a)[3], const long long (&q)[3]) {
+    if constexpr (ADAPTIVE) add_tile_pixel(P, tm, tp, lp, a, q);
+    else store_tile_pixel<MOMENTS>(P, tm, lp, a, q);
+}
+
 // After the block's last path: thread t writes tile pixel t.
-template <bool MOMENTS = false>
-__device__ __forceinline__ void pool_write_tile(const RenderParams &P, const TileMap &tm, TilePoolOf<MOMENTS> &tp) {
+template <bool MOMENTS = false, bool ADAPTIVE = false>
+__device__ __forceinline__ void pool_write_tile(const RenderParams &P, const TileMap &tm, TilePoolOf<MOMENTS, ADAPTIVE> &tp) {
     __syncthreads();
     const uint32_t lp = threadIdx.x;
     if (lp < tm.n_valid) {
         const long long a[3] = {tp.acc[lp * 3 + 0], tp.acc[lp * 3 + 1], tp.acc[lp * 3 + 2]};
         long long q[3] = {0, 0, 0};
         if constexpr (MOMENTS) { q[0] = tp.acc2[lp * 3 + 0]; q[1] = tp.acc2[lp * 3 + 1]; q[2] = tp.acc2[lp * 3 + 2]; }
-        store_tile_pixel<MOMENTS>(P, tm, lp, a, q);
+        finish_tile_pixel<MOMENTS, ADAPTIVE>(P, tm, tp, lp, a, q);
     }
 }
 
@@ -406,8 +438,8 @@ __device__ __forceinline__ void pool_write_tile(const RenderParams &P, const Til
 // total does not depend on how the samples were split or in which order the chunks finish), then count the block in.
 // The chunk that arrives last takes the totals -- leaving the slot and its counter zero for the next launch -- and writes
 // the pixels exactly as pool_write_tile does.  No block waits for another.
-template <bool MOMENTS = false>
-__device__ __forceinline__ void pool_merge_chunk(const RenderParams &P, const TileMap &tm, TilePoolOf<MOMENTS> &tp, uint32_t slot) {
+template <bool MOMENTS = false, bool ADAPTIVE = false>
+__device__ __forceinline__ void pool_merge_chunk(const RenderParams &P, const TileMap &tm, TilePoolOf<MOMENTS, ADAPTIVE> &tp, uint32_t slot) {
     constexpr uint32_t kPlane = (uint32_t)kPathBlock * 3u;
     unsigned long long *part = reinterpret_cast<unsigned long long *>(P.tail_acc) + (size_t)slot * kPlane * (MOMENTS ? 2u : 1u);
     for (uint32_t i = threadIdx.x; i < kPlane; i += kPathBlock) {
@@ -428,7 +460,7 @@ __device__ __forceinline__ void pool_merge_chunk(const RenderParams &P, const Ti
         if constexpr (MOMENTS) q[c] = (long long)atomicExch(&part[kPlane + lp * 3 + c], 0ull);
     }
     if (lp == 0) P.tail_arrivals[slot] = 0u;
-    if (lp < tm.n_valid) store_tile_pixel<MOMENTS>(P, tm, lp, a, q);
+    if (lp < tm.n_valid) finish_tile_pixel<MOMENTS, ADAPTIVE>(P, tm, tp, lp, a, q);
 }
 
 __device__ __forceinline__ void write_counters(const RenderParams &P, uint32_t lane_rays, bool count, const TraversalCounters &ctr) {
@@ -470,17 +502,55 @@ cudaError_t set_block_times(unsigned long long *buf, uint32_t n_blocks) {
 }
 #endif
 
+__device__ __forceinline__ uint32_t image_tiles(const CameraParams &C) {
+    return ((C.w + (uint32_t)kPathTileW - 1u) / (uint32_t)kPathTileW) * ((C.h + (uint32_t)kPathTileH - 1u) / (uint32_t)kPathTileH);
+}
+
+// Start of an ADAPTIVE block: the tile of list entry `entry`, and its active pixels (its mask bits) in ascending tile-pixel
+// order in tp.act.  Returns the tile's map with n_valid = the number of active pixels, so that block_items and pool_fetch
+// number the items over them exactly as they number a whole tile's pixels.
+__device__ __forceinline__ TileMap adaptive_tile(const RenderParams &P, uint32_t entry, TilePoolAdaptive &tp) {
+    uint32_t tile = 0;
+    bool ok = B200RT_CHECK(P.scene, entry < P.ad_n_list, 3);
+    if (ok) {
+        tile = P.ad_list[entry];
+        ok = B200RT_CHECK(P.scene, tile < image_tiles(P.cam), 3);
+    }
+    TileMap tm = map_tile(P.cam, ok ? tile : 0u);
+    const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31u, base = warp * 32u;
+    const uint32_t valid = tm.n_valid >= base + 32u ? 0xFFFFFFFFu : (tm.n_valid > base ? (1u << (tm.n_valid - base)) - 1u : 0u);
+    uint32_t word = ok ? P.ad_mask[(size_t)tile * kAdaptiveMaskWords + warp] : 0u;
+    if (!B200RT_CHECK(P.scene, (word & ~valid) == 0u, 3)) word &= valid;
+    if (lane == 0) tp.warp_act[warp] = __popc(word);
+    __syncthreads();
+    uint32_t before = 0, total = 0;
+#pragma unroll
+    for (uint32_t k = 0; k < (uint32_t)kAdaptiveMaskWords; ++k) {
+        const uint32_t c = tp.warp_act[k];
+        before += k < warp ? c : 0u;
+        total += c;
+    }
+    if ((word >> lane) & 1u) tp.act[before + __popc(word & ((1u << lane) - 1u))] = (unsigned char)threadIdx.x;
+    tm.n_valid = total;
+    return tm;
+}
+
 // path_megakernel_pool (variant 0, default): every lane runs traverse-then-shade in a loop and takes the tile's next
 // (pixel, sample) item as soon as its path ends.  MOMENTS: also the per-pixel sum of x^2 into P.out_m2 (b200rt_render_moments).
-template <int STACK, bool COUNT, bool LEAF_FIRST = false, int MINB = kPathMinBlocks, bool MOMENTS = false>
+// ADAPTIVE (implies MOMENTS; b200rt_render_adaptive): a block renders the active pixels of an entry of P.ad_list and adds
+// both sums into P.ad_planes; the host sets sample_begin to the pass's first sample, so the Philox keys are unchanged.
+template <int STACK, bool COUNT, bool LEAF_FIRST = false, int MINB = kPathMinBlocks, bool MOMENTS = false, bool ADAPTIVE = false>
 __global__ void __launch_bounds__(kPathBlock, MINB) path_megakernel_pool(const __grid_constant__ RenderParams P) {
-    __shared__ TilePoolOf<MOMENTS> tp;
+    static_assert(!ADAPTIVE || MOMENTS, "the adaptive kernel sums x^2");
+    __shared__ TilePoolOf<MOMENTS, ADAPTIVE> tp;
 #ifdef B200RT_BLOCK_TIMES
     const unsigned long long t_start = globaltimer_ns();
 #endif
     const CameraParams &C = P.cam;
     const BlockWork w = block_work(P);
-    const TileMap tm = map_tile(C, w.tile);
+    TileMap tm;
+    if constexpr (ADAPTIVE) tm = adaptive_tile(P, w.tile, tp);
+    else tm = map_tile(C, w.tile);
     uint32_t first_item;
     const uint32_t total_items = block_items(P, tm, w, first_item);
     pool_init<MOMENTS>(tp, first_item, w.slot);
@@ -488,15 +558,15 @@ __global__ void __launch_bounds__(kPathBlock, MINB) path_megakernel_pool(const _
     Ray ray;
     TraversalCounters ctr;
     Hit best{0.0, kNoHit};
-    while (pool_shade_and_advance<MOMENTS>(P, tm, tp, total_items, best, L, ray)) {
+    while (pool_shade_and_advance<MOMENTS, ADAPTIVE>(P, tm, tp, total_items, best, L, ray)) {
         // world.hit_by(ray, Interval::with_min(0.00001))  (camera.h:217)
         best = closest_hit<STACK, COUNT, LEAF_FIRST>(P.scene, ray.ox, ray.oy, ray.oz, ray.dx, ray.dy, ray.dz, 0.00001,
                                                   __longlong_as_double(0x7ff0000000000000LL), &ctr);
     }
     __syncthreads();
     const uint32_t slot = tp.slot;
-    if (slot == kWholeTile) pool_write_tile<MOMENTS>(P, tm, tp);
-    else pool_merge_chunk<MOMENTS>(P, tm, tp, slot);
+    if (slot == kWholeTile) pool_write_tile<MOMENTS, ADAPTIVE>(P, tm, tp);
+    else pool_merge_chunk<MOMENTS, ADAPTIVE>(P, tm, tp, slot);
     write_counters(P, L.rays, COUNT, ctr);
 #ifdef B200RT_BLOCK_TIMES
     record_block_time(t_start);
@@ -793,14 +863,166 @@ cudaError_t launch_path_megakernel(int stack, const RenderParams &P, bool count,
     return launch_path_t<128>(P, count, leaf_first, st, moments);
 }
 
+template <int STACK>
+static cudaError_t launch_path_adaptive_t(const RenderParams &P, bool leaf_first, cudaStream_t st) {
+    if (P.ad_n_list == 0) return cudaSuccess;
+    const uint32_t blocks = P.tail_chunks ? P.tail_first + (P.ad_n_list - P.tail_first) * P.tail_chunks : P.ad_n_list;
+    if (leaf_first) path_megakernel_pool<STACK, false, true, kPathMinBlocks, true, true><<<blocks, kPathBlock, 0, st>>>(P);
+    else path_megakernel_pool<STACK, false, false, kPathMinBlocks, true, true><<<blocks, kPathBlock, 0, st>>>(P);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_path_adaptive(int stack, const RenderParams &P, bool leaf_first, cudaStream_t st) {
+    if (stack <= 32) return launch_path_adaptive_t<32>(P, leaf_first, st);
+    if (stack <= 64) return launch_path_adaptive_t<64>(P, leaf_first, st);
+    return launch_path_adaptive_t<128>(P, leaf_first, st);
+}
+
+// ------------------------------------------------------------------------------------------
+// Adaptive sampling between passes.  Every kernel below runs one block of kPathBlock threads per tile, thread t on tile
+// pixel t, so that warp k owns mask word k of the tile.
+__device__ __forceinline__ TileMap adaptive_map(const AdaptiveState &A, uint32_t tile) {
+    CameraParams C;
+    C.w = A.w;
+    C.h = A.h;
+    return map_tile(C, tile);
+}
+__device__ __forceinline__ uint32_t adaptive_tiles(const AdaptiveState &A) {
+    return ((A.w + (uint32_t)kPathTileW - 1u) / (uint32_t)kPathTileW) * ((A.h + (uint32_t)kPathTileH - 1u) / (uint32_t)kPathTileH);
+}
+
+__global__ void __launch_bounds__(kPathBlock) adaptive_init_kernel(const __grid_constant__ AdaptiveState A) {
+    const uint32_t tile = blockIdx.x, warp = threadIdx.x >> 5;
+    const TileMap tm = adaptive_map(A, tile);
+    const unsigned bits = __ballot_sync(0xFFFFFFFFu, threadIdx.x < tm.n_valid);
+    if ((threadIdx.x & 31u) == 0) {
+        A.mask[(size_t)tile * kAdaptiveMaskWords + warp] = bits;
+        A.unconv[(size_t)tile * kAdaptiveMaskWords + warp] = 0u;
+    }
+    if (threadIdx.x == 0) A.list[tile] = tile;
+}
+
+// Camera::sample_variance of one channel, from the mean-plane floats of x and x^2 over n >= 2 samples.
+__device__ __forceinline__ double channel_variance(float mean, float m2, uint32_t n) {
+    const double d = (double)m2 - (double)mean * (double)mean;
+    if (d <= ldexp((double)m2, -20) + 0x1p-24) return 0.0;
+    return (double)n / (double)(n - 1u) * d;
+}
+
+// The convergence rule (b200rt.h, b200rt_render_adaptive): the mean-plane floats exactly as store_tile_pixel writes them,
+// then err = sqrt(sum of the channel variances / 3n) against rel_noise x the mean of the three channel means + abs_noise.
+// In double; the library is built with -fmad=false, so nothing is contracted and the host can replay it bit for bit.
+__device__ __forceinline__ bool pixel_converged(const AdaptiveState &A, const long long *p, uint32_t n) {
+    const float inv = (float)(1.0 / (double)n);
+    double var = 0.0, level = 0.0;
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+        const float mean = (float)((double)p[c] * kFixInv) * inv;
+        const float m2 = (float)((double)p[3 + c] * kFix2Inv) * inv;
+        var += channel_variance(mean, m2, n);
+        level += (double)mean;
+    }
+    const double err = sqrt(var / (3.0 * (double)n));
+    return err <= A.rel_noise * (level / 3.0) + A.abs_noise;
+}
+
+// The pixels a pass rendered now have n samples; with judge, each one's unconverged bit is set from the rule.
+__global__ void __launch_bounds__(kPathBlock) adaptive_judge_kernel(const __grid_constant__ AdaptiveState A, uint32_t n, int judge,
+                                                                    const __grid_constant__ DeviceScene S) {
+    const uint32_t tile = A.list[blockIdx.x];
+    if (!B200RT_CHECK(S, tile < adaptive_tiles(A), 3)) return;
+    const TileMap tm = adaptive_map(A, tile);
+    const uint32_t lp = threadIdx.x, lane = lp & 31u;
+    const size_t mw = (size_t)tile * kAdaptiveMaskWords + (lp >> 5);
+    bool unconv = false;
+    if (((A.mask[mw] >> lane) & 1u) && B200RT_CHECK(S, lp < tm.n_valid, 3)) {
+        const uint32_t pixel = (tm.y0 + lp / tm.vw) * A.w + tm.x0 + lp % tm.vw;
+        A.counts[pixel] = n;
+        if (judge) unconv = !pixel_converged(A, A.planes + (size_t)pixel * kAdaptivePlanes, n);
+    }
+    const unsigned bits = __ballot_sync(0xFFFFFFFFu, unconv);
+    if (lane == 0) A.unconv[mw] = bits;
+}
+
+// A pixel of the pass stays active if any pixel of its 3 x 3 neighbourhood (clipped at the image edge) is unconverged.
+// A pixel that stopped earlier was converged when it stopped and its sums have not changed since, so only the pass's own
+// tiles can hold unconverged bits; every other tile's are zero.  Stopping is final: a pixel outside the mask stays out.
+__global__ void __launch_bounds__(kPathBlock) adaptive_decide_kernel(const __grid_constant__ AdaptiveState A,
+                                                                     const __grid_constant__ DeviceScene S) {
+    const uint32_t tile = A.list[blockIdx.x];
+    if (!B200RT_CHECK(S, tile < adaptive_tiles(A), 3)) return;
+    const TileMap tm = adaptive_map(A, tile);
+    const uint32_t lp = threadIdx.x, lane = lp & 31u;
+    const uint32_t tiles_x = (A.w + (uint32_t)kPathTileW - 1u) / (uint32_t)kPathTileW;
+    const size_t mw = (size_t)tile * kAdaptiveMaskWords + (lp >> 5);
+    bool keep = false;
+    if (((A.mask[mw] >> lane) & 1u) && lp < tm.n_valid) {
+        const int px = (int)(tm.x0 + lp % tm.vw), py = (int)(tm.y0 + lp / tm.vw);
+        for (int qy = max(py - 1, 0); qy <= min(py + 1, (int)A.h - 1); ++qy)
+            for (int qx = max(px - 1, 0); qx <= min(px + 1, (int)A.w - 1); ++qx) {
+                const uint32_t tq = (uint32_t)qy / (uint32_t)kPathTileH * tiles_x + (uint32_t)qx / (uint32_t)kPathTileW;
+                const TileMap tn = adaptive_map(A, tq);
+                const uint32_t lq = ((uint32_t)qy - tn.y0) * tn.vw + ((uint32_t)qx - tn.x0);
+                keep |= (A.unconv[(size_t)tq * kAdaptiveMaskWords + lq / 32u] >> (lq & 31u)) & 1u;
+            }
+    }
+    const unsigned bits = __ballot_sync(0xFFFFFFFFu, keep);
+    if (lane == 0) A.mask[mw] = bits;
+    const int n_keep = __syncthreads_count(keep);
+    if (threadIdx.x == 0 && n_keep) {
+        const uint32_t slot = atomicAdd(&A.totals[0], 1u);
+        if (B200RT_CHECK(S, slot < adaptive_tiles(A), 3)) A.next_list[slot] = tile;
+        atomicAdd(&A.totals[1], (uint32_t)n_keep);
+    }
+}
+
+// planes / counts -> the output floats: store_tile_pixel's expression with the pixel's own count (k = 1 for sums).
+__global__ void adaptive_finish_kernel(const __grid_constant__ AdaptiveState A, int sum, float *__restrict__ out_rgb,
+                                       float *__restrict__ out_m2) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (long long)A.w * A.h) return;
+    const uint32_t n = A.counts[i];
+    const float k = sum || n == 0 ? 1.0f : (float)(1.0 / (double)n);
+    const long long *p = A.planes + i * kAdaptivePlanes;
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+        out_rgb[i * 3 + c] = (float)((double)p[c] * kFixInv) * k;
+        out_m2[i * 3 + c] = (float)((double)p[3 + c] * kFix2Inv) * k;
+    }
+}
+
+cudaError_t launch_adaptive_init(const AdaptiveState &A, uint32_t tiles, cudaStream_t st) {
+    if (tiles == 0) return cudaSuccess;
+    adaptive_init_kernel<<<tiles, kPathBlock, 0, st>>>(A);
+    return cudaGetLastError();
+}
+cudaError_t launch_adaptive_judge(const AdaptiveState &A, uint32_t n, bool judge, const DeviceScene &S, cudaStream_t st) {
+    if (A.n_list == 0) return cudaSuccess;
+    adaptive_judge_kernel<<<A.n_list, kPathBlock, 0, st>>>(A, n, judge ? 1 : 0, S);
+    return cudaGetLastError();
+}
+cudaError_t launch_adaptive_decide(const AdaptiveState &A, const DeviceScene &S, cudaStream_t st) {
+    if (A.n_list == 0) return cudaSuccess;
+    adaptive_decide_kernel<<<A.n_list, kPathBlock, 0, st>>>(A, S);
+    return cudaGetLastError();
+}
+cudaError_t launch_adaptive_finish(const AdaptiveState &A, bool sum, float *out_rgb, float *out_m2, cudaStream_t st) {
+    const long long n = (long long)A.w * A.h;
+    if (n == 0) return cudaSuccess;
+    adaptive_finish_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(A, sum ? 1 : 0, out_rgb, out_m2);
+    return cudaGetLastError();
+}
+
 size_t tail_scratch_bytes(uint32_t tail_tiles, bool moments) {
     return (size_t)tail_tiles * ((size_t)kPathBlock * 3 * sizeof(long long) * (moments ? 2 : 1) + sizeof(uint32_t));
 }
 
 template <int STACK>
-static cudaError_t path_blocks_per_sm(bool count, bool leaf_first, bool moments, int &n) {
+static cudaError_t path_blocks_per_sm(bool count, bool leaf_first, bool moments, bool adaptive, int &n) {
     cudaError_t e;
-    if (moments) e = leaf_first ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, path_megakernel_pool<STACK, false, true, kPathMinBlocks, true>, kPathBlock, 0)
+    if (adaptive) e = leaf_first ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, path_megakernel_pool<STACK, false, true, kPathMinBlocks, true, true>, kPathBlock, 0)
+                                 : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, path_megakernel_pool<STACK, false, false, kPathMinBlocks, true, true>, kPathBlock, 0);
+    else if (moments) e = leaf_first ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, path_megakernel_pool<STACK, false, true, kPathMinBlocks, true>, kPathBlock, 0)
                                 : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, path_megakernel_pool<STACK, false, false, kPathMinBlocks, true>, kPathBlock, 0);
     else if (leaf_first) e = count ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, path_megakernel_pool<STACK, true, true>, kPathBlock, 0)
                                    : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, path_megakernel_pool<STACK, false, true>, kPathBlock, 0);
@@ -809,11 +1031,11 @@ static cudaError_t path_blocks_per_sm(bool count, bool leaf_first, bool moments,
     return e;
 }
 
-cudaError_t path_resident_blocks(int stack, bool count, bool leaf_first, bool moments, int sm_count, int *blocks) {
+cudaError_t path_resident_blocks(int stack, bool count, bool leaf_first, bool moments, int sm_count, int *blocks, bool adaptive) {
     int n = 0;
-    const cudaError_t e = stack <= 32   ? path_blocks_per_sm<32>(count, leaf_first, moments, n)
-                          : stack <= 64 ? path_blocks_per_sm<64>(count, leaf_first, moments, n)
-                                        : path_blocks_per_sm<128>(count, leaf_first, moments, n);
+    const cudaError_t e = stack <= 32   ? path_blocks_per_sm<32>(count, leaf_first, moments, adaptive, n)
+                          : stack <= 64 ? path_blocks_per_sm<64>(count, leaf_first, moments, adaptive, n)
+                                        : path_blocks_per_sm<128>(count, leaf_first, moments, adaptive, n);
     *blocks = n * sm_count;
     return e;
 }

@@ -53,11 +53,46 @@ struct RenderParams {
     uint32_t tail_first, tail_chunks, tail_chunk_samples;
     long long *tail_acc;               // per tail tile: kPathBlock x 3 sums (x 2 with moments), zero between launches
     uint32_t *tail_arrivals;           // per tail tile: chunk blocks done, zero between launches
+    // Adaptive launches only (b200rt_render_adaptive): block b renders tile ad_list[b] (its tail chunks: the entries from
+    // tail_first on), only the pixels whose bit is set in that tile's ad_mask words, and adds its sums into ad_planes.
+    const uint32_t *ad_list;
+    uint32_t ad_n_list;
+    const uint32_t *ad_mask;
+    long long *ad_planes;
 };
+// Adaptive sampling (b200rt_render_adaptive).  Per tile: kAdaptiveMaskWords 32-bit words, bit lp = tile pixel lp (pool
+// numbering, kernels.cu map_tile).  Per pixel: 6 int64 sums -- radiance in 2^-30 units, then x^2 in 2^-24 units, as the
+// moments kernel keeps them in shared memory -- and a uint32 sample count.
+constexpr int kAdaptiveMaskWords = kPathBlock / 32;
+constexpr int kAdaptivePlanes = 6;
+struct AdaptiveState {
+    uint32_t w, h;
+    uint32_t *list;                    // this pass's active tiles
+    uint32_t n_list;
+    uint32_t *mask;                    // active pixels
+    uint32_t *unconv;                  // pixels not converged at their current count (zero outside the pass's tiles)
+    const long long *planes;
+    uint32_t *counts;
+    uint32_t *next_list;               // the next pass's active tiles ...
+    uint32_t *totals;                  // ... [0] how many, [1] their active pixels; zero before adaptive_decide
+    double rel_noise, abs_noise;
+};
+// Path blocks of the adaptive tile-pool kernel: one per entry of P.ad_list, or tail_chunks for the entries from tail_first.
+cudaError_t launch_path_adaptive(int stack, const RenderParams &P, bool leaf_first, cudaStream_t st);
+// Every pixel active, list = all tiles (tiles x kPathBlock threads).
+cudaError_t launch_adaptive_init(const AdaptiveState &A, uint32_t tiles, cudaStream_t st);
+// After a pass that took the active pixels to n samples: their counts become n and, with judge, their unconverged bits
+// are set from the convergence rule (b200rt.h).
+cudaError_t launch_adaptive_judge(const AdaptiveState &A, uint32_t n, bool judge, const DeviceScene &S, cudaStream_t st);
+// A pixel stays active if any pixel of its 3 x 3 neighbourhood is unconverged; writes the next list and totals.
+cudaError_t launch_adaptive_decide(const AdaptiveState &A, const DeviceScene &S, cudaStream_t st);
+// planes + counts -> the output planes (mean, or with sum the sums) and nothing else.
+cudaError_t launch_adaptive_finish(const AdaptiveState &A, bool sum, float *out_rgb, float *out_m2, cudaStream_t st);
 // Scratch of a launch with `tail_tiles` chunked tail tiles: tail_acc, then tail_arrivals.
 size_t tail_scratch_bytes(uint32_t tail_tiles, bool moments);
 // Path blocks of the tile-pool kernel resident on the current device at once (occupancy x SM count).
-cudaError_t path_resident_blocks(int stack, bool count, bool leaf_first, bool moments, int sm_count, int *blocks);
+cudaError_t path_resident_blocks(int stack, bool count, bool leaf_first, bool moments, int sm_count, int *blocks,
+                                 bool adaptive = false);
 #ifdef B200RT_BLOCK_TIMES
 cudaError_t set_block_times(unsigned long long *buf, uint32_t n_blocks);   // diagnostic build: see kernels.cu
 #endif

@@ -992,6 +992,29 @@ public:
         return to_image(sum, image_w, image_h, 1.0 / (double)std::max<size_t>(1, done));
     }
 
+    // Extension: adaptive sampling.  Each pixel gets samples until ITS noise reaches the target (b200rt_render_adaptive):
+    // min_spp in the first pass, then samples_per_pass per pass while the pixel or a neighbour is still noisy, up to
+    // samples_per_pixel.  A pixel is converged when the standard error of its mean, sqrt(mean of the channel variances /
+    // n), is <= rel_noise x its mean radiance.  Returns the mean image and each pixel's sample count (row-major); every
+    // pixel is the one render(bvh) gives at that pixel's count.  stats().paths is the sum of the counts.
+    std::pair<Image, std::vector<uint32_t>> render_adaptive(const BVH &bvh, double rel_noise, size_t min_spp, size_t samples_per_pass) {
+        const B200rtCamera cam = to_abi();
+        B200rtRenderOpts opts{};
+        opts.seed = rng_seed;
+        B200rtAdaptiveOpts aopts{};
+        aopts.min_spp = (uint32_t)std::min<size_t>(min_spp, 0xFFFFFFFFu);
+        aopts.step_spp = (uint32_t)std::min<size_t>(samples_per_pass, 0xFFFFFFFFu);
+        aopts.rel_noise = rel_noise;
+        std::vector<float> hdr(image_w * image_h * 3);
+        std::vector<uint32_t> spp(image_w * image_h);
+        if (b200rt_render_adaptive(bvh.handle(), &cam, &opts, &aopts, hdr.data(), nullptr, spp.data(), &last_stats) != B200RT_OK) {
+            std::cout << "Error: In Camera::render_adaptive(), " << b200rt_last_error() << std::endl;
+            std::exit(-1);
+        }
+        last_info = bvh.info();
+        return {to_image(hdr, image_w, image_h), std::move(spp)};
+    }
+
     // The frame relative noise (see render_to_noise) of SUM planes over n samples.
     static double frame_relative_noise(const std::vector<double> &sum, const std::vector<double> &sum2, size_t n) {
         if (n < 2 || sum.empty()) return std::numeric_limits<double>::infinity();

@@ -276,6 +276,34 @@ int b200rt_render_device(void *scene, const B200rtCamera *cam, const B200rtRende
 int b200rt_render_moments(void *scene, const B200rtCamera *cam, const B200rtRenderOpts *opts,
                           float *out_rgb, float *out_m2, B200rtStats *stats);
 
+/* Adaptive sampling: every pixel gets samples until IT reaches a noise target.  Pixel p renders samples
+ * [offset, offset + n_p) of its own stream, and its out_rgb / out_m2 values are the same bits b200rt_render_moments
+ * returns for a uniform render of n_p samples with the same seed and offset; out_spp_or_null[p] = n_p.  The maximum
+ * n_p is the sample count of `opts` (resolved as for b200rt_render), at most 2^16.
+ *   Passes: the first renders min(min_spp, max) samples of every pixel; each later one renders the next
+ * min(step_spp, max - n) samples of every pixel still active, all of which have the same count n.  After a pass,
+ * pixel p at count n is CONVERGED when err <= rel_noise * level + abs_noise, evaluated in double without FMA:
+ *   mean_c = (float)(S_c * 2^-30) * (float)(1.0 / n),  m2_c = (float)(Q_c * 2^-24) * (float)(1.0 / n)
+ *     (the mean-plane floats, from the pixel's fixed-point sums S of x and Q of x^2);
+ *   var_c = 0 if d = m2_c - mean_c^2 <= ldexp(m2_c, -20) + 2^-24, else n / (n - 1) * d;
+ *   err = sqrt((var_r + var_g + var_b) / (3 n)),  level = (mean_r + mean_g + mean_b) / 3.
+ * A pixel stays active while any pixel of its 3 x 3 neighbourhood (clipped at the image edge) is not converged, so a
+ * pixel that has not yet seen a light its neighbours see keeps sampling; a pixel that stops never resumes.  With
+ * rel_noise = abs_noise = 0 only pixels whose whole neighbourhood has exactly zero variance stop early.
+ *   B200RT_FLAG_SUM: both planes are sums.  B200RT_FLAG_ACCUMULATE is ignored.  B200RT_EINVAL with the wavefront
+ * variant, B200RT_FLAG_THREAD_PIXELS, B200RT_FLAG_COUNTERS, a multi-device handle, min_spp < 2, step_spp == 0, more
+ * than 2^16 samples, or a negative or non-finite rel_noise / abs_noise.  stats->paths is the sum of n_p.  The scene keeps
+ * about 52 bytes per pixel of device state for it (int64 sums, counts, masks), grown on first use. */
+typedef struct B200rtAdaptiveOpts {
+    uint32_t min_spp;     /* samples every pixel gets in the first pass; >= 2 */
+    uint32_t step_spp;    /* samples added to each still-active pixel per later pass; >= 1 */
+    double rel_noise;     /* converged: err <= rel_noise * level + abs_noise */
+    double abs_noise;
+} B200rtAdaptiveOpts;
+int b200rt_render_adaptive(void *scene, const B200rtCamera *cam, const B200rtRenderOpts *opts,
+                           const B200rtAdaptiveOpts *aopts, float *out_rgb, float *out_m2_or_null,
+                           uint32_t *out_spp_or_null, B200rtStats *stats);
+
 /* Replaces: Camera::render(const Scene &) end to end (camera.h:301-303): build + upload +
  * render + read back + free, all inside one call on host buffers. */
 int b200rt_render_scene(const B200rtSceneDesc *desc, const B200rtCamera *cam,
