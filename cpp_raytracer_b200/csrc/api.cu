@@ -299,10 +299,6 @@ int fill_camera(const B200rtCamera *cam, CameraParams &C) {
     return B200RT_OK;
 }
 
-uint32_t image_tiles(const CameraParams &C) {
-    return ((C.w + (uint32_t)kPathTileW - 1u) / (uint32_t)kPathTileW) * ((C.h + (uint32_t)kPathTileH - 1u) / (uint32_t)kPathTileH);
-}
-
 // Resolves the sample range of a render call: count 0 means camera.spp unless B200RT_FLAG_EXACT_COUNT is set.
 int sample_range_of(const B200rtCamera *cam, const B200rtRenderOpts &o, uint64_t *count_out) {
     const uint64_t count = (o.sample_count || (o.flags & B200RT_FLAG_EXACT_COUNT)) ? o.sample_count : cam->spp;
@@ -310,6 +306,37 @@ int sample_range_of(const B200rtCamera *cam, const B200rtRenderOpts &o, uint64_t
     if (o.variant != B200RT_VARIANT_MEGAKERNEL && o.variant != B200RT_VARIANT_WAVEFRONT)
         return fail(B200RT_EINVAL, "unknown kernel variant");
     *count_out = count;
+    return B200RT_OK;
+}
+
+// What a render of `cam` with `opts` (NULL: the defaults) on scene s takes from its arguments: the options in o; the camera,
+// the sample range, the seed, flags and counters in P; and the two schedule rules of the path kernels -- the work-pool
+// item order (P.group_shift) and the order of the traversal steps (leaf_first).  The caller sets the outputs and the scale.
+int render_setup(SceneImpl *s, const B200rtCamera *cam, const B200rtRenderOpts *opts, B200rtRenderOpts &o, RenderParams &P,
+                 bool &leaf_first) {
+    if (int rc = fill_camera(cam, P.cam)) return rc;
+    o = opts ? *opts : B200rtRenderOpts{};
+    uint64_t count = 0;
+    if (int rc = sample_range_of(cam, o, &count)) return rc;
+    P.scene = s->d;
+    P.seed = o.seed;
+    P.sample_begin = (uint32_t)o.sample_offset;
+    P.sample_count = (uint32_t)count;
+    P.flags = o.flags;
+    P.counters = s->d_counters;
+    // work-pool item order (kernels.cu): same-pixel groups of 8 when only light hits contribute (black background)
+    P.group_shift = (cam->background[0] == 0.0 && cam->background[1] == 0.0 && cam->background[2] == 0.0) ? 3u : 0u;
+    if (const char *g = std::getenv("B200RT_GROUP_SHIFT")) P.group_shift = (uint32_t)std::min(5, std::max(0, std::atoi(g)));   // experiments
+    // order of the node and the leaf step inside a traversal iteration (traverse.cuh): leaf first when quads dominate
+    leaf_first = s->info.n_quads > s->info.n_spheres;
+    if (const char *lf = std::getenv("B200RT_LEAF_FIRST")) leaf_first = lf[0] == '1';   // experiments
+    return B200RT_OK;
+}
+
+// Moments and adaptive renders run on the tile-pool kernel without traversal counters; `what` starts the message.
+int require_default_kernel(const B200rtRenderOpts &o, const char *what) {
+    if (o.variant == B200RT_VARIANT_WAVEFRONT || (o.flags & (B200RT_FLAG_THREAD_PIXELS | B200RT_FLAG_COUNTERS)))
+        return fail(B200RT_EINVAL, std::string(what) + " the default kernel only: no wavefront variant, B200RT_FLAG_THREAD_PIXELS or B200RT_FLAG_COUNTERS");
     return B200RT_OK;
 }
 
@@ -321,8 +348,8 @@ struct TailPlan {
     uint32_t tiles = 0, chunks = 8, min_chunk = 8;
     bool forced = false;
 };
-int plan_tail(SceneImpl *s, const CameraParams &C, bool count, bool leaf_first, bool moments, TailPlan *t, bool adaptive = false) {
-    const uint32_t tiles = ((C.w + (uint32_t)kPathTileW - 1u) / (uint32_t)kPathTileW) * ((C.h + (uint32_t)kPathTileH - 1u) / (uint32_t)kPathTileH);
+int plan_tail(SceneImpl *s, const CameraParams &C, PathMode mode, bool leaf_first, TailPlan *t) {
+    const uint32_t tiles = path_tiles(C.w, C.h);
     if (const char *e = std::getenv("B200RT_TAIL_TILES")) {
         long long r = 0, k = 0;
         const int n = std::sscanf(e, "%lld,%lld", &r, &k);
@@ -332,7 +359,7 @@ int plan_tail(SceneImpl *s, const CameraParams &C, bool count, bool leaf_first, 
         return B200RT_OK;
     }
     int resident = 0;
-    if (cudaError_t e = path_resident_blocks(s->stack, count, leaf_first, moments, s->sm_count, &resident, adaptive); e != cudaSuccess) {
+    if (cudaError_t e = path_resident_blocks(s->stack, mode, leaf_first, s->sm_count, &resident); e != cudaSuccess) {
         cudaGetLastError();
         return fail(B200RT_ECUDA, std::string("path kernel occupancy: ") + cudaGetErrorString(e));
     }
@@ -370,30 +397,44 @@ void chunk_tail(const TailPlan &t, uint32_t tiles, RenderParams &Q) {
     Q.tail_chunk_samples = chunk;
 }
 
+// After a render enqueued on `st` between s->ev0 and s->ev1: its four counters and its kernel time into *stats.  The copy
+// is ordered on st, which may be a caller's non-blocking stream, and st is synchronised.
+cudaError_t read_stats(SceneImpl *s, cudaStream_t st, B200rtStats *stats) {
+    unsigned long long c[4];
+    float ms = 0;
+    cudaError_t e = cudaMemcpyAsync(c, s->d_counters, sizeof c, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    if (e == cudaSuccess) e = cudaEventElapsedTime(&ms, s->ev0, s->ev1);
+    if (e != cudaSuccess) return e;
+    stats->kernel_ms = ms;
+    stats->rays = c[0]; stats->node_visits = c[1]; stats->prim_tests = c[2]; stats->quad_tests = c[3];
+    return cudaSuccess;
+}
+
+// Grows the scene's scratch frame (the host-buffer renders' device output) to at least `floats` floats.
+cudaError_t grow_frame(SceneImpl *s, size_t floats) {
+    if (floats <= s->frame_floats) return cudaSuccess;
+    if (s->d_frame) { dev_free(s->d_frame); s->d_frame = nullptr; s->frame_floats = 0; }
+    if (cudaError_t e = dev_alloc(&s->d_frame, floats * sizeof(float)); e != cudaSuccess) return e;
+    s->frame_floats = floats;
+    return cudaSuccess;
+}
+
 // Enqueues the path kernel(s) of one render call on `st` (the caller holds s->mu and has made s->device current).
 // d_m2 (optional): the second-moment plane, written by the moments instantiation of the default kernel.
 int render_on_device(SceneImpl *s, const B200rtCamera *cam, const B200rtRenderOpts *opts, float *d_out,
                      cudaStream_t st, B200rtStats *stats, bool sync_for_stats, float *d_m2 = nullptr) {
     RenderParams P{};
-    if (int rc = fill_camera(cam, P.cam)) return rc;
-    B200rtRenderOpts o{};
-    if (opts) o = *opts;
-    uint64_t count = 0;
-    if (int rc = sample_range_of(cam, o, &count)) return rc;
-    if (d_m2 && (o.variant == B200RT_VARIANT_WAVEFRONT || (o.flags & (B200RT_FLAG_THREAD_PIXELS | B200RT_FLAG_COUNTERS))))
-        return fail(B200RT_EINVAL, "moments are rendered by the default kernel only: no wavefront variant, B200RT_FLAG_THREAD_PIXELS or B200RT_FLAG_COUNTERS");
-    P.scene = s->d;
-    P.seed = o.seed;
-    P.sample_begin = (uint32_t)o.sample_offset;
-    P.sample_count = (uint32_t)count;
+    B200rtRenderOpts o;
+    bool leaf_first;
+    if (int rc = render_setup(s, cam, opts, o, P, leaf_first)) return rc;
+    if (d_m2)
+        if (int rc = require_default_kernel(o, "moments are rendered by")) return rc;
+    const uint64_t count = P.sample_count;
+    const PathMode mode = d_m2 ? PathMode::Moments : (o.flags & B200RT_FLAG_COUNTERS) ? PathMode::Counters : PathMode::Plain;
     P.out = d_out;
     P.out_m2 = d_m2;
-    P.flags = o.flags;
     P.scale = (o.flags & B200RT_FLAG_SUM) || count == 0 ? 1.0f : (float)(1.0 / (double)count);
-    P.counters = s->d_counters;
-    // work-pool item order (kernels.cu): same-pixel groups of 8 when only light hits contribute (black background)
-    P.group_shift = (cam->background[0] == 0.0 && cam->background[1] == 0.0 && cam->background[2] == 0.0) ? 3u : 0u;
-    if (const char *g = std::getenv("B200RT_GROUP_SHIFT")) P.group_shift = (uint32_t)std::min(5, std::max(0, std::atoi(g)));   // experiments
     CUDA_TRY(cudaMemsetAsync(s->d_counters, 0, 4 * sizeof(unsigned long long), st));
     unsigned long long launches = 1;
     CUDA_TRY(cudaEventRecord(s->ev0, st));
@@ -420,16 +461,12 @@ int render_on_device(SceneImpl *s, const B200rtCamera *cam, const B200rtRenderOp
         WavefrontPool W{};
         wavefront_pool_layout(s->d_pool, s->pool_slots, W);
         launches = 0;
-        CUDA_TRY(run_wavefront(s->stack, P, W, (o.flags & B200RT_FLAG_COUNTERS) != 0, st, s->sm_count, &launches));
+        CUDA_TRY(run_wavefront(s->stack, P, W, mode == PathMode::Counters, st, s->sm_count, &launches));
         CUDA_TRY(cudaEventRecord(s->ev_pool, st));
     } else {
-        // order of the node and the leaf step inside a traversal iteration (traverse.cuh): leaf first when quads dominate
-        bool leaf_first = s->info.n_quads > s->info.n_spheres;
-        if (const char *lf = std::getenv("B200RT_LEAF_FIRST")) leaf_first = lf[0] == '1';   // experiments
-        const bool count_flag = (o.flags & B200RT_FLAG_COUNTERS) != 0;
         TailPlan tail;
         if (!(o.flags & B200RT_FLAG_THREAD_PIXELS)) {
-            if (int rc = plan_tail(s, P.cam, count_flag, leaf_first, d_m2 != nullptr, &tail)) return rc;
+            if (int rc = plan_tail(s, P.cam, mode, leaf_first, &tail)) return rc;
             if (tail.tiles) CUDA_TRY(tail_scratch(s, tail.tiles, d_m2 != nullptr, st, &P));
         }
         // the tile work pool counts (pixel, sample) items in 32 bits: more than 2^22 samples per pixel go in several launches
@@ -441,8 +478,8 @@ int render_on_device(SceneImpl *s, const B200rtCamera *cam, const B200rtRenderOp
             Q.sample_begin = (uint32_t)(o.sample_offset + done);
             Q.sample_count = (uint32_t)std::min<uint64_t>(per_launch, count - done);
             if (done) Q.flags |= kRenderAccumulate;
-            if (tail.tiles) chunk_tail(tail, image_tiles(P.cam), Q);
-            CUDA_TRY(launch_path_megakernel(s->stack, Q, count_flag, leaf_first, st, d_m2 != nullptr));
+            if (tail.tiles) chunk_tail(tail, path_tiles(P.cam.w, P.cam.h), Q);
+            CUDA_TRY(launch_path_megakernel(s->stack, Q, mode, leaf_first, st));
             ++launches;
         }
         if (tail.tiles) CUDA_TRY(cudaEventRecord(s->ev_tail, st));
@@ -453,15 +490,7 @@ int render_on_device(SceneImpl *s, const B200rtCamera *cam, const B200rtRenderOp
         stats->paths = (uint64_t)cam->image_w * cam->image_h * count;
         stats->kernel_launches = launches;
         stats->n_devices = 1;
-        if (sync_for_stats) {
-            unsigned long long c[4];
-            CUDA_TRY(cudaMemcpyAsync(c, s->d_counters, sizeof c, cudaMemcpyDeviceToHost, st));
-            CUDA_TRY(cudaStreamSynchronize(st));
-            float ms = 0;
-            CUDA_TRY(cudaEventElapsedTime(&ms, s->ev0, s->ev1));
-            stats->kernel_ms = ms;
-            stats->rays = c[0]; stats->node_visits = c[1]; stats->prim_tests = c[2]; stats->quad_tests = c[3];
-        }
+        if (sync_for_stats) CUDA_TRY(read_stats(s, st, stats));
     }
     return B200RT_OK;
 }
@@ -478,8 +507,7 @@ int finish_scene(SceneImpl *s, const B200rtSceneInfo &info) {
     if (reinterpret_cast<uintptr_t>(s->d.nodes) & 127)   // trav_node_step forms plane addresses with OR / XOR on the low bits
         return fail(B200RT_ECUDA, "node array is not 128-byte aligned");
     s->info = info;
-    const int need_stack = (int)(3 * info.tree_depth);
-    s->stack = need_stack <= 32 ? 32 : (need_stack <= 64 ? 64 : 128);
+    s->stack = with_stack((int)(3 * info.tree_depth), [](auto K) { return K.value; });
     s->info.stack_entries = (uint32_t)s->stack;
     s->info.device_bytes = 0;
     for (size_t b : s->alloc_bytes) s->info.device_bytes += b;
@@ -643,15 +671,6 @@ int replicate_scene_on(const SceneImpl *src, int dev, SceneImpl **out) {
     return B200RT_OK;
 }
 
-void collect_stats(SceneImpl *s, B200rtStats *st) {   // after the stream that rendered has been synchronised
-    unsigned long long c[4] = {0, 0, 0, 0};
-    cudaMemcpy(c, s->d_counters, sizeof c, cudaMemcpyDeviceToHost);
-    float ms = 0;
-    if (cudaEventElapsedTime(&ms, s->ev0, s->ev1) != cudaSuccess) { cudaGetLastError(); ms = 0; }
-    st->kernel_ms = ms;
-    st->rays = c[0]; st->node_visits = c[1]; st->prim_tests = c[2]; st->quad_tests = c[3];
-}
-
 // One frame on all devices of `m` into the caller's host buffer(s): sample split, exchange, scale, read back.  With
 // out_m2 every device's frame holds [image | second moment] and both planes go through the same per-float exchange.
 int render_multi(MultiImpl *m, const B200rtCamera *cam, const B200rtRenderOpts *opts, float *out_rgb, float *out_m2,
@@ -746,8 +765,7 @@ int render_multi(MultiImpl *m, const B200rtCamera *cam, const B200rtRenderOpts *
     total.peer_exchange = m->peers ? 1u : 0u;
     for (int d = 0; d < n; ++d) {
         DeviceGuard g(m->dev[d]->device);
-        CUDA_TRY(cudaStreamSynchronize(m->stream[d]));   // also: nobody reads this device's frame any more
-        collect_stats(m->dev[d], &st[d]);
+        CUDA_TRY(read_stats(m->dev[d], m->stream[d], &st[d]));   // synchronises: nobody reads this device's frame any more
         total.kernel_ms = std::max(total.kernel_ms, st[d].kernel_ms);
         total.paths += st[d].paths; total.rays += st[d].rays;
         total.node_visits += st[d].node_visits; total.prim_tests += st[d].prim_tests; total.quad_tests += st[d].quad_tests;
@@ -782,11 +800,7 @@ int render_host(void *scene, const B200rtCamera *cam, const B200rtRenderOpts *op
     const double t0 = now_ms();
     const size_t floats = (size_t)cam->image_w * cam->image_h * 3;   // one plane
     const size_t all_floats = floats * (out_m2 ? 2 : 1);
-    if (all_floats > s->frame_floats) {
-        if (s->d_frame) { dev_free(s->d_frame); s->d_frame = nullptr; s->frame_floats = 0; }
-        CUDA_TRY(dev_alloc(&s->d_frame, all_floats * sizeof(float)));
-        s->frame_floats = all_floats;
-    }
+    CUDA_TRY(grow_frame(s, all_floats));
     B200rtRenderOpts o{};
     if (opts) o = *opts;
     o.flags &= ~(uint32_t)B200RT_FLAG_ACCUMULATE;   // host entry always overwrites
@@ -834,14 +848,12 @@ int render_adaptive_host(void *scene, const B200rtCamera *cam, const B200rtRende
     if (!s) return fail(B200RT_EINVAL, "bad scene handle");
     if (!cam || !aopts || !out_rgb) return fail(B200RT_EINVAL, "camera, adaptive options or output pointer is NULL");
     RenderParams P{};
-    if (int rc = fill_camera(cam, P.cam)) return rc;
-    B200rtRenderOpts o{};
-    if (opts) o = *opts;
-    o.flags &= ~(uint32_t)B200RT_FLAG_ACCUMULATE;   // host entry always overwrites
-    uint64_t max_spp = 0;
-    if (int rc = sample_range_of(cam, o, &max_spp)) return rc;
-    if (o.variant == B200RT_VARIANT_WAVEFRONT || (o.flags & (B200RT_FLAG_THREAD_PIXELS | B200RT_FLAG_COUNTERS)))
-        return fail(B200RT_EINVAL, "adaptive renders use the default kernel only: no wavefront variant, B200RT_FLAG_THREAD_PIXELS or B200RT_FLAG_COUNTERS");
+    B200rtRenderOpts o;
+    bool leaf_first;
+    if (int rc = render_setup(s, cam, opts, o, P, leaf_first)) return rc;
+    if (int rc = require_default_kernel(o, "adaptive renders use")) return rc;
+    P.flags &= ~(uint32_t)B200RT_FLAG_ACCUMULATE;   // host entry always overwrites
+    const uint64_t max_spp = P.sample_count;
     const B200rtAdaptiveOpts a = *aopts;
     if (a.min_spp < 2 || a.step_spp == 0) return fail(B200RT_EINVAL, "adaptive options need min_spp >= 2 and step_spp >= 1");
     if (max_spp > kMaxSamplesPerLaunchMoments) return fail(B200RT_EINVAL, "an adaptive render takes at most 2^16 samples per pixel");
@@ -852,12 +864,8 @@ int render_adaptive_host(void *scene, const B200rtCamera *cam, const B200rtRende
     const double t0 = now_ms();
     const cudaStream_t st = 0;
     const size_t pixels = (size_t)cam->image_w * cam->image_h, floats = pixels * 3;
-    const uint32_t tiles = image_tiles(P.cam);
-    if (2 * floats > s->frame_floats) {
-        if (s->d_frame) { dev_free(s->d_frame); s->d_frame = nullptr; s->frame_floats = 0; }
-        CUDA_TRY(dev_alloc(&s->d_frame, 2 * floats * sizeof(float)));
-        s->frame_floats = 2 * floats;
-    }
+    const uint32_t tiles = path_tiles(P.cam.w, P.cam.h);
+    CUDA_TRY(grow_frame(s, 2 * floats));
     AdaptiveBuffers b{};
     const size_t bytes = adaptive_layout(nullptr, pixels, tiles, &b);
     if (bytes > s->adapt_bytes) {
@@ -867,18 +875,10 @@ int render_adaptive_host(void *scene, const B200rtCamera *cam, const B200rtRende
     }
     adaptive_layout(static_cast<char *>(s->d_adapt), pixels, tiles, &b);
 
-    P.scene = s->d;
-    P.seed = o.seed;
-    P.flags = o.flags;
-    P.counters = s->d_counters;
-    P.group_shift = (cam->background[0] == 0.0 && cam->background[1] == 0.0 && cam->background[2] == 0.0) ? 3u : 0u;   // as render_on_device
-    if (const char *gs = std::getenv("B200RT_GROUP_SHIFT")) P.group_shift = (uint32_t)std::min(5, std::max(0, std::atoi(gs)));
     P.ad_mask = b.mask;
     P.ad_planes = b.planes;
-    bool leaf_first = s->info.n_quads > s->info.n_spheres;
-    if (const char *lf = std::getenv("B200RT_LEAF_FIRST")) leaf_first = lf[0] == '1';
     TailPlan tail;
-    if (int rc = plan_tail(s, P.cam, false, leaf_first, true, &tail, true)) return rc;
+    if (int rc = plan_tail(s, P.cam, PathMode::Adaptive, leaf_first, &tail)) return rc;
     tail.tiles = std::min(tail.tiles, tiles);
 
     AdaptiveState A{};
@@ -904,7 +904,7 @@ int render_adaptive_host(void *scene, const B200rtCamera *cam, const B200rtRende
         Q.ad_list = A.list;
         Q.ad_n_list = n_list;
         if (tail.tiles) chunk_tail(tail, n_list, Q);
-        CUDA_TRY(launch_path_adaptive(s->stack, Q, leaf_first, st));
+        CUDA_TRY(launch_path_megakernel(s->stack, Q, PathMode::Adaptive, leaf_first, st));
         paths += active_pixels * k;
         n += k;
         A.n_list = n_list;
@@ -926,21 +926,15 @@ int render_adaptive_host(void *scene, const B200rtCamera *cam, const B200rtRende
     ++launches;
     if (tail.tiles) CUDA_TRY(cudaEventRecord(s->ev_tail, st));
     CUDA_TRY(cudaEventRecord(s->ev1, st));
-    unsigned long long c[4];
-    CUDA_TRY(cudaMemcpyAsync(c, s->d_counters, sizeof c, cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(cudaStreamSynchronize(st));
+    B200rtStats local{};
+    CUDA_TRY(read_stats(s, st, &local));
     const double t1 = now_ms();
     CUDA_TRY(staged_download(out_rgb, s->d_frame, floats * sizeof(float), st));
     if (out_m2) CUDA_TRY(staged_download(out_m2, s->d_frame + floats, floats * sizeof(float), st));
     if (out_spp) CUDA_TRY(staged_download(out_spp, b.counts, pixels * sizeof(uint32_t), st));
     const double t2 = now_ms();
     if (stats) {
-        B200rtStats local{};
-        float ms = 0;
-        CUDA_TRY(cudaEventElapsedTime(&ms, s->ev0, s->ev1));
-        local.kernel_ms = ms;
         local.paths = paths;
-        local.rays = c[0];
         local.kernel_launches = launches;
         local.n_devices = 1;
         local.d2h_ms = t2 - t1;
@@ -1222,21 +1216,17 @@ int b200rt_debug_lane_accounting(void *scene, const B200rtCamera *cam, const B20
     std::lock_guard<std::mutex> lk(s->mu);
     DeviceGuard g(s->device);
     RenderParams P{};
-    if (int rc = fill_camera(cam, P.cam)) return rc;
-    B200rtRenderOpts o{};
-    if (opts) o = *opts;
-    uint64_t count = 0;
-    if (int rc = sample_range_of(cam, o, &count)) return rc;
+    B200rtRenderOpts o;
+    bool leaf_first;
+    if (int rc = render_setup(s, cam, opts, o, P, leaf_first)) return rc;
     float *d_frame = nullptr;
     unsigned long long *d_acc = nullptr;
     CUDA_TRY(dev_alloc(&d_frame, (size_t)cam->image_w * cam->image_h * 3 * sizeof(float)));
     cudaError_t e = dev_alloc(&d_acc, 16 * sizeof(unsigned long long));
     if (e == cudaSuccess) e = cudaMemsetAsync(d_acc, 0, 16 * sizeof(unsigned long long), 0);
     if (e == cudaSuccess) e = cudaMemsetAsync(s->d_counters, 0, 4 * sizeof(unsigned long long), 0);
-    P.scene = s->d; P.seed = o.seed; P.sample_begin = (uint32_t)o.sample_offset; P.sample_count = (uint32_t)count;
-    P.out = d_frame; P.flags = o.flags & B200RT_FLAG_THREAD_PIXELS; P.scale = 1.0f; P.counters = s->d_counters;
-    P.group_shift = (cam->background[0] == 0.0 && cam->background[1] == 0.0 && cam->background[2] == 0.0) ? 3u : 0u;
-    if (e == cudaSuccess) e = launch_path_lanes(s->stack, P, d_acc, s->info.n_quads > s->info.n_spheres, 0);
+    P.out = d_frame; P.flags &= B200RT_FLAG_THREAD_PIXELS; P.scale = 1.0f;
+    if (e == cudaSuccess) e = launch_path_lanes(s->stack, P, d_acc, leaf_first, 0);
     if (e == cudaSuccess) e = cudaMemcpy(counters_out, d_acc, 16 * sizeof(unsigned long long), cudaMemcpyDeviceToHost);
     cudaStreamSynchronize(0);
     dev_free(d_frame); dev_free(d_acc);

@@ -116,7 +116,7 @@ struct PixelMap {
     bool valid;
 };
 __device__ __forceinline__ PixelMap map_pixel(const CameraParams &C) {
-    const uint32_t tiles_x = (C.w + (uint32_t)kPathTileW - 1u) / (uint32_t)kPathTileW;
+    const uint32_t tiles_x = path_tiles_x(C.w);
     const uint32_t tile_x = blockIdx.x % tiles_x, tile_y = blockIdx.x / tiles_x;
     PixelMap m;
     m.px = tile_x * (uint32_t)kPathTileW + (threadIdx.x % (uint32_t)kPathTileW);
@@ -126,17 +126,15 @@ __device__ __forceinline__ PixelMap map_pixel(const CameraParams &C) {
     return m;
 }
 
-__device__ __forceinline__ void write_pixel_and_counters(const RenderParams &P, const PixelMap &m, float sum_r, float sum_g,
-                                                         float sum_b, uint32_t lane_rays, bool count,
-                                                         const TraversalCounters &ctr) {
+// A pixel's three channels, times k: stored, or with accumulate added to what is there.
+__device__ __forceinline__ void store_rgb(float *o, float r, float g, float b, float k, bool accumulate) {
+    if (accumulate) { o[0] += r * k; o[1] += g * k; o[2] += b * k; }
+    else { o[0] = r * k; o[1] = g * k; o[2] = b * k; }
+}
+
+// The rays (and with count the traversal counters) of the warp's lanes into P.counters: one atomic per warp and counter.
+__device__ __forceinline__ void write_counters(const RenderParams &P, uint32_t lane_rays, bool count, const TraversalCounters &ctr) {
     unsigned long long rays = lane_rays;
-    if (m.valid && B200RT_CHECK(P.scene, m.pixel < P.cam.w * P.cam.h, 3)) {
-        float *o = P.out + (size_t)m.pixel * 3;
-        const float k = P.scale;
-        if (P.flags & kRenderAccumulate) { o[0] += sum_r * k; o[1] += sum_g * k; o[2] += sum_b * k; }
-        else { o[0] = sum_r * k; o[1] = sum_g * k; o[2] = sum_b * k; }
-    }
-    // counters: one atomic per warp
     for (int off = 16; off; off >>= 1) rays += __shfl_down_sync(0xffffffffu, rays, off);
     if ((threadIdx.x & 31) == 0 && rays) atomicAdd(&P.counters[0], rays);
     if (count) {
@@ -148,6 +146,14 @@ __device__ __forceinline__ void write_pixel_and_counters(const RenderParams &P, 
         }
         if ((threadIdx.x & 31) == 0) { atomicAdd(&P.counters[1], a); atomicAdd(&P.counters[2], b); atomicAdd(&P.counters[3], c); }
     }
+}
+
+__device__ __forceinline__ void write_pixel_and_counters(const RenderParams &P, const PixelMap &m, float sum_r, float sum_g,
+                                                         float sum_b, uint32_t lane_rays, bool count,
+                                                         const TraversalCounters &ctr) {
+    if (m.valid && B200RT_CHECK(P.scene, m.pixel < P.cam.w * P.cam.h, 3))
+        store_rgb(P.out + (size_t)m.pixel * 3, sum_r, sum_g, sum_b, P.scale, (P.flags & kRenderAccumulate) != 0);
+    write_counters(P, lane_rays, count, ctr);
 }
 
 // One path segment's worth of "shade + continue or regenerate": consumes the finished traversal
@@ -224,12 +230,17 @@ constexpr float kFixScale = 1073741824.0f;            // 2^30
 constexpr double kFixInv = 1.0 / 1073741824.0;
 constexpr float kFix2Scale = 16777216.0f;             // 2^24
 constexpr double kFix2Inv = 1.0 / 16777216.0;
+// A fixed-point sum of radiance (fix_rgb) or of x^2 (fix_x2) as the float every reader of the sums starts from: the image
+// and the second-moment plane (store_tile_pixel), the adaptive rule (pixel_converged) and the adaptive output planes
+// (adaptive_finish_kernel).  So a pixel an adaptive render stops at n samples has the bits of an n-sample render_moments.
+__device__ __forceinline__ float fix_rgb(long long a) { return (float)((double)a * kFixInv); }
+__device__ __forceinline__ float fix_x2(long long q) { return (float)((double)q * kFix2Inv); }
 
 struct TileMap {
     uint32_t x0, y0, vw, n_valid;      // tile origin, valid width, valid pixel count (edge tiles are ragged)
 };
 __device__ __forceinline__ TileMap map_tile(const CameraParams &C, uint32_t tile) {
-    const uint32_t tiles_x = (C.w + (uint32_t)kPathTileW - 1u) / (uint32_t)kPathTileW;
+    const uint32_t tiles_x = path_tiles_x(C.w);
     const uint32_t tile_x = tile % tiles_x, tile_y = tile / tiles_x;
     TileMap t;
     t.x0 = tile_x * (uint32_t)kPathTileW;
@@ -386,23 +397,16 @@ __device__ __forceinline__ void store_tile_pixel(const RenderParams &P, const Ti
     const uint32_t px = tm.x0 + lp % tm.vw, py = tm.y0 + lp / tm.vw;
     const uint32_t pixel = py * P.cam.w + px;
     if (B200RT_CHECK(P.scene, pixel < P.cam.w * P.cam.h, 3)) {
-        const float sum_r = (float)((double)a[0] * kFixInv), sum_g = (float)((double)a[1] * kFixInv), sum_b = (float)((double)a[2] * kFixInv);
-        float *o = P.out + (size_t)pixel * 3;
         const float k = P.scale;
-        if (P.flags & kRenderAccumulate) { o[0] += sum_r * k; o[1] += sum_g * k; o[2] += sum_b * k; }
-        else { o[0] = sum_r * k; o[1] = sum_g * k; o[2] = sum_b * k; }
-        if constexpr (MOMENTS) {
-            const float q_r = (float)((double)q[0] * kFix2Inv), q_g = (float)((double)q[1] * kFix2Inv), q_b = (float)((double)q[2] * kFix2Inv);
-            float *o2 = P.out_m2 + (size_t)pixel * 3;
-            if (P.flags & kRenderAccumulate) { o2[0] += q_r * k; o2[1] += q_g * k; o2[2] += q_b * k; }
-            else { o2[0] = q_r * k; o2[1] = q_g * k; o2[2] = q_b * k; }
-        }
+        store_rgb(P.out + (size_t)pixel * 3, fix_rgb(a[0]), fix_rgb(a[1]), fix_rgb(a[2]), k, (P.flags & kRenderAccumulate) != 0);
+        if constexpr (MOMENTS)
+            store_rgb(P.out_m2 + (size_t)pixel * 3, fix_x2(q[0]), fix_x2(q[1]), fix_x2(q[2]), k, (P.flags & kRenderAccumulate) != 0);
     }
 }
 
 // ADAPTIVE: active pixel lp's sums of this pass are added to its int64 planes.  A pixel has one writer per pass (the
 // block of a whole tile, or the last chunk of a tail tile to arrive), so a plain add is exact; the conversion to floats
-// happens once, after the last pass (adaptive_finish_kernel), with the expression store_tile_pixel uses.
+// happens once, after the last pass (adaptive_finish_kernel, through fix_rgb / fix_x2).
 __device__ __forceinline__ void add_tile_pixel(const RenderParams &P, const TileMap &tm, const TilePoolAdaptive &tp, uint32_t lp,
                                                const long long (&a)[3], const long long (&q)[3]) {
     const uint32_t lt = tp.act[lp];
@@ -463,21 +467,6 @@ __device__ __forceinline__ void pool_merge_chunk(const RenderParams &P, const Ti
     if (lp < tm.n_valid) finish_tile_pixel<MOMENTS, ADAPTIVE>(P, tm, tp, lp, a, q);
 }
 
-__device__ __forceinline__ void write_counters(const RenderParams &P, uint32_t lane_rays, bool count, const TraversalCounters &ctr) {
-    unsigned long long rays = lane_rays;
-    for (int off = 16; off; off >>= 1) rays += __shfl_down_sync(0xffffffffu, rays, off);
-    if ((threadIdx.x & 31) == 0 && rays) atomicAdd(&P.counters[0], rays);
-    if (count) {
-        unsigned long long a = ctr.nodes, b = ctr.prims, c = ctr.quads;
-        for (int off = 16; off; off >>= 1) {
-            a += __shfl_down_sync(0xffffffffu, a, off);
-            b += __shfl_down_sync(0xffffffffu, b, off);
-            c += __shfl_down_sync(0xffffffffu, c, off);
-        }
-        if ((threadIdx.x & 31) == 0) { atomicAdd(&P.counters[1], a); atomicAdd(&P.counters[2], b); atomicAdd(&P.counters[3], c); }
-    }
-}
-
 #ifdef B200RT_BLOCK_TIMES
 // Diagnostic build (-DB200RT_BLOCK_TIMES, scripts/tail_profile.py): thread 0 of every path_megakernel_pool block records
 // {start ns, end ns, SM} of %globaltimer into g_block_times[blockIdx.x] (armed by b200rt_debug_block_times).
@@ -502,10 +491,6 @@ cudaError_t set_block_times(unsigned long long *buf, uint32_t n_blocks) {
 }
 #endif
 
-__device__ __forceinline__ uint32_t image_tiles(const CameraParams &C) {
-    return ((C.w + (uint32_t)kPathTileW - 1u) / (uint32_t)kPathTileW) * ((C.h + (uint32_t)kPathTileH - 1u) / (uint32_t)kPathTileH);
-}
-
 // Start of an ADAPTIVE block: the tile of list entry `entry`, and its active pixels (its mask bits) in ascending tile-pixel
 // order in tp.act.  Returns the tile's map with n_valid = the number of active pixels, so that block_items and pool_fetch
 // number the items over them exactly as they number a whole tile's pixels.
@@ -514,7 +499,7 @@ __device__ __forceinline__ TileMap adaptive_tile(const RenderParams &P, uint32_t
     bool ok = B200RT_CHECK(P.scene, entry < P.ad_n_list, 3);
     if (ok) {
         tile = P.ad_list[entry];
-        ok = B200RT_CHECK(P.scene, tile < image_tiles(P.cam), 3);
+        ok = B200RT_CHECK(P.scene, tile < path_tiles(P.cam.w, P.cam.h), 3);
     }
     TileMap tm = map_tile(P.cam, ok ? tile : 0u);
     const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31u, base = warp * 32u;
@@ -536,12 +521,14 @@ __device__ __forceinline__ TileMap adaptive_tile(const RenderParams &P, uint32_t
 }
 
 // path_megakernel_pool (variant 0, default): every lane runs traverse-then-shade in a loop and takes the tile's next
-// (pixel, sample) item as soon as its path ends.  MOMENTS: also the per-pixel sum of x^2 into P.out_m2 (b200rt_render_moments).
-// ADAPTIVE (implies MOMENTS; b200rt_render_adaptive): a block renders the active pixels of an entry of P.ad_list and adds
-// both sums into P.ad_planes; the host sets sample_begin to the pass's first sample, so the Philox keys are unchanged.
-template <int STACK, bool COUNT, bool LEAF_FIRST = false, int MINB = kPathMinBlocks, bool MOMENTS = false, bool ADAPTIVE = false>
-__global__ void __launch_bounds__(kPathBlock, MINB) path_megakernel_pool(const __grid_constant__ RenderParams P) {
-    static_assert(!ADAPTIVE || MOMENTS, "the adaptive kernel sums x^2");
+// (pixel, sample) item as soon as its path ends.  Moments: also the per-pixel sum of x^2 into P.out_m2
+// (b200rt_render_moments).  Adaptive (b200rt_render_adaptive): a block renders the active pixels of an entry of P.ad_list
+// and adds both sums into P.ad_planes; the host sets sample_begin to the pass's first sample, so the Philox keys are unchanged.
+template <int STACK, PathMode MODE, bool LEAF_FIRST>
+__global__ void __launch_bounds__(kPathBlock, kPathMinBlocks) path_megakernel_pool(const __grid_constant__ RenderParams P) {
+    constexpr bool COUNT = MODE == PathMode::Counters;
+    constexpr bool MOMENTS = MODE == PathMode::Moments || MODE == PathMode::Adaptive;
+    constexpr bool ADAPTIVE = MODE == PathMode::Adaptive;
     __shared__ TilePoolOf<MOMENTS, ADAPTIVE> tp;
 #ifdef B200RT_BLOCK_TIMES
     const unsigned long long t_start = globaltimer_ns();
@@ -577,8 +564,8 @@ __global__ void __launch_bounds__(kPathBlock, MINB) path_megakernel_pool(const _
 // path_megakernel (thread-owns-pixel form, kept for A/B: B200RT_FLAG_THREAD_PIXELS): every lane runs traverse-then-shade
 // in a loop over ITS pixel's samples and starts the next sample as soon as a path ends.  64 registers (16 blocks = 32 warps per SM) measured
 // fastest on B200: 8/12/16/20/24 blocks per SM gave 2707/3171/3263/2630/2307 Mpaths/s on C2.
-template <int STACK, bool COUNT, bool LEAF_FIRST = false, int MINB = kPathMinBlocks>
-__global__ void __launch_bounds__(kPathBlock, MINB) path_megakernel(const __grid_constant__ RenderParams P) {
+template <int STACK, bool COUNT>
+__global__ void __launch_bounds__(kPathBlock, kPathMinBlocks) path_megakernel(const __grid_constant__ RenderParams P) {
     const CameraParams &C = P.cam;
     const PixelMap m = map_pixel(C);
     LaneState L;
@@ -587,7 +574,7 @@ __global__ void __launch_bounds__(kPathBlock, MINB) path_megakernel(const __grid
     if (m.valid && C.max_depth > 0 && P.sample_count > 0) {
         while (shade_and_advance(P, m, best, L)) {
             // world.hit_by(ray, Interval::with_min(0.00001))  (camera.h:217)
-            best = closest_hit<STACK, COUNT, LEAF_FIRST>(P.scene, L.ray.ox, L.ray.oy, L.ray.oz, L.ray.dx, L.ray.dy, L.ray.dz, 0.00001,
+            best = closest_hit<STACK, COUNT>(P.scene, L.ray.ox, L.ray.oy, L.ray.oz, L.ray.dx, L.ray.dy, L.ray.dz, 0.00001,
                                              __longlong_as_double(0x7ff0000000000000LL), &ctr);
         }
     }
@@ -679,19 +666,23 @@ __global__ void __launch_bounds__(kPathBlock) path_lanes_kernel(const __grid_con
 }
 
 // ------------------------------------------------------------------------------------------
-__global__ void tonemap_kernel(const float *__restrict__ hdr, long long n_pixels, int32_t *__restrict__ out, int clamp) {
-    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n_pixels) return;
-    const double r = hdr[i * 3 + 0], g = hdr[i * 3 + 1], b = hdr[i * 3 + 2];
+// One pixel's tone map into q[0..2]: Reinhard + gamma 2 + int(255.999999 v)   [RGB::as_string, rgb.h:90-113]
+__device__ __forceinline__ void tonemap_pixel(double r, double g, double b, int clamp, int32_t *__restrict__ q) {
     const double L = 0.2126 * r + 0.7152 * g + 0.0722 * b;          // rgb.h:28-30
     const double scale = 255 + 0.999999;                             // rgb.h:106
     const double v[3] = {r / (1 + L), g / (1 + L), b / (1 + L)};     // rgb.h:99-104
 #pragma unroll
     for (int c = 0; c < 3; ++c) {
-        int q = (int)(scale * sqrt(v[c]));                           // pow(v, 1/2), truncation (rgb.h:107-111)
-        if (clamp) q = q < 0 ? 0 : (q > 255 ? 255 : q);
-        out[i * 3 + c] = q;
+        int t = (int)(scale * sqrt(v[c]));                           // pow(v, 1/2), truncation (rgb.h:107-111)
+        if (clamp) t = t < 0 ? 0 : (t > 255 ? 255 : t);
+        q[c] = t;
     }
+}
+
+__global__ void tonemap_kernel(const float *__restrict__ hdr, long long n_pixels, int32_t *__restrict__ out, int clamp) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_pixels) return;
+    tonemap_pixel(hdr[i * 3 + 0], hdr[i * 3 + 1], hdr[i * 3 + 2], clamp, out + i * 3);
 }
 
 // Frame epilogue on the reducing rank: sum -> mean in place (pixel_color /= spp, camera.h:290) and,
@@ -701,18 +692,7 @@ __global__ void finalize_kernel(float *__restrict__ frame, long long n_pixels, f
     if (i >= n_pixels) return;
     const float rf = frame[i * 3 + 0] * scale, gf = frame[i * 3 + 1] * scale, bf = frame[i * 3 + 2] * scale;
     frame[i * 3 + 0] = rf; frame[i * 3 + 1] = gf; frame[i * 3 + 2] = bf;
-    if (ldr) {
-        const double r = rf, g = gf, b = bf;
-        const double L = 0.2126 * r + 0.7152 * g + 0.0722 * b;
-        const double s255 = 255 + 0.999999;
-        const double v[3] = {r / (1 + L), g / (1 + L), b / (1 + L)};
-#pragma unroll
-        for (int c = 0; c < 3; ++c) {
-            int q = (int)(s255 * sqrt(v[c]));
-            if (clamp) q = q < 0 ? 0 : (q > 255 ? 255 : q);
-            ldr[i * 3 + c] = q;
-        }
-    }
+    if (ldr) tonemap_pixel(rf, gf, bf, clamp, ldr + i * 3);
 }
 
 // Multi-GPU frame exchange as ONE kernel over peer memory (NVLink / NVSwitch): this rank's slice of
@@ -756,20 +736,12 @@ __global__ void __launch_bounds__(kPeerThreads) reduce_finalize_peers_kernel(con
     }
     if (!root_ldr) return;
     __syncthreads();
-    int q[kPeerTilePx / kPeerThreads][3];
+    int32_t q[kPeerTilePx / kPeerThreads][3];
 #pragma unroll
     for (int k = 0; k < kPeerTilePx / kPeerThreads; ++k) {
         const int px = threadIdx.x + k * kPeerThreads;
-        const double r = tile[px * 3 + 0], g = tile[px * 3 + 1], b = tile[px * 3 + 2];
-        const double L = 0.2126 * r + 0.7152 * g + 0.0722 * b;
-        const double s255 = 255 + 0.999999;
-        const double v[3] = {r / (1 + L), g / (1 + L), b / (1 + L)};
-#pragma unroll
-        for (int c = 0; c < 3; ++c) {
-            int t = (px * 3 < n_fl) ? (int)(s255 * sqrt(v[c])) : 0;
-            if (clamp) t = t < 0 ? 0 : (t > 255 ? 255 : t);
-            q[k][c] = t;
-        }
+        if (px * 3 < n_fl) tonemap_pixel(tile[px * 3 + 0], tile[px * 3 + 1], tile[px * 3 + 2], clamp, q[k]);
+        else q[k][0] = q[k][1] = q[k][2] = 0;                                                // past the ragged end of the frame
     }
     __syncthreads();
     int32_t *itile = reinterpret_cast<int32_t *>(tile);
@@ -788,20 +760,14 @@ __global__ void __launch_bounds__(kPeerThreads) reduce_finalize_peers_kernel(con
 }
 
 // ------------------------------------------------------------------------------------------
-template <int STACK>
-static cudaError_t launch_raycast_t(const DeviceScene &S, const double *rays, long long n, double tmin, double tmax,
-                                    int32_t *prim, double *t, cudaStream_t st) {
-    if (n == 0) return cudaSuccess;
-    const int block = 128;
-    raycast_kernel<STACK><<<(unsigned)((n + block - 1) / block), block, 0, st>>>(S, rays, n, tmin, tmax, prim, t);
-    return cudaGetLastError();
-}
-
 cudaError_t launch_raycast(int stack, const DeviceScene &S, const double *rays, long long n, double tmin, double tmax,
                            int32_t *prim, double *t, cudaStream_t st) {
-    if (stack <= 32) return launch_raycast_t<32>(S, rays, n, tmin, tmax, prim, t, st);
-    if (stack <= 64) return launch_raycast_t<64>(S, rays, n, tmin, tmax, prim, t, st);
-    return launch_raycast_t<128>(S, rays, n, tmin, tmax, prim, t, st);
+    if (n == 0) return cudaSuccess;
+    const int block = 128;
+    with_stack(stack, [&](auto K) {
+        raycast_kernel<K.value><<<(unsigned)((n + block - 1) / block), block, 0, st>>>(S, rays, n, tmin, tmax, prim, t);
+    });
+    return cudaGetLastError();
 }
 
 cudaError_t launch_debug_camera(const CameraParams &C, const uint32_t *pixels, const uint32_t *rnd, long long n, double *rays_out,
@@ -827,55 +793,40 @@ cudaError_t launch_debug_shade(int stack, const DeviceScene &S, const double *ra
     if (n == 0) return cudaSuccess;
     const unsigned blocks = (unsigned)((n + 127) / 128);
     ShadeRecord *out = static_cast<ShadeRecord *>(records);
-    if (stack <= 32) debug_shade_kernel<32><<<blocks, 128, 0, st>>>(S, rays, rnd, n, tmin, tmax, out);
-    else if (stack <= 64) debug_shade_kernel<64><<<blocks, 128, 0, st>>>(S, rays, rnd, n, tmin, tmax, out);
-    else debug_shade_kernel<128><<<blocks, 128, 0, st>>>(S, rays, rnd, n, tmin, tmax, out);
+    with_stack(stack, [&](auto K) { debug_shade_kernel<K.value><<<blocks, 128, 0, st>>>(S, rays, rnd, n, tmin, tmax, out); });
     return cudaGetLastError();
 }
 
-template <int STACK>
-static cudaError_t launch_path_t(const RenderParams &P, bool count, bool leaf_first, cudaStream_t st, bool moments) {
-    const uint32_t tiles = ((P.cam.w + (uint32_t)kPathTileW - 1u) / (uint32_t)kPathTileW) * ((P.cam.h + (uint32_t)kPathTileH - 1u) / (uint32_t)kPathTileH);
-    if (tiles == 0) return cudaSuccess;
-    // tile pool: whole-tile blocks, then tail_chunks chunk blocks for each tile from tail_first on
-    const uint32_t blocks = P.tail_chunks ? P.tail_first + (tiles - P.tail_first) * P.tail_chunks : tiles;
-    if (moments) {   // tile pool, no counters (the caller has rejected kRenderThreadPixels and the counters flag)
-        if (leaf_first) path_megakernel_pool<STACK, false, true, kPathMinBlocks, true><<<blocks, kPathBlock, 0, st>>>(P);
-        else path_megakernel_pool<STACK, false, false, kPathMinBlocks, true><<<blocks, kPathBlock, 0, st>>>(P);
+// The tile-pool kernel instance of (stack, mode, leaf_first).  The launch and the occupancy query that sizes its chunked
+// tail both take it from here, so they always name the same instance.
+template <int STACK, PathMode MODE>
+static const void *pool_instance(bool leaf_first) {
+    return leaf_first ? (const void *)path_megakernel_pool<STACK, MODE, true> : (const void *)path_megakernel_pool<STACK, MODE, false>;
+}
+static const void *path_pool_kernel(int stack, PathMode mode, bool leaf_first) {
+    return with_stack(stack, [&](auto K) {
+        return mode == PathMode::Plain      ? pool_instance<K.value, PathMode::Plain>(leaf_first)
+               : mode == PathMode::Counters ? pool_instance<K.value, PathMode::Counters>(leaf_first)
+               : mode == PathMode::Moments  ? pool_instance<K.value, PathMode::Moments>(leaf_first)
+                                            : pool_instance<K.value, PathMode::Adaptive>(leaf_first);
+    });
+}
+
+cudaError_t launch_path_megakernel(int stack, const RenderParams &P, PathMode mode, bool leaf_first, cudaStream_t st) {
+    // one block per tile, or per entry of the pass's tile list
+    const uint32_t units = mode == PathMode::Adaptive ? P.ad_n_list : path_tiles(P.cam.w, P.cam.h);
+    if (units == 0) return cudaSuccess;
+    if ((P.flags & kRenderThreadPixels) && (mode == PathMode::Plain || mode == PathMode::Counters)) {
+        with_stack(stack, [&](auto K) {   // round-1 work distribution: node-then-leaf only
+            if (mode == PathMode::Counters) path_megakernel<K.value, true><<<units, kPathBlock, 0, st>>>(P);
+            else path_megakernel<K.value, false><<<units, kPathBlock, 0, st>>>(P);
+        });
         return cudaGetLastError();
     }
-    if (!(P.flags & kRenderThreadPixels)) {
-        if (leaf_first) {
-            if (count) path_megakernel_pool<STACK, true, true><<<blocks, kPathBlock, 0, st>>>(P);
-            else path_megakernel_pool<STACK, false, true><<<blocks, kPathBlock, 0, st>>>(P);
-        } else if (count) path_megakernel_pool<STACK, true><<<blocks, kPathBlock, 0, st>>>(P);
-        else path_megakernel_pool<STACK, false><<<blocks, kPathBlock, 0, st>>>(P);
-        return cudaGetLastError();
-    }
-    if (count) path_megakernel<STACK, true><<<tiles, kPathBlock, 0, st>>>(P);      // round-1 work distribution: node-then-leaf only
-    else path_megakernel<STACK, false><<<tiles, kPathBlock, 0, st>>>(P);
-    return cudaGetLastError();
-}
-
-cudaError_t launch_path_megakernel(int stack, const RenderParams &P, bool count, bool leaf_first, cudaStream_t st, bool moments) {
-    if (stack <= 32) return launch_path_t<32>(P, count, leaf_first, st, moments);
-    if (stack <= 64) return launch_path_t<64>(P, count, leaf_first, st, moments);
-    return launch_path_t<128>(P, count, leaf_first, st, moments);
-}
-
-template <int STACK>
-static cudaError_t launch_path_adaptive_t(const RenderParams &P, bool leaf_first, cudaStream_t st) {
-    if (P.ad_n_list == 0) return cudaSuccess;
-    const uint32_t blocks = P.tail_chunks ? P.tail_first + (P.ad_n_list - P.tail_first) * P.tail_chunks : P.ad_n_list;
-    if (leaf_first) path_megakernel_pool<STACK, false, true, kPathMinBlocks, true, true><<<blocks, kPathBlock, 0, st>>>(P);
-    else path_megakernel_pool<STACK, false, false, kPathMinBlocks, true, true><<<blocks, kPathBlock, 0, st>>>(P);
-    return cudaGetLastError();
-}
-
-cudaError_t launch_path_adaptive(int stack, const RenderParams &P, bool leaf_first, cudaStream_t st) {
-    if (stack <= 32) return launch_path_adaptive_t<32>(P, leaf_first, st);
-    if (stack <= 64) return launch_path_adaptive_t<64>(P, leaf_first, st);
-    return launch_path_adaptive_t<128>(P, leaf_first, st);
+    // tile pool: whole-tile blocks, then tail_chunks chunk blocks for each unit from tail_first on
+    const uint32_t blocks = P.tail_chunks ? P.tail_first + (units - P.tail_first) * P.tail_chunks : units;
+    void *args[] = {const_cast<RenderParams *>(&P)};
+    return cudaLaunchKernel(path_pool_kernel(stack, mode, leaf_first), blocks, kPathBlock, args, 0, st);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -887,9 +838,7 @@ __device__ __forceinline__ TileMap adaptive_map(const AdaptiveState &A, uint32_t
     C.h = A.h;
     return map_tile(C, tile);
 }
-__device__ __forceinline__ uint32_t adaptive_tiles(const AdaptiveState &A) {
-    return ((A.w + (uint32_t)kPathTileW - 1u) / (uint32_t)kPathTileW) * ((A.h + (uint32_t)kPathTileH - 1u) / (uint32_t)kPathTileH);
-}
+__device__ __forceinline__ uint32_t adaptive_tiles(const AdaptiveState &A) { return path_tiles(A.w, A.h); }
 
 __global__ void __launch_bounds__(kPathBlock) adaptive_init_kernel(const __grid_constant__ AdaptiveState A) {
     const uint32_t tile = blockIdx.x, warp = threadIdx.x >> 5;
@@ -909,16 +858,17 @@ __device__ __forceinline__ double channel_variance(float mean, float m2, uint32_
     return (double)n / (double)(n - 1u) * d;
 }
 
-// The convergence rule (b200rt.h, b200rt_render_adaptive): the mean-plane floats exactly as store_tile_pixel writes them,
-// then err = sqrt(sum of the channel variances / 3n) against rel_noise x the mean of the three channel means + abs_noise.
-// In double; the library is built with -fmad=false, so nothing is contracted and the host can replay it bit for bit.
+// The convergence rule (b200rt.h, b200rt_render_adaptive): the mean-plane floats exactly as store_tile_pixel writes them
+// (fix_rgb / fix_x2 times the float 1/n), then err = sqrt(sum of the channel variances / 3n) against rel_noise x the mean
+// of the three channel means + abs_noise.  In double; the library is built with -fmad=false, so nothing is contracted and
+// the host can replay it bit for bit.
 __device__ __forceinline__ bool pixel_converged(const AdaptiveState &A, const long long *p, uint32_t n) {
     const float inv = (float)(1.0 / (double)n);
     double var = 0.0, level = 0.0;
 #pragma unroll
     for (int c = 0; c < 3; ++c) {
-        const float mean = (float)((double)p[c] * kFixInv) * inv;
-        const float m2 = (float)((double)p[3 + c] * kFix2Inv) * inv;
+        const float mean = fix_rgb(p[c]) * inv;
+        const float m2 = fix_x2(p[3 + c]) * inv;
         var += channel_variance(mean, m2, n);
         level += (double)mean;
     }
@@ -953,7 +903,7 @@ __global__ void __launch_bounds__(kPathBlock) adaptive_decide_kernel(const __gri
     if (!B200RT_CHECK(S, tile < adaptive_tiles(A), 3)) return;
     const TileMap tm = adaptive_map(A, tile);
     const uint32_t lp = threadIdx.x, lane = lp & 31u;
-    const uint32_t tiles_x = (A.w + (uint32_t)kPathTileW - 1u) / (uint32_t)kPathTileW;
+    const uint32_t tiles_x = path_tiles_x(A.w);
     const size_t mw = (size_t)tile * kAdaptiveMaskWords + (lp >> 5);
     bool keep = false;
     if (((A.mask[mw] >> lane) & 1u) && lp < tm.n_valid) {
@@ -976,7 +926,7 @@ __global__ void __launch_bounds__(kPathBlock) adaptive_decide_kernel(const __gri
     }
 }
 
-// planes / counts -> the output floats: store_tile_pixel's expression with the pixel's own count (k = 1 for sums).
+// planes / counts -> the output floats: store_tile_pixel's conversion with the pixel's own count (k = 1 for sums).
 __global__ void adaptive_finish_kernel(const __grid_constant__ AdaptiveState A, int sum, float *__restrict__ out_rgb,
                                        float *__restrict__ out_m2) {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -986,8 +936,8 @@ __global__ void adaptive_finish_kernel(const __grid_constant__ AdaptiveState A, 
     const long long *p = A.planes + i * kAdaptivePlanes;
 #pragma unroll
     for (int c = 0; c < 3; ++c) {
-        out_rgb[i * 3 + c] = (float)((double)p[c] * kFixInv) * k;
-        out_m2[i * 3 + c] = (float)((double)p[3 + c] * kFix2Inv) * k;
+        out_rgb[i * 3 + c] = fix_rgb(p[c]) * k;
+        out_m2[i * 3 + c] = fix_x2(p[3 + c]) * k;
     }
 }
 
@@ -1017,36 +967,21 @@ size_t tail_scratch_bytes(uint32_t tail_tiles, bool moments) {
     return (size_t)tail_tiles * ((size_t)kPathBlock * 3 * sizeof(long long) * (moments ? 2 : 1) + sizeof(uint32_t));
 }
 
-template <int STACK>
-static cudaError_t path_blocks_per_sm(bool count, bool leaf_first, bool moments, bool adaptive, int &n) {
-    cudaError_t e;
-    if (adaptive) e = leaf_first ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, path_megakernel_pool<STACK, false, true, kPathMinBlocks, true, true>, kPathBlock, 0)
-                                 : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, path_megakernel_pool<STACK, false, false, kPathMinBlocks, true, true>, kPathBlock, 0);
-    else if (moments) e = leaf_first ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, path_megakernel_pool<STACK, false, true, kPathMinBlocks, true>, kPathBlock, 0)
-                                : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, path_megakernel_pool<STACK, false, false, kPathMinBlocks, true>, kPathBlock, 0);
-    else if (leaf_first) e = count ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, path_megakernel_pool<STACK, true, true>, kPathBlock, 0)
-                                   : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, path_megakernel_pool<STACK, false, true>, kPathBlock, 0);
-    else e = count ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, path_megakernel_pool<STACK, true>, kPathBlock, 0)
-                   : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, path_megakernel_pool<STACK, false>, kPathBlock, 0);
-    return e;
-}
-
-cudaError_t path_resident_blocks(int stack, bool count, bool leaf_first, bool moments, int sm_count, int *blocks, bool adaptive) {
+cudaError_t path_resident_blocks(int stack, PathMode mode, bool leaf_first, int sm_count, int *blocks) {
     int n = 0;
-    const cudaError_t e = stack <= 32   ? path_blocks_per_sm<32>(count, leaf_first, moments, adaptive, n)
-                          : stack <= 64 ? path_blocks_per_sm<64>(count, leaf_first, moments, adaptive, n)
-                                        : path_blocks_per_sm<128>(count, leaf_first, moments, adaptive, n);
+    const cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, path_pool_kernel(stack, mode, leaf_first), kPathBlock, 0);
     *blocks = n * sm_count;
     return e;
 }
 
 cudaError_t launch_path_lanes(int stack, const RenderParams &P, unsigned long long *acc, bool leaf_first, cudaStream_t st) {
-    const uint32_t tiles = ((P.cam.w + (uint32_t)kPathTileW - 1u) / (uint32_t)kPathTileW) * ((P.cam.h + (uint32_t)kPathTileH - 1u) / (uint32_t)kPathTileH);
+    const uint32_t tiles = path_tiles(P.cam.w, P.cam.h);
     if (tiles == 0) return cudaSuccess;
     const bool pool = !(P.flags & kRenderThreadPixels);
-    if (stack <= 32) { if (pool) path_lanes_kernel<32, true><<<tiles, kPathBlock, 0, st>>>(P, acc, leaf_first); else path_lanes_kernel<32, false><<<tiles, kPathBlock, 0, st>>>(P, acc, leaf_first); }
-    else if (stack <= 64) { if (pool) path_lanes_kernel<64, true><<<tiles, kPathBlock, 0, st>>>(P, acc, leaf_first); else path_lanes_kernel<64, false><<<tiles, kPathBlock, 0, st>>>(P, acc, leaf_first); }
-    else { if (pool) path_lanes_kernel<128, true><<<tiles, kPathBlock, 0, st>>>(P, acc, leaf_first); else path_lanes_kernel<128, false><<<tiles, kPathBlock, 0, st>>>(P, acc, leaf_first); }
+    with_stack(stack, [&](auto K) {
+        if (pool) path_lanes_kernel<K.value, true><<<tiles, kPathBlock, 0, st>>>(P, acc, leaf_first);
+        else path_lanes_kernel<K.value, false><<<tiles, kPathBlock, 0, st>>>(P, acc, leaf_first);
+    });
     return cudaGetLastError();
 }
 

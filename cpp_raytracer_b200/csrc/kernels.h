@@ -1,6 +1,7 @@
 // kernels.h -- launch interface between the C ABI (api.cu) and the kernels (kernels.cu).
 #pragma once
 #include <cstdint>
+#include <type_traits>
 #include <cuda_runtime.h>
 
 #include "shade.cuh"
@@ -21,6 +22,11 @@ constexpr int kPathBlock = B200RT_PATH_BLOCK;       // threads per block of the 
 constexpr int kPathTileW = B200RT_TILE_W;           // tile = kPathTileW x (kPathBlock / kPathTileW) pixels
 constexpr int kPathTileH = kPathBlock / kPathTileW;
 static_assert(kPathBlock % kPathTileW == 0 && kPathBlock % 32 == 0, "tile shape");
+// Tile columns and tiles of a w x h image (tile t is column t % path_tiles_x(w), row t / path_tiles_x(w)).
+__host__ __device__ __forceinline__ uint32_t path_tiles_x(uint32_t w) { return (w + (uint32_t)kPathTileW - 1u) / (uint32_t)kPathTileW; }
+__host__ __device__ __forceinline__ uint32_t path_tiles(uint32_t w, uint32_t h) {
+    return path_tiles_x(w) * ((h + (uint32_t)kPathTileH - 1u) / (uint32_t)kPathTileH);
+}
 #ifdef B200RT_PATH_MINB
 constexpr int kPathMinBlocks = B200RT_PATH_MINB;    // occupancy experiments
 #else
@@ -29,11 +35,13 @@ constexpr int kPathMinBlocks = 1024 / kPathBlock;   // 1024 threads = 32 warps p
 constexpr uint32_t kRenderAccumulate = 2u;    // == B200RT_FLAG_ACCUMULATE
 constexpr uint32_t kRenderThreadPixels = 16u; // == B200RT_FLAG_THREAD_PIXELS
 constexpr uint32_t kMaxSamplesPerLaunch = 1u << 22;   // tile items (up to 1024 pixels x samples, + one group) are counted in 32 bits
-// Second-moment plane (path_megakernel_pool<..., MOMENTS = true>): the sum of x^2 per pixel and channel is kept in 64-bit
+// Second-moment plane (path_megakernel_pool in PathMode::Moments): the sum of x^2 per pixel and channel is kept in 64-bit
 // fixed point of 2^-24 units -- per-sample resolution 6.0e-8, range +-5.5e11 per pixel per launch.  At most 2^16 samples
 // per launch, so a mean x^2 of up to 8.4e6 per sample (x up to about 2900) fits; the brightest emitter of the scene
 // set (500 x 0.8) gives x^2 <= 1.6e5.
 constexpr uint32_t kMaxSamplesPerLaunchMoments = 1u << 16;
+// What a launch of the tile-pool path kernel writes (launch_path_megakernel).
+enum class PathMode { Plain, Counters, Moments, Adaptive };
 
 struct RenderParams {
     DeviceScene scene;
@@ -77,8 +85,6 @@ struct AdaptiveState {
     uint32_t *totals;                  // ... [0] how many, [1] their active pixels; zero before adaptive_decide
     double rel_noise, abs_noise;
 };
-// Path blocks of the adaptive tile-pool kernel: one per entry of P.ad_list, or tail_chunks for the entries from tail_first.
-cudaError_t launch_path_adaptive(int stack, const RenderParams &P, bool leaf_first, cudaStream_t st);
 // Every pixel active, list = all tiles (tiles x kPathBlock threads).
 cudaError_t launch_adaptive_init(const AdaptiveState &A, uint32_t tiles, cudaStream_t st);
 // After a pass that took the active pixels to n samples: their counts become n and, with judge, their unconverged bits
@@ -91,8 +97,7 @@ cudaError_t launch_adaptive_finish(const AdaptiveState &A, bool sum, float *out_
 // Scratch of a launch with `tail_tiles` chunked tail tiles: tail_acc, then tail_arrivals.
 size_t tail_scratch_bytes(uint32_t tail_tiles, bool moments);
 // Path blocks of the tile-pool kernel resident on the current device at once (occupancy x SM count).
-cudaError_t path_resident_blocks(int stack, bool count, bool leaf_first, bool moments, int sm_count, int *blocks,
-                                 bool adaptive = false);
+cudaError_t path_resident_blocks(int stack, PathMode mode, bool leaf_first, int sm_count, int *blocks);
 #ifdef B200RT_BLOCK_TIMES
 cudaError_t set_block_times(unsigned long long *buf, uint32_t n_blocks);   // diagnostic build: see kernels.cu
 #endif
@@ -127,13 +132,22 @@ cudaError_t run_wavefront(int stack, const RenderParams &P, const WavefrontPool 
                           unsigned long long *launches);
 
 // `stack` = traversal stack entries the scene needs (3 x depth of the 4-wide tree); the
-// launchers pick the smallest instantiation that fits (32 / 64 / 128).
+// launchers pick the smallest instantiation that fits (32 / 64 / 128): with_stack calls f with it as a compile-time constant.
+template <typename F>
+auto with_stack(int stack, F &&f) {
+    if (stack <= 32) return f(std::integral_constant<int, 32>{});
+    if (stack <= 64) return f(std::integral_constant<int, 64>{});
+    return f(std::integral_constant<int, 128>{});
+}
 cudaError_t launch_raycast(int stack, const DeviceScene &S, const double *rays, long long n, double tmin, double tmax,
                            int32_t *prim, double *t, cudaStream_t st);
-// leaf_first: order of the two steps inside one iteration of the traversal loop (see closest_hit).  moments: the tile-pool
-// kernel that also writes P.out_m2 (not with count, not with kRenderThreadPixels; at most kMaxSamplesPerLaunchMoments samples)
-cudaError_t launch_path_megakernel(int stack, const RenderParams &P, bool count, bool leaf_first, cudaStream_t st,
-                                   bool moments = false);
+// The path kernel of a render.  mode: what the tile-pool kernel writes besides the image --
+//   Counters  also the traversal counters P.counters[1..3]
+//   Moments   also the second-moment plane P.out_m2 (at most kMaxSamplesPerLaunchMoments samples per launch)
+//   Adaptive  both sums of the active pixels of the tiles in P.ad_list into P.ad_planes, instead of the image
+// Plain and Counters run the thread-owns-pixel kernel under kRenderThreadPixels.  leaf_first: order of the two steps
+// inside one iteration of the traversal loop (see closest_hit).
+cudaError_t launch_path_megakernel(int stack, const RenderParams &P, PathMode mode, bool leaf_first, cudaStream_t st);
 // measurement only: 16 lane-accounting counters (see path_lanes_kernel)
 cudaError_t launch_path_lanes(int stack, const RenderParams &P, unsigned long long *acc, bool leaf_first, cudaStream_t st);
 cudaError_t launch_finalize(float *frame, long long n_pixels, float scale, int32_t *ldr, int clamp, cudaStream_t st);

@@ -314,9 +314,7 @@ static cudaError_t run_wavefront_t(const RenderParams &P, WavefrontPool W, bool 
 
 cudaError_t run_wavefront(int stack, const RenderParams &P, const WavefrontPool &W, bool count, cudaStream_t st, int sm_count,
                           unsigned long long *launches) {
-    if (stack <= 32) return run_wavefront_t<32>(P, W, count, st, sm_count, launches);
-    if (stack <= 64) return run_wavefront_t<64>(P, W, count, st, sm_count, launches);
-    return run_wavefront_t<128>(P, W, count, st, sm_count, launches);
+    return with_stack(stack, [&](auto K) { return run_wavefront_t<K.value>(P, W, count, st, sm_count, launches); });
 }
 
 }  // namespace b200rt
