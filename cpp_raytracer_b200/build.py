@@ -17,7 +17,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libb200rt.so")
 SOURCES = ["api.cu", "kernels.cu", "wavefront.cu", "lbvh.cu", "scene_layout.cu", "devmem.cu", "bvh_builder.cpp"]
-HEADERS = ["bvh_builder.h", "devmem.h", "kernels.h", "thread_pool.h", "traverse.cuh", "shade.cuh", "rng.cuh",
+HEADERS = ["bvh_builder.h", "devmem.h", "kernels.h", "thread_pool.h", "traverse.cuh", "shade.cuh", "path.cuh", "rng.cuh",
            os.path.join("..", "..", "include", "b200rt.h")]
 
 NVCC_FLAGS = [

@@ -3,14 +3,14 @@
 //
 //   raycast_kernel        one thread per ray, closest hit -> (canonical prim index, t)
 //                         [BVH::hit_by / Scene::hit_by, reference bvh.h:585-715, scene.h:59-75]
-//   path_megakernel       one thread per pixel, all of that pixel's samples, with path regeneration:
-//                         a lane whose path ended starts its next sample right away
-//                         [Camera::render<T> + ray_color, reference camera.h:205-297]
+//   path_megakernel_pool  the default path kernel: a block's lanes take its tile's (pixel, sample) items from a pool
+//                         [Camera::render<T> + ray_color, reference camera.h:205-297; the rules of a path: path.cuh]
+//   path_megakernel       the thread-owns-pixel form (B200RT_FLAG_THREAD_PIXELS): one thread per pixel, all its samples
 //   tonemap_kernel        Reinhard + gamma 2 + int(255.999999 v)   [RGB::as_string, rgb.h:90-113]
 #include <type_traits>
 
 #include "kernels.h"
-#include "shade.cuh"
+#include "path.cuh"
 
 namespace b200rt {
 
@@ -132,22 +132,6 @@ __device__ __forceinline__ void store_rgb(float *o, float r, float g, float b, f
     else { o[0] = r * k; o[1] = g * k; o[2] = b * k; }
 }
 
-// The rays (and with count the traversal counters) of the warp's lanes into P.counters: one atomic per warp and counter.
-__device__ __forceinline__ void write_counters(const RenderParams &P, uint32_t lane_rays, bool count, const TraversalCounters &ctr) {
-    unsigned long long rays = lane_rays;
-    for (int off = 16; off; off >>= 1) rays += __shfl_down_sync(0xffffffffu, rays, off);
-    if ((threadIdx.x & 31) == 0 && rays) atomicAdd(&P.counters[0], rays);
-    if (count) {
-        unsigned long long a = ctr.nodes, b = ctr.prims, c = ctr.quads;
-        for (int off = 16; off; off >>= 1) {
-            a += __shfl_down_sync(0xffffffffu, a, off);
-            b += __shfl_down_sync(0xffffffffu, b, off);
-            c += __shfl_down_sync(0xffffffffu, c, off);
-        }
-        if ((threadIdx.x & 31) == 0) { atomicAdd(&P.counters[1], a); atomicAdd(&P.counters[2], b); atomicAdd(&P.counters[3], c); }
-    }
-}
-
 __device__ __forceinline__ void write_pixel_and_counters(const RenderParams &P, const PixelMap &m, float sum_r, float sum_g,
                                                          float sum_b, uint32_t lane_rays, bool count,
                                                          const TraversalCounters &ctr) {
@@ -167,20 +151,12 @@ struct LaneState {
     uint32_t rays = 0;
 };
 __device__ __forceinline__ bool shade_and_advance(const RenderParams &P, const PixelMap &m, const Hit &best, LaneState &L) {
-    const CameraParams &C = P.cam;
-    const uint32_t k0 = (uint32_t)P.seed, k1 = (uint32_t)(P.seed >> 32);
     if (L.has_path) {
         ++L.rays;
-        bool cont;
-        if (best.ref == kNoHit) {
-            L.sum_r += L.p.tr * C.background[0]; L.sum_g += L.p.tg * C.background[1]; L.sum_b += L.p.tb * C.background[2];
-            cont = false;   // camera.h:248
-        } else {
-            const Philox4 rnd = philox4x32_10(m.pixel, P.sample_begin + L.s, L.bounce + 1u, 0u, k0, k1);
-            cont = shade_hit(P.scene, best, rnd, L.ray, L.p, L.sum_r, L.sum_g, L.sum_b);
-            // ray_color(scattered, depth_left - 1): contributes nothing once depth_left hits 0 (camera.h:211-213)
-            if (cont && ++L.bounce == C.max_depth) cont = false;
-        }
+        float er, eg, eb;
+        // the sums start at +0 and so are never -0: adding the zero contribution of a hit that is not a light changes no bit
+        const bool cont = path_bounce(P, best, m.pixel, L.s, L.bounce, L.ray, L.p, er, eg, eb);
+        L.sum_r += er; L.sum_g += eg; L.sum_b += eb;
         if (!cont) {
             L.has_path = false;
             ++L.s;
@@ -188,8 +164,7 @@ __device__ __forceinline__ bool shade_and_advance(const RenderParams &P, const P
     }
     if (!L.has_path) {
         if (L.s == P.sample_count) return false;
-        const Philox4 rnd = philox4x32_10(m.pixel, P.sample_begin + L.s, 0u, 0u, k0, k1);
-        camera_ray(C, m.px, m.py, rnd, L.ray, L.p);
+        path_start(P, m.pixel, m.px, m.py, L.s, L.ray, L.p);
         L.bounce = 0;
         L.has_path = true;
     }
@@ -239,6 +214,8 @@ __device__ __forceinline__ float fix_x2(long long q) { return (float)((double)q 
 struct TileMap {
     uint32_t x0, y0, vw, n_valid;      // tile origin, valid width, valid pixel count (edge tiles are ragged)
 };
+// Image column and row of tile pixel lt.
+__device__ __forceinline__ uint2 tile_xy(const TileMap &tm, uint32_t lt) { return make_uint2(tm.x0 + lt % tm.vw, tm.y0 + lt / tm.vw); }
 __device__ __forceinline__ TileMap map_tile(const CameraParams &C, uint32_t tile) {
     const uint32_t tiles_x = path_tiles_x(C.w);
     const uint32_t tile_x = tile % tiles_x, tile_y = tile / tiles_x;
@@ -349,33 +326,21 @@ __device__ __forceinline__ bool pool_fetch(const RenderParams &P, const TileMap 
     return true;
 }
 
-// shade_and_advance with the tile pool: same path semantics, same Philox keys (pixel, sample, bounce).
+// shade_and_advance with the tile pool: the lane's path takes one step or, once ended, the lane takes the next item.
 template <bool MOMENTS = false, bool ADAPTIVE = false>
 __device__ __forceinline__ bool pool_shade_and_advance(const RenderParams &P, const TileMap &tm, TilePoolOf<MOMENTS, ADAPTIVE> &tp,
                                                        uint32_t total_items, const Hit &best, PoolLane &L, Ray &ray) {
-    const CameraParams &C = P.cam;
-    const uint32_t k0 = (uint32_t)P.seed, k1 = (uint32_t)(P.seed >> 32);
     if (L.has_path) {
         ++L.rays;
-        bool cont;
-        float er = 0.0f, eg = 0.0f, eb = 0.0f;
-        if (best.ref == kNoHit) {
-            er = L.p.tr * C.background[0]; eg = L.p.tg * C.background[1]; eb = L.p.tb * C.background[2];
-            cont = false;   // camera.h:248
-        } else {
-            const Philox4 rnd = philox4x32_10(L.pixel, P.sample_begin + L.s, L.bounce + 1u, 0u, k0, k1);
-            cont = shade_hit(P.scene, best, rnd, ray, L.p, er, eg, eb);
-            // ray_color(scattered, depth_left - 1): contributes nothing once depth_left hits 0 (camera.h:211-213)
-            if (cont && ++L.bounce == C.max_depth) cont = false;
-        }
+        float er, eg, eb;
+        const bool cont = path_bounce(P, best, L.pixel, L.s, L.bounce, ray, L.p, er, eg, eb);
         pool_contribute<MOMENTS>(tp, L.lp, er, eg, eb);   // the path's only non-zero contribution, if any (see pool_contribute)
         if (!cont) L.has_path = false;
     }
     if (!L.has_path) {
         uint32_t px, py;
         if (!pool_fetch<ADAPTIVE>(P, tm, tp, total_items, L, px, py)) return false;
-        const Philox4 rnd = philox4x32_10(L.pixel, P.sample_begin + L.s, 0u, 0u, k0, k1);
-        camera_ray(C, px, py, rnd, ray, L.p);
+        path_start(P, L.pixel, px, py, L.s, ray, L.p);
         L.has_path = true;
     }
     return true;
@@ -394,8 +359,8 @@ __device__ __forceinline__ void pool_init(TilePoolOf<MOMENTS> &tp, uint32_t firs
 template <bool MOMENTS = false>
 __device__ __forceinline__ void store_tile_pixel(const RenderParams &P, const TileMap &tm, uint32_t lp, const long long (&a)[3],
                                                  const long long (&q)[3]) {
-    const uint32_t px = tm.x0 + lp % tm.vw, py = tm.y0 + lp / tm.vw;
-    const uint32_t pixel = py * P.cam.w + px;
+    const uint2 xy = tile_xy(tm, lp);
+    const uint32_t pixel = xy.y * P.cam.w + xy.x;
     if (B200RT_CHECK(P.scene, pixel < P.cam.w * P.cam.h, 3)) {
         const float k = P.scale;
         store_rgb(P.out + (size_t)pixel * 3, fix_rgb(a[0]), fix_rgb(a[1]), fix_rgb(a[2]), k, (P.flags & kRenderAccumulate) != 0);
@@ -410,7 +375,8 @@ __device__ __forceinline__ void store_tile_pixel(const RenderParams &P, const Ti
 __device__ __forceinline__ void add_tile_pixel(const RenderParams &P, const TileMap &tm, const TilePoolAdaptive &tp, uint32_t lp,
                                                const long long (&a)[3], const long long (&q)[3]) {
     const uint32_t lt = tp.act[lp];
-    const uint32_t pixel = (tm.y0 + lt / tm.vw) * P.cam.w + tm.x0 + lt % tm.vw;
+    const uint2 xy = tile_xy(tm, lt);
+    const uint32_t pixel = xy.y * P.cam.w + xy.x;
     if (B200RT_CHECK(P.scene, lt < kPathBlock && pixel < P.cam.w * P.cam.h, 3)) {
         long long *o = P.ad_planes + (size_t)pixel * kAdaptivePlanes;
         o[0] += a[0]; o[1] += a[1]; o[2] += a[2];
@@ -546,9 +512,7 @@ __global__ void __launch_bounds__(kPathBlock, kPathMinBlocks) path_megakernel_po
     TraversalCounters ctr;
     Hit best{0.0, kNoHit};
     while (pool_shade_and_advance<MOMENTS, ADAPTIVE>(P, tm, tp, total_items, best, L, ray)) {
-        // world.hit_by(ray, Interval::with_min(0.00001))  (camera.h:217)
-        best = closest_hit<STACK, COUNT, LEAF_FIRST>(P.scene, ray.ox, ray.oy, ray.oz, ray.dx, ray.dy, ray.dz, 0.00001,
-                                                  __longlong_as_double(0x7ff0000000000000LL), &ctr);
+        best = closest_hit<STACK, COUNT, LEAF_FIRST>(P.scene, ray.ox, ray.oy, ray.oz, ray.dx, ray.dy, ray.dz, kRayTmin, kRayTmax, &ctr);
     }
     __syncthreads();
     const uint32_t slot = tp.slot;
@@ -573,9 +537,7 @@ __global__ void __launch_bounds__(kPathBlock, kPathMinBlocks) path_megakernel(co
     Hit best{0.0, kNoHit};
     if (m.valid && C.max_depth > 0 && P.sample_count > 0) {
         while (shade_and_advance(P, m, best, L)) {
-            // world.hit_by(ray, Interval::with_min(0.00001))  (camera.h:217)
-            best = closest_hit<STACK, COUNT>(P.scene, L.ray.ox, L.ray.oy, L.ray.oz, L.ray.dx, L.ray.dy, L.ray.dz, 0.00001,
-                                             __longlong_as_double(0x7ff0000000000000LL), &ctr);
+            best = closest_hit<STACK, COUNT>(P.scene, L.ray.ox, L.ray.oy, L.ray.oz, L.ray.dx, L.ray.dy, L.ray.dz, kRayTmin, kRayTmax, &ctr);
         }
     }
     write_pixel_and_counters(P, m, L.sum_r, L.sum_g, L.sum_b, L.rays, COUNT, ctr);
@@ -620,10 +582,10 @@ __global__ void __launch_bounds__(kPathBlock) path_lanes_kernel(const __grid_con
             bool go;
             if (POOL) {
                 go = pool_shade_and_advance(P, tm, tp, total_items, T.best, Lp, T.ray);
-                if (go) trav_setup(T, 0.00001, __longlong_as_double(0x7ff0000000000000LL));
+                if (go) trav_setup(T, kRayTmin, kRayTmax);
             } else {
                 go = shade_and_advance(P, m, T.best, L);
-                if (go) trav_init(T, L.ray.ox, L.ray.oy, L.ray.oz, L.ray.dx, L.ray.dy, L.ray.dz, 0.00001, __longlong_as_double(0x7ff0000000000000LL));
+                if (go) trav_init(T, L.ray.ox, L.ray.oy, L.ray.oz, L.ray.dx, L.ray.dy, L.ray.dz, kRayTmin, kRayTmax);
             }
             if (go) a[15]++;
             else { finished = true; T.cur = kTravDone; }
@@ -886,7 +848,8 @@ __global__ void __launch_bounds__(kPathBlock) adaptive_judge_kernel(const __grid
     const size_t mw = (size_t)tile * kAdaptiveMaskWords + (lp >> 5);
     bool unconv = false;
     if (((A.mask[mw] >> lane) & 1u) && B200RT_CHECK(S, lp < tm.n_valid, 3)) {
-        const uint32_t pixel = (tm.y0 + lp / tm.vw) * A.w + tm.x0 + lp % tm.vw;
+        const uint2 xy = tile_xy(tm, lp);
+        const uint32_t pixel = xy.y * A.w + xy.x;
         A.counts[pixel] = n;
         if (judge) unconv = !pixel_converged(A, A.planes + (size_t)pixel * kAdaptivePlanes, n);
     }
@@ -907,7 +870,8 @@ __global__ void __launch_bounds__(kPathBlock) adaptive_decide_kernel(const __gri
     const size_t mw = (size_t)tile * kAdaptiveMaskWords + (lp >> 5);
     bool keep = false;
     if (((A.mask[mw] >> lane) & 1u) && lp < tm.n_valid) {
-        const int px = (int)(tm.x0 + lp % tm.vw), py = (int)(tm.y0 + lp / tm.vw);
+        const uint2 xy = tile_xy(tm, lp);
+        const int px = (int)xy.x, py = (int)xy.y;
         for (int qy = max(py - 1, 0); qy <= min(py + 1, (int)A.h - 1); ++qy)
             for (int qx = max(px - 1, 0); qx <= min(px + 1, (int)A.w - 1); ++qx) {
                 const uint32_t tq = (uint32_t)qy / (uint32_t)kPathTileH * tiles_x + (uint32_t)qx / (uint32_t)kPathTileW;

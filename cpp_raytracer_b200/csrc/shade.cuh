@@ -9,6 +9,7 @@
 // distributions are identical (uniform on the unit sphere / in the unit disk), the streams
 // necessarily are not.
 #pragma once
+#include "../../include/b200rt.h"
 #include "rng.cuh"
 #include "traverse.cuh"
 
@@ -96,12 +97,12 @@ __device__ __forceinline__ bool shade_hit(const DeviceScene &S, const Hit &h, co
 #endif
     const float4 m0 = __ldg((const float4 *)(S.materials + mat_id));
     const uint32_t kind = __float_as_uint(m0.w);
-    if (kind == 3u) {   // DiffuseLight: emits on both faces, never scatters (material.h:248-263)
+    if (kind == B200RT_MAT_LIGHT) {   // DiffuseLight: emits on both faces, never scatters (material.h:248-263)
         acc_r += p.tr * m0.x; acc_g += p.tg * m0.y; acc_b += p.tb * m0.z;
         return false;
     }
     double sx, sy, sz;
-    if (kind == 0u) {   // Lambertian (material.h:64-86)
+    if (kind == B200RT_MAT_LAMBERTIAN) {   // Lambertian (material.h:64-86)
         double ux, uy, uz;
         sample_unit_sphere(u01(rnd.x), u01(rnd.y), ux, uy, uz);
         sx = nx + ux; sy = ny + uy; sz = nz + uz;
@@ -114,7 +115,7 @@ __device__ __forceinline__ bool shade_hit(const DeviceScene &S, const Hit &h, co
         const double vdotn = vx * nx + vy * ny + vz * nz;
         // reflected(v, n) = v - 2*dot(v,n)*n (vec3d.h:144-155)
         const double rx = vx - (2 * vdotn) * nx, ry = vy - (2 * vdotn) * ny, rz = vz - (2 * vdotn) * nz;
-        if (kind == 1u) {   // Metal (material.h:116-139)
+        if (kind == B200RT_MAT_METAL) {   // Metal (material.h:116-139)
             const double fuzz = __ldg(&S.materials[mat_id].param);
             double ux, uy, uz;
             sample_unit_sphere(u01(rnd.x), u01(rnd.y), ux, uy, uz);

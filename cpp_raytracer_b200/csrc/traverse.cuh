@@ -205,7 +205,7 @@ __device__ __forceinline__ bool trav_at_leaf(const Trav &T) { return (T.cur & kL
 __device__ __forceinline__ bool trav_done(const Trav &T) { return T.cur == kTravDone; }
 
 // double -> float rounded towards -inf / +inf, written with plain casts and integer steps so that it
-// constant-folds when the argument is a literal (the path kernel's tmin = 0.00001, tmax = inf): the
+// constant-folds when the argument is a compile-time constant (the path kernels' kRayTmin / kRayTmax, path.cuh): the
 // cvt.rd / cvt.ru intrinsics do not fold, and under the 64-register cap the compiler then re-executes the
 // conversion (an XU-pipe instruction) in every node step instead of keeping the value in a register.
 __device__ __forceinline__ float float_toward(double x, bool up) {
@@ -373,7 +373,25 @@ __device__ __forceinline__ uint32_t trav_leaf_step(const DeviceScene &S, Trav &T
 // node-then-leaf C1 +6.5 %, C2 +5.7 %, C3 +4.6 %, C4 -1.3 %, C4b -1 %, C5 +4.4 %; leaf-then-node C1 +6.5 %, C2 +3.7 %,
 // C3 +4.7 %, C4 0 %, C4b +2.5 %, C5 +3.2 %.  The launcher uses leaf-first when quads outnumber spheres.  Two steps of a
 // kind per iteration (L N L, N L N) lose again (-1 ... +1 %), and so did round 1's while-while form, which these loops
-// replace even on the depth-3 Cornell tree (+4.6 % over it).
+// replace even on the depth-3 Cornell tree (+4.6 % over it).  With COUNT the steps are counted into *ctr.
+template <bool COUNT>
+__device__ __forceinline__ void trav_node_counted(const DeviceScene &S, Trav &T, uint2 *stack, TraversalCounters *ctr) {
+    if (trav_at_node(T)) { if (COUNT) ctr->nodes++; trav_node_step(S, T, stack); }
+}
+template <bool COUNT>
+__device__ __forceinline__ void trav_leaf_counted(const DeviceScene &S, Trav &T, uint2 *stack, TraversalCounters *ctr) {
+    if (trav_at_leaf(T)) {
+        const bool is_quad = T.cur & kQuadFlagD;
+        const uint32_t c = trav_leaf_step(S, T, stack);
+        if (COUNT) { ctr->prims += c; if (is_quad) ctr->quads += c; }
+    }
+}
+template <bool COUNT, bool LEAF_FIRST = false>
+__device__ __forceinline__ void trav_iteration(const DeviceScene &S, Trav &T, uint2 *stack, TraversalCounters *ctr) {
+    if (LEAF_FIRST) { trav_leaf_counted<COUNT>(S, T, stack, ctr); trav_node_counted<COUNT>(S, T, stack, ctr); }
+    else { trav_node_counted<COUNT>(S, T, stack, ctr); trav_leaf_counted<COUNT>(S, T, stack, ctr); }
+}
+
 template <int STACK, bool COUNT, bool LEAF_FIRST = false>
 __device__ __forceinline__ Hit closest_hit(const DeviceScene &S, double ox, double oy, double oz,
                                            double dx, double dy, double dz, double tmin, double tmax,
@@ -381,18 +399,7 @@ __device__ __forceinline__ Hit closest_hit(const DeviceScene &S, double ox, doub
     Trav T;
     uint2 stack[STACK];
     trav_init(T, ox, oy, oz, dx, dy, dz, tmin, tmax);
-#define B200RT_NODE_ if (trav_at_node(T)) { if (COUNT) ctr->nodes++; trav_node_step(S, T, stack); }
-#define B200RT_LEAF_ if (trav_at_leaf(T)) {                                                     \
-        const bool is_quad = T.cur & kQuadFlagD;                                                \
-        const uint32_t c = trav_leaf_step(S, T, stack);                                         \
-        if (COUNT) { ctr->prims += c; if (is_quad) ctr->quads += c; }                           \
-    }
-    while (!trav_done(T)) {
-        if (LEAF_FIRST) { B200RT_LEAF_ B200RT_NODE_ }
-        else { B200RT_NODE_ B200RT_LEAF_ }
-    }
-#undef B200RT_NODE_
-#undef B200RT_LEAF_
+    while (!trav_done(T)) trav_iteration<COUNT, LEAF_FIRST>(S, T, stack, ctr);
     return T.best;
 }
 

@@ -1,8 +1,8 @@
 // wavefront.cu -- the wavefront variant of the path kernel (B200RT_VARIANT_WAVEFRONT).
 //
-// Same path semantics and the SAME random streams as path_megakernel (Philox keyed by seed,
-// pixel, sample, bounce), so both variants compute identical per-path radiance; images differ only
-// by FP32 summation order (frame accumulation here is atomic).  What changes is the execution
+// A path is started and advanced by the same functions as in the other path kernels (path.cuh), so
+// all of them compute identical per-path radiance; images differ only by FP32 summation order
+// (frame accumulation here is atomic).  What changes is the execution
 // shape, aimed at the two divergence sources ncu shows in the megakernel (12 of 32 threads active
 // per instruction; material code at 6-7):
 //
@@ -26,7 +26,7 @@
 #include <cstdlib>
 
 #include "kernels.h"
-#include "shade.cuh"
+#include "path.cuh"
 
 namespace b200rt {
 
@@ -62,11 +62,9 @@ __device__ __forceinline__ void wf_spawn(const RenderParams &P, PathSlot *s, uns
     const CameraParams &C = P.cam;
     uint32_t pixel, smp;
     item_to_pixel_sample(item, C.w * C.h, pixel, smp);
-    const uint32_t px = pixel % C.w, py = pixel / C.w;
-    const Philox4 rnd = philox4x32_10(pixel, P.sample_begin + smp, 0u, 0u, (uint32_t)P.seed, (uint32_t)(P.seed >> 32));
     Ray r;
     PathState p;
-    camera_ray(C, px, py, rnd, r, p);
+    path_start(P, pixel, pixel % C.w, pixel / C.w, smp, r, p);
     slot_store_ray(s, r);
     reinterpret_cast<uint4 *>(s)[3] = make_uint4(0u, 0u, kNoHit, pixel);                              // hit_t, hit_ref, pixel
     reinterpret_cast<float4 *>(s)[4] = make_float4(p.tr, p.tg, p.tb, __uint_as_float(smp));          // throughput, sample
@@ -91,7 +89,6 @@ __global__ void __launch_bounds__(kPathBlock, kPathMinBlocks) wf_trace(const __g
     Trav T;
     uint2 stack[STACK];
     T.cur = kTravDone;
-    const uint32_t lane = threadIdx.x & 31u;
     const uint32_t warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, n_warps = (gridDim.x * blockDim.x) >> 5;
     const uint32_t per_warp = (W.n_slots + n_warps - 1) / n_warps;
     uint32_t cursor = warp * per_warp;                                   // warp-uniform
@@ -111,7 +108,8 @@ __global__ void __launch_bounds__(kPathBlock, kPathMinBlocks) wf_trace(const __g
                     const uint32_t mat = (T.best.ref & kQuadFlagD) ? __ldg(&P.scene.quad_meta[T.best.ref & ~kQuadFlagD]).y
                                                                    : __ldg(&P.scene.sphere_meta[T.best.ref]).y;
                     const uint32_t kind = __ldg(&P.scene.materials[mat].kind);
-                    cls = kind == 3u ? WF_LIGHT : (kind == 0u ? WF_LAMBERT : (kind == 1u ? WF_METAL : WF_DIELECTRIC));
+                    cls = kind == B200RT_MAT_LIGHT ? WF_LIGHT
+                          : (kind == B200RT_MAT_LAMBERTIAN ? WF_LAMBERT : (kind == B200RT_MAT_METAL ? WF_METAL : WF_DIELECTRIC));
                 }
                 PathSlot *s = W.slots + slot;
                 s->hit_t = T.best.t;
@@ -129,7 +127,7 @@ __global__ void __launch_bounds__(kPathBlock, kPathMinBlocks) wf_trace(const __g
                     if (s->pixel != kDeadPixel) {
                         Ray r;
                         slot_load_ray(s, r);
-                        trav_init(T, r.ox, r.oy, r.oz, r.dx, r.dy, r.dz, 0.00001, __longlong_as_double(0x7ff0000000000000LL));   // camera.h:217
+                        trav_init(T, r.ox, r.oy, r.oz, r.dx, r.dy, r.dz, kRayTmin, kRayTmax);
                         have = true;
                     }
                 }
@@ -138,28 +136,11 @@ __global__ void __launch_bounds__(kPathBlock, kPathMinBlocks) wf_trace(const __g
             }
         }
         if (have) {
-            if (trav_at_node(T)) {          // node step, then -- same iteration -- the leaf it may have landed on (see closest_hit)
-                if (COUNT) ctr.nodes++;
-                trav_node_step(P.scene, T, stack);
-            }
-            if (trav_at_leaf(T)) {
-                const bool is_quad = T.cur & kQuadFlagD;
-                const uint32_t c = trav_leaf_step(P.scene, T, stack);
-                if (COUNT) { ctr.prims += c; if (is_quad) ctr.quads += c; }
-            }
+            trav_iteration<COUNT>(P.scene, T, stack, &ctr);
             if (trav_done(T)) { have = false; parked = true; ++rays; }
         }
     }
-    unsigned long long r = rays;
-    for (int off = 16; off; off >>= 1) r += __shfl_down_sync(0xffffffffu, r, off);
-    if (lane == 0 && r) atomicAdd(&P.counters[0], r);
-    if (COUNT) {
-        unsigned long long a = ctr.nodes, b = ctr.prims, q = ctr.quads;
-        for (int off = 16; off; off >>= 1) {
-            a += __shfl_down_sync(0xffffffffu, a, off); b += __shfl_down_sync(0xffffffffu, b, off); q += __shfl_down_sync(0xffffffffu, q, off);
-        }
-        if (lane == 0) { atomicAdd(&P.counters[1], a); atomicAdd(&P.counters[2], b); atomicAdd(&P.counters[3], q); }
-    }
+    write_counters(P, rays, COUNT, ctr);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -199,7 +180,6 @@ __global__ void __launch_bounds__(kSortBlock) wf_sort(const WavefrontPool W) {
 // wf_shade: one thread per queue entry; the five queues are walked back to back, so all lanes of
 // a warp (except at the four boundaries) shade the same material class.
 __global__ void __launch_bounds__(128) wf_shade(const __grid_constant__ RenderParams P, const WavefrontPool W) {
-    const CameraParams &C = P.cam;
     uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     uint32_t cls = 0;
     bool valid = false;
@@ -218,18 +198,11 @@ __global__ void __launch_bounds__(128) wf_shade(const __grid_constant__ RenderPa
     uint32_t bounce = s->bounce;
     const uint32_t pixel = hq.w, smp = __float_as_uint(th.w);
     PathState p{th.x, th.y, th.z};
-    float add_r = 0.f, add_g = 0.f, add_b = 0.f;
-    bool cont = false;
+    const Hit h{__hiloint2double((int)hq.y, (int)hq.x), hq.z};
     Ray r;
-    if (cls == WF_MISS) {
-        add_r = p.tr * C.background[0]; add_g = p.tg * C.background[1]; add_b = p.tb * C.background[2];   // camera.h:248
-    } else {
-        slot_load_ray(s, r);
-        const Hit h{__hiloint2double((int)hq.y, (int)hq.x), hq.z};
-        const Philox4 rnd = philox4x32_10(pixel, P.sample_begin + smp, bounce + 1u, 0u, (uint32_t)P.seed, (uint32_t)(P.seed >> 32));
-        cont = shade_hit(P.scene, h, rnd, r, p, add_r, add_g, add_b);
-        if (cont && ++bounce == C.max_depth) cont = false;   // camera.h:211-213
-    }
+    if (h.ref != kNoHit) slot_load_ray(s, r);
+    float add_r, add_g, add_b;
+    const bool cont = path_bounce(P, h, pixel, smp, bounce, r, p, add_r, add_g, add_b);
     if (add_r != 0.f || add_g != 0.f || add_b != 0.f) {
         float *o = P.out + (size_t)pixel * 3;
         atomicAdd(o + 0, add_r * P.scale); atomicAdd(o + 1, add_g * P.scale); atomicAdd(o + 2, add_b * P.scale);
