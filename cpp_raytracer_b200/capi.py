@@ -51,7 +51,7 @@ class SceneInfo(C.Structure):
     _fields_ = [("n_prims", C.c_uint64), ("n_spheres", C.c_uint64), ("n_quads", C.c_uint64),
                 ("n_materials", C.c_uint64), ("n_nodes", C.c_uint64), ("device_bytes", C.c_uint64),
                 ("tree_depth", C.c_uint32), ("stack_entries", C.c_uint32),
-                ("build_ms", C.c_double), ("upload_ms", C.c_double)]
+                ("build_ms", C.c_double), ("upload_ms", C.c_double), ("n_hoisted", C.c_uint32)]
 
     def as_dict(self):
         return {k: getattr(self, k) for k, _ in self._fields_}

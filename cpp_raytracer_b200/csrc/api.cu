@@ -27,8 +27,8 @@ using namespace b200rt;
 
 namespace b200rt {
 cudaError_t build_lbvh_device(const B200rtSphere *d_sph, uint32_t n_sph, const B200rtQuad *d_quads, uint32_t n_quad,
-                              uint32_t *sphere_order, uint32_t *quad_order, float4 **nodes_out, uint32_t *n_nodes_out,
-                              uint32_t *depth_out);
+                              uint32_t max_hoisted, uint32_t *sphere_order, uint32_t *quad_order, float4 **nodes_out,
+                              uint32_t *n_nodes_out, uint32_t *depth_out, uint32_t *n_hoisted_out, uint32_t hoisted_ref_out[kMaxHoisted]);
 cudaError_t assemble_scene_device(const B200rtSphere *sph, const uint32_t *sphere_order, uint32_t n_sph, const B200rtQuad *quads,
                                   const uint32_t *quad_order, uint32_t n_quad, const B200rtMaterial *mats, uint32_t n_mat,
                                   double2 *out_sph, uint2 *out_sph_meta, double2 *out_quads, uint2 *out_quad_meta,
@@ -367,6 +367,13 @@ int plan_tail(SceneImpl *s, const CameraParams &C, PathMode mode, bool leaf_firs
     return B200RT_OK;
 }
 
+// Scene-spanning primitives the builders take out of the tree (bvh_builder.h spanning_key): up to kMaxHoisted by
+// default.  B200RT_HOISTED=0 keeps every primitive in the tree, for A/B measurements and tests.
+uint32_t max_hoisted() {
+    const char *e = std::getenv("B200RT_HOISTED");
+    return e ? (uint32_t)std::max(0ll, std::min<long long>(std::atoll(e), kMaxHoisted)) : kMaxHoisted;
+}
+
 // Points P at the scene's tail scratch for `tail_tiles` tiles, growing it if needed.  Renders of one scene share the
 // scratch: the caller's stream waits (on the device) until the previous render is done with it.  Every launch leaves it zero.
 cudaError_t tail_scratch(SceneImpl *s, uint32_t tail_tiles, bool moments, cudaStream_t st, RenderParams *P) {
@@ -495,9 +502,13 @@ int render_on_device(SceneImpl *s, const B200rtCamera *cam, const B200rtRenderOp
     return B200RT_OK;
 }
 
-// Points s->d at the arrays in s->allocs, takes `info`, sizes the traversal stack from the tree depth and creates the
-// per-scene launch state (counters, events, the bounds-check table of the debug build); `s->device` is current.
-int finish_scene(SceneImpl *s, const B200rtSceneInfo &info) {
+// Points s->d at the arrays in s->allocs, takes `info` and the info.n_hoisted references of the scene-spanning primitives,
+// sizes the traversal stack from the tree depth and creates the per-scene launch state (counters, events, the
+// bounds-check table of the debug build); `s->device` is current.
+int finish_scene(SceneImpl *s, const B200rtSceneInfo &info, const uint32_t *hoisted_ref) {
+    static_assert(sizeof(s->d.hoisted_ref) / sizeof(s->d.hoisted_ref[0]) == kMaxHoisted, "DeviceScene::hoisted_ref");
+    s->d.n_hoisted = info.n_hoisted;
+    for (uint32_t k = 0; k < kMaxHoisted; ++k) s->d.hoisted_ref[k] = k < info.n_hoisted ? hoisted_ref[k] : 0u;
     s->d.nodes = static_cast<const float4 *>(s->allocs[0]);
     s->d.spheres = static_cast<const double2 *>(s->allocs[1]);
     s->d.sphere_meta = static_cast<const uint2 *>(s->allocs[2]);
@@ -567,19 +578,20 @@ int scene_build(const B200rtSceneDesc *desc, const B200rtBuildOpts *opts, bool g
     CUDA_TRY(staged_upload(raw.quad, desc->quads, (size_t)n_quad * sizeof(B200rtQuad), 0));
     CUDA_TRY(staged_upload(raw.mat, desc->materials, (size_t)n_mat * sizeof(B200rtMaterial), 0));
     uint32_t *sphere_order = raw.order, *quad_order = raw.order + n_sph;
-    uint32_t n_nodes = 0, depth = 0;
+    uint32_t n_nodes = 0, depth = 0, n_hoisted = 0, hoisted_ref[kMaxHoisted] = {};
     bool have_tree = false;
     if (gpu_build) {
         const bool trace = std::getenv("B200RT_TRACE") != nullptr;
         if (trace) cudaStreamSynchronize(0);
         const double t_up = now_ms();
         float4 *d_nodes = nullptr;
-        const cudaError_t e = build_lbvh_device(raw.sph, n_sph, raw.quad, n_quad, sphere_order, quad_order, &d_nodes, &n_nodes, &depth);
+        const cudaError_t e = build_lbvh_device(raw.sph, n_sph, raw.quad, n_quad, max_hoisted(), sphere_order, quad_order, &d_nodes,
+                                                &n_nodes, &depth, &n_hoisted, hoisted_ref);
         if (e != cudaSuccess) { cudaGetLastError(); return fail(B200RT_ECUDA, std::string("GPU BVH build: ") + cudaGetErrorString(e)); }
         if (trace) std::fprintf(stderr, "scene_build: upload %.2f ms, lbvh %.2f ms, depth %u\n", t_up - t0, now_ms() - t_up, depth);
-        have_tree = 3 * depth <= 128;
+        have_tree = n_nodes && 3 * depth <= 128;
         if (!have_tree) {
-            dev_free(d_nodes);   // pathological depth: the depth-capped host builder below takes over
+            dev_free(d_nodes);   // pathological depth, or too few primitives left for a radix tree: the host builder below takes over
         } else if (s->peer_visible) {
             // the builder sized the node array for the worst case (n - 1 nodes) in pool memory; a multi-device scene
             // keeps an exact-size copy in a peer-visible buffer instead (a device-to-device copy at HBM speed)
@@ -599,9 +611,11 @@ int scene_build(const B200rtSceneDesc *desc, const B200rtBuildOpts *opts, bool g
         compute_boxes(desc, boxes, host_threads(opts));
         BuiltBVH bvh;
         const char *err = nullptr;
-        if (!build_bvh4(boxes, desc->n_spheres, desc->n_quads, build_params(opts), bvh, &err))
+        if (!build_bvh4(boxes, desc->n_spheres, desc->n_quads, select_spanning(boxes, max_hoisted()), build_params(opts), bvh, &err))
             return fail(B200RT_EINVAL, std::string("BVH build failed: ") + (err ? err : "?"));
         host_ms = now_ms() - t1;
+        n_hoisted = (uint32_t)bvh.hoisted_ref.size();
+        std::copy(bvh.hoisted_ref.begin(), bvh.hoisted_ref.end(), hoisted_ref);
         n_nodes = (uint32_t)bvh.nodes.size();
         depth = bvh.depth;
         if (3 * depth > 128) return fail(B200RT_EINTERNAL, "BVH deeper than the largest traversal stack");
@@ -622,10 +636,11 @@ int scene_build(const B200rtSceneDesc *desc, const B200rtBuildOpts *opts, bool g
     info.n_spheres = n_sph; info.n_quads = n_quad; info.n_materials = n_mat;
     info.n_nodes = n_nodes;
     info.tree_depth = depth;
+    info.n_hoisted = n_hoisted;
     const double total = now_ms() - t0;
     info.build_ms = host_ms >= 0 ? host_ms : total;
     info.upload_ms = total - info.build_ms;
-    return finish_scene(s, info);
+    return finish_scene(s, info, hoisted_ref);
 }
 
 // Builds the acceleration structure for `desc` (structure already validated) and makes the scene resident on device `dev`.
@@ -666,7 +681,7 @@ int replicate_scene_on(const SceneImpl *src, int dev, SceneImpl **out) {
             return fail(e == cudaErrorMemoryAllocation ? B200RT_ENOMEM : B200RT_ECUDA, std::string("scene copy to a peer device: ") + cudaGetErrorString(e));
         }
     }
-    if (int rc = finish_scene(s, src->info)) { free_scene(s); return rc; }
+    if (int rc = finish_scene(s, src->info, src->d.hoisted_ref)) { free_scene(s); return rc; }
     *out = s;
     return B200RT_OK;
 }
@@ -1370,7 +1385,8 @@ int b200rt_tonemap(const float *hdr, int64_t n_pixels, int32_t *out, int clamp) 
 }
 
 // ---- CPU-side self test of the host builder (no GPU needed; used by tests -m "not gpu") -------
-// Builds the BVH for `desc` and checks its structural invariants.  Fills depth / node count.
+// Builds the BVH for `desc`, with the scene-spanning primitives taken out as scene creation takes them out, and checks its
+// structural invariants.  Fills depth / node count / hoisted count.
 int b200rt_selftest_bvh(const B200rtSceneDesc *desc, const B200rtBuildOpts *opts, B200rtSceneInfo *info) {
     if (int rc = validate_desc(desc)) return rc;
     std::vector<Box3> boxes;
@@ -1378,7 +1394,7 @@ int b200rt_selftest_bvh(const B200rtSceneDesc *desc, const B200rtBuildOpts *opts
     BuiltBVH bvh;
     const char *err = nullptr;
     const double t0 = now_ms();
-    if (!build_bvh4(boxes, desc->n_spheres, desc->n_quads, build_params(opts), bvh, &err))
+    if (!build_bvh4(boxes, desc->n_spheres, desc->n_quads, select_spanning(boxes, max_hoisted()), build_params(opts), bvh, &err))
         return fail(B200RT_EINVAL, std::string("BVH build failed: ") + (err ? err : "?"));
     const double t1 = now_ms();
     if (!validate_bvh4(bvh, boxes, desc->n_spheres, desc->n_quads, &err))
@@ -1391,6 +1407,7 @@ int b200rt_selftest_bvh(const B200rtSceneDesc *desc, const B200rtBuildOpts *opts
         info->tree_depth = bvh.depth;
         info->stack_entries = 3 * bvh.depth;
         info->build_ms = t1 - t0;
+        info->n_hoisted = (uint32_t)bvh.hoisted_ref.size();
     }
     return B200RT_OK;
 }

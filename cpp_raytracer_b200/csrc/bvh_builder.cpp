@@ -10,6 +10,7 @@
 #include <cstdlib>
 #include <cmath>
 #include <cstring>
+#include <functional>
 #include <limits>
 
 #include "thread_pool.h"
@@ -440,12 +441,33 @@ void collapse_tree(const Builder &B, int threads, uint64_t n, BuiltBVH &out) {
 
 }  // namespace
 
+std::vector<uint32_t> select_spanning(const std::vector<Box3> &prim_boxes, uint32_t max_hoisted) {
+    const size_t n = prim_boxes.size();
+    const size_t keep = std::min<size_t>(std::min(max_hoisted, kMaxHoisted), n ? n - 1 : 0);
+    if (!keep) return {};
+    Box3 scene = empty_box();
+    for (const Box3 &b : prim_boxes) grow(scene, b);
+    std::vector<uint64_t> keys;
+    for (size_t i = 0; i < n; ++i)
+        if (const uint64_t k = spanning_key(prim_boxes[i].lo, prim_boxes[i].hi, scene.lo, scene.hi, (uint32_t)i)) keys.push_back(k);
+    std::sort(keys.begin(), keys.end(), std::greater<uint64_t>());
+    std::vector<uint32_t> out;
+    for (size_t k = 0; k < keys.size() && k < keep; ++k) out.push_back(0xFFFFFFFFu - (uint32_t)keys[k]);
+    return out;
+}
+
 bool build_bvh4(const std::vector<Box3> &prim_boxes, uint64_t n_spheres, uint64_t n_quads,
-                const BuildParams &params_in, BuiltBVH &out, const char **err) {
-    const uint64_t n = n_spheres + n_quads;
+                const std::vector<uint32_t> &hoisted, const BuildParams &params_in, BuiltBVH &out, const char **err) {
+    const uint64_t n_all = n_spheres + n_quads, n = n_all - hoisted.size();   // n: primitives in the tree
     out = BuiltBVH{};
-    if (prim_boxes.size() != n) { *err = "prim_boxes size mismatch"; return false; }
+    if (prim_boxes.size() != n_all) { *err = "prim_boxes size mismatch"; return false; }
     if (n_spheres > kLeafIndexMask || n_quads > kLeafIndexMask) { *err = "too many primitives for the leaf encoding (max 2^26 per type)"; return false; }
+    std::vector<uint8_t> is_hoisted(n_all, 0);
+    for (uint32_t p : hoisted) {
+        if (p >= n_all || is_hoisted[p]) { *err = "hoisted primitive out of range or listed twice"; return false; }
+        is_hoisted[p] = 1;
+    }
+    if (n_all && !n) { *err = "every primitive hoisted"; return false; }
     BuildParams P = params_in;
     P.max_leaf_prims = std::clamp(P.max_leaf_prims, 1, kMaxLeafPrims);
     P.sah_bins = std::clamp(P.sah_bins, 4, 64);
@@ -466,8 +488,9 @@ bool build_bvh4(const std::vector<Box3> &prim_boxes, uint64_t n_spheres, uint64_
     }
 
     Builder B(prim_boxes, n_spheres, P);
-    B.idx.resize(n);
-    for (uint64_t i = 0; i < n; ++i) B.idx[i] = (uint32_t)i;
+    B.idx.reserve(n);
+    for (uint64_t i = 0; i < n_all; ++i)
+        if (!is_hoisted[i]) B.idx.push_back((uint32_t)i);
     B.nodes.resize(2 * n);
     B.n_nodes = 1;
     const auto t_start = std::chrono::steady_clock::now();
@@ -494,6 +517,12 @@ bool build_bvh4(const std::vector<Box3> &prim_boxes, uint64_t n_spheres, uint64_
         out.depth = 1;
     } else {
         collapse_tree(B, threads, n, out);
+    }
+    for (uint32_t p : hoisted) {
+        const bool quad = p >= n_spheres;
+        std::vector<uint32_t> &order = quad ? out.quad_order : out.sphere_order;
+        out.hoisted_ref.push_back((quad ? kQuadFlag : 0u) | (uint32_t)order.size());
+        order.push_back(quad ? (uint32_t)(p - n_spheres) : p);
     }
     if (out.sphere_order.size() != n_spheres || out.quad_order.size() != n_quads) { *err = "internal: leaf order size mismatch"; return false; }
     if (std::getenv("B200RT_BUILD_TIMING")) {
@@ -548,6 +577,21 @@ bool validate_bvh4(const BuiltBVH &bvh, const std::vector<Box3> &prim_boxes, uin
                 stack.push_back({(int32_t)c, it.depth + 1, slot});
             }
         }
+    }
+    // the hoisted primitives: the last of their type in the leaf order, each in no leaf
+    size_t hoisted_of[2] = {0, 0};
+    for (uint32_t r : bvh.hoisted_ref) hoisted_of[(r & kQuadFlag) ? 1 : 0]++;
+    for (uint32_t r : bvh.hoisted_ref) {
+        const bool quad = r & kQuadFlag;
+        const auto &order = quad ? bvh.quad_order : bvh.sphere_order;
+        const uint32_t pos = r & kLeafIndexMask;
+        if ((r & ~(kQuadFlag | kLeafIndexMask)) || pos >= order.size() || pos < order.size() - hoisted_of[quad ? 1 : 0]) {
+            *err = "hoisted reference is not among the last of its type in the leaf order"; return false;
+        }
+        auto &seen = quad ? seen_q : seen_s;
+        const uint32_t p = order[pos];
+        if (p >= seen.size() || seen[p]) { *err = "hoisted primitive also in the tree, or out of range"; return false; }
+        seen[p] = 1;
     }
     for (auto s : seen_s) if (!s) { *err = "sphere missing from the tree"; return false; }
     for (auto s : seen_q) if (!s) { *err = "quad missing from the tree"; return false; }

@@ -552,7 +552,8 @@ __global__ void __launch_bounds__(kPathBlock, kPathMinBlocks) path_megakernel(co
 //   acc[2] node-step executions       acc[3] lanes at a node     acc[4] idle: at a leaf   acc[5] idle: traversal done,
 //                                                                waiting for the round    acc[6] idle: pixel out of samples
 //   acc[7] leaf-step executions       acc[8] lanes at a leaf     acc[9] idle: at a node   acc[10] idle: done   acc[11] idle: finished
-//   acc[12] primitive-test executions (a leaf step loops over its primitives)            acc[13] lanes taking part
+//   acc[12] primitive-test executions (a leaf step loops over its primitives; each       acc[13] lanes taking part
+//           scene-spanning primitive, traverse.cuh trav_hoisted, is one more per round)
 //   acc[14] warps   acc[15] lane-rounds (shade calls that started a ray)
 // Same Philox keys and the same arithmetic as path_megakernel, so it also writes the same image.
 template <int STACK, bool POOL>
@@ -578,8 +579,8 @@ __global__ void __launch_bounds__(kPathBlock) path_lanes_kernel(const __grid_con
         const unsigned ms = __ballot_sync(full, !finished);
         if (!ms) break;
         a[0]++; a[1] += __popc(ms);
+        bool go = false;
         if (!finished) {
-            bool go;
             if (POOL) {
                 go = pool_shade_and_advance(P, tm, tp, total_items, T.best, Lp, T.ray);
                 if (go) trav_setup(T, kRayTmin, kRayTmax);
@@ -589,6 +590,11 @@ __global__ void __launch_bounds__(kPathBlock) path_lanes_kernel(const __grid_con
             }
             if (go) a[15]++;
             else { finished = true; T.cur = kTravDone; }
+        }
+        {   // the scene-spanning primitives: one primitive-test execution each, by the lanes that started a ray
+            const unsigned mg = __ballot_sync(full, go);
+            if (mg) { a[12] += P.scene.n_hoisted; a[13] += (unsigned long long)__popc(mg) * P.scene.n_hoisted; }
+            if (go) trav_hoisted<false>(P.scene, T, nullptr);
         }
         while (true) {   // one iteration of closest_hit's loop: both kinds of step, in the product's order
             if (!__ballot_sync(full, !finished && !trav_done(T))) break;

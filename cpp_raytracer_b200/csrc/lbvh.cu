@@ -9,17 +9,21 @@
 // primitive records are laid out in that order by scene_layout.cu, as for the host builder:
 //   1. prim_setup      primitive bounds exactly as the reference's constructors compute them
 //                      (sphere.h:112-123, parallelogram.h:281-295) in double, rounded outward to FP32;
-//                      centroid bounds by warp shuffle + ordered-int atomics
-//   2. morton_codes    63-bit Morton code of the centroid (21 bits per axis)
-//   3. cub radix sort  (key, primitive) pairs                    [library call: a plain sort]
-//   4. radix_tree      Karras 2012, "Maximizing parallelism in the construction of BVHs, octrees and
+//                      the scene's box by warp shuffle + ordered-int atomics
+//   2. spanning_keys,  the scene-spanning primitives the tree leaves out (bvh_builder.h spanning_key):
+//      pick_spanning   one key per primitive, then one atomicMax pass per pick
+//   3. centroid_bounds centroid bounds of the primitives the tree holds
+//   4. morton_codes    63-bit Morton code of the centroid (21 bits per axis); the hoisted primitives sort last
+//   5. cub radix sort  (key, primitive) pairs                    [library call: a plain sort]
+//   6. radix_tree      Karras 2012, "Maximizing parallelism in the construction of BVHs, octrees and
 //                      k-d trees": one thread per internal node, duplicates broken by index
-//   5. fit_boxes       bottom-up union of child boxes, second arrival continues (atomic counters)
-//   6. leaf_order      leaf (= Morton) position -> per-type position: sphere_order / quad_order
-//   7. collapse_level  binary -> 4-wide, breadth first, one launch per level: each task pulls up the
+//   7. fit_boxes       bottom-up union of child boxes, second arrival continues (atomic counters)
+//   8. leaf_order      leaf (= Morton) position -> per-type position: sphere_order / quad_order
+//   9. collapse_level  binary -> 4-wide, breadth first, one launch per level: each task pulls up the
 //                      larger-area grandchildren until four slots are used, reserves its Node4 with an
 //                      atomic counter, patches its parent's child slot and queues its interior children
 // Closest-hit results do not depend on the tree, so the parity tests run against this builder too.
+#include <algorithm>
 #include <cstdio>
 #include <cub/cub.cuh>
 
@@ -44,40 +48,98 @@ struct PrimBoxes {
     float *cx, *cy, *cz;                         // centroid
 };
 
+// Primitive i's box in double, exactly as the reference's constructors compute it (and api.cu's sphere_box / quad_box).
+__device__ __forceinline__ void prim_box(const B200rtSphere *sph, uint32_t n_sph, const B200rtQuad *quads, uint32_t i,
+                                         double lo[3], double hi[3]) {
+    if (i < n_sph) {                                   // sphere.h:112-123
+        const B200rtSphere s = sph[i];
+        for (int a = 0; a < 3; ++a) {
+            const double p = s.c[a] - s.r, q = s.c[a] + s.r;
+            lo[a] = fmin(p, q); hi[a] = fmax(p, q);
+        }
+    } else {                                           // parallelogram.h:281-295 + ensure_min_axis_length(1e-4)
+        const B200rtQuad q = quads[i - n_sph];
+        for (int a = 0; a < 3; ++a) {
+            const double p0 = q.v[a], p1 = q.v[a] + q.s1[a], p2 = q.v[a] + q.s2[a], p3 = (q.v[a] + q.s1[a]) + q.s2[a];
+            lo[a] = fmin(fmin(p0, p1), fmin(p2, p3));
+            hi[a] = fmax(fmax(p0, p1), fmax(p2, p3));
+            const double size = hi[a] - lo[a];
+            if (size < 1e-4) { const double pad = (1e-4 - size) / 2; lo[a] -= pad; hi[a] += pad; }
+        }
+    }
+}
+
+__device__ __forceinline__ long long double_to_ordered(double d) {
+    const long long i = __double_as_longlong(d);
+    return i >= 0 ? i : i ^ 0x7fffffffffffffffll;
+}
+__device__ __forceinline__ double ordered_to_double(long long i) { return __longlong_as_double(i >= 0 ? i : i ^ 0x7fffffffffffffffll); }
+
 __global__ void prim_setup(const B200rtSphere *sph, uint32_t n_sph, const B200rtQuad *quads, uint32_t n_quad, PrimBoxes B,
-                           int *cbounds /* [6]: ordered-int min xyz, max xyz */) {
+                           long long *sbounds /* [6]: ordered-int64 min xyz, max xyz of the primitive boxes */) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     const uint32_t n = n_sph + n_quad;
-    float c[3] = {0.f, 0.f, 0.f};
     const bool valid = i < n;
+    const double inf = __longlong_as_double(0x7ff0000000000000ll);
+    double lo[3] = {inf, inf, inf}, hi[3] = {-inf, -inf, -inf};
     if (valid) {
-        double lo[3], hi[3];
-        if (i < n_sph) {                                   // sphere.h:112-123
-            const B200rtSphere s = sph[i];
-            for (int a = 0; a < 3; ++a) {
-                const double p = s.c[a] - s.r, q = s.c[a] + s.r;
-                lo[a] = fmin(p, q); hi[a] = fmax(p, q);
-            }
-        } else {                                           // parallelogram.h:281-295 + ensure_min_axis_length(1e-4)
-            const B200rtQuad q = quads[i - n_sph];
-            for (int a = 0; a < 3; ++a) {
-                const double p0 = q.v[a], p1 = q.v[a] + q.s1[a], p2 = q.v[a] + q.s2[a], p3 = (q.v[a] + q.s1[a]) + q.s2[a];
-                lo[a] = fmin(fmin(p0, p1), fmin(p2, p3));
-                hi[a] = fmax(fmax(p0, p1), fmax(p2, p3));
-                const double size = hi[a] - lo[a];
-                if (size < 1e-4) { const double pad = (1e-4 - size) / 2; lo[a] -= pad; hi[a] += pad; }
-            }
-        }
+        prim_box(sph, n_sph, quads, i, lo, hi);
         B.lox[i] = __double2float_rd(lo[0]); B.loy[i] = __double2float_rd(lo[1]); B.loz[i] = __double2float_rd(lo[2]);
         B.hix[i] = __double2float_ru(hi[0]); B.hiy[i] = __double2float_ru(hi[1]); B.hiz[i] = __double2float_ru(hi[2]);
-        for (int a = 0; a < 3; ++a) c[a] = (float)(0.5 * lo[a] + 0.5 * hi[a]);
-        B.cx[i] = c[0]; B.cy[i] = c[1]; B.cz[i] = c[2];
+        B.cx[i] = (float)(0.5 * lo[0] + 0.5 * hi[0]); B.cy[i] = (float)(0.5 * lo[1] + 0.5 * hi[1]); B.cz[i] = (float)(0.5 * lo[2] + 0.5 * hi[2]);
     }
-    // centroid bounds: warp reduce, then one atomic per warp and axis
+    // the scene's box (spanning_key): warp reduce, then one atomic per warp and bound
+#pragma unroll
+    for (int a = 0; a < 3; ++a) {
+        double mn = lo[a], mx = hi[a];
+        for (int off = 16; off; off >>= 1) {
+            mn = fmin(mn, __shfl_down_sync(0xffffffffu, mn, off));
+            mx = fmax(mx, __shfl_down_sync(0xffffffffu, mx, off));
+        }
+        if ((threadIdx.x & 31) == 0) {
+            atomicMin(&sbounds[a], double_to_ordered(mn));
+            atomicMax(&sbounds[3 + a], double_to_ordered(mx));
+        }
+    }
+}
+
+// spanning_key of every primitive (0: does not span the scene)
+__global__ void spanning_keys(const B200rtSphere *sph, uint32_t n_sph, const B200rtQuad *quads, uint32_t n, const long long *sbounds,
+                              unsigned long long *keys) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    double lo[3], hi[3], slo[3], shi[3];
+    prim_box(sph, n_sph, quads, i, lo, hi);
+    for (int a = 0; a < 3; ++a) { slo[a] = ordered_to_double(sbounds[a]); shi[a] = ordered_to_double(sbounds[3 + a]); }
+    keys[i] = spanning_key(lo, hi, slo, shi, i);
+}
+
+// Round r of the selection: the largest key below the one round r - 1 picked (0: none left).
+__global__ void pick_spanning(const unsigned long long *keys, uint32_t n, unsigned long long *picked, int r) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const unsigned long long k = keys[i], bound = r ? picked[r - 1] : ~0ull;
+    if (k && k < bound) atomicMax(&picked[r], k);
+}
+
+struct Hoisted {
+    uint32_t n, prim[kMaxHoisted];
+    __device__ __forceinline__ bool has(uint32_t i) const {
+        bool h = false;
+        for (uint32_t k = 0; k < n; ++k) h |= prim[k] == i;
+        return h;
+    }
+};
+
+// Centroid bounds of the primitives the tree holds: warp shuffle + ordered-int atomics.
+__global__ void centroid_bounds(PrimBoxes B, uint32_t n, Hoisted H, int *cbounds /* [6]: ordered-int min xyz, max xyz */) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    const bool valid = i < n && !H.has(i);
+    const float *c[3] = {B.cx, B.cy, B.cz};
     const float inf = __int_as_float(0x7f800000);
 #pragma unroll
     for (int a = 0; a < 3; ++a) {
-        float mn = valid ? c[a] : inf, mx = valid ? c[a] : -inf;
+        float mn = valid ? c[a][i] : inf, mx = valid ? c[a][i] : -inf;
         for (int off = 16; off; off >>= 1) {
             mn = fminf(mn, __shfl_down_sync(0xffffffffu, mn, off));
             mx = fmaxf(mx, __shfl_down_sync(0xffffffffu, mx, off));
@@ -99,9 +161,12 @@ __device__ __forceinline__ unsigned long long spread21(unsigned long long x) {  
     return x;
 }
 
-__global__ void morton_codes(PrimBoxes B, uint32_t n, const int *cbounds, unsigned long long *keys, uint32_t *vals) {
+// The hoisted primitives get bit 63, above every 63-bit code: the sort puts them after the tree's primitives.
+__global__ void morton_codes(PrimBoxes B, uint32_t n, const int *cbounds, Hoisted H, unsigned long long *keys, uint32_t *vals) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
+    vals[i] = i;
+    if (H.has(i)) { keys[i] = ~0ull; return; }
     unsigned long long code = 0;
     const float *c[3] = {B.cx, B.cy, B.cz};
 #pragma unroll
@@ -114,7 +179,6 @@ __global__ void morton_codes(PrimBoxes B, uint32_t n, const int *cbounds, unsign
         code |= spread21(q) << a;
     }
     keys[i] = code;
-    vals[i] = i;
 }
 
 // Common-prefix length of sorted keys i and j (-1 out of range); equal keys are told apart by index.
@@ -265,14 +329,17 @@ __global__ void collapse_level(BinTree T, PrimBoxes B, const uint32_t *vals, con
     }
 }
 
-// the caller's index of the primitive at each leaf (Morton) position, per type
-__global__ void leaf_order(const uint32_t *vals, const uint32_t *quad_rank, uint32_t n, uint32_t n_sph, uint32_t *sphere_order,
-                           uint32_t *quad_order) {
+// the caller's index of the primitive at each leaf (Morton) position, per type; positions from n_tree on hold the hoisted
+// primitives, whose references go to hoisted_ref[p - n_tree]
+__global__ void leaf_order(const uint32_t *vals, const uint32_t *quad_rank, uint32_t n, uint32_t n_tree, uint32_t n_sph,
+                           uint32_t *sphere_order, uint32_t *quad_order, uint32_t *hoisted_ref) {
     const uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= n) return;
     const uint32_t prim = vals[p];
-    if (prim < n_sph) sphere_order[p - quad_rank[p]] = prim;
+    const uint32_t ref = prim < n_sph ? p - quad_rank[p] : kQuadFlag | quad_rank[p];
+    if (prim < n_sph) sphere_order[ref] = prim;
     else quad_order[quad_rank[p]] = prim - n_sph;
+    if (p >= n_tree) hoisted_ref[p - n_tree] = ref;
 }
 
 template <typename T>
@@ -288,12 +355,17 @@ cudaError_t tmp_alloc(std::vector<void *> &owned, T **p, size_t count) {
 }  // namespace
 
 // Builds the 4-wide tree on the GPU.  d_sph / d_quads are the caller's flat structs already on the device.
-// Outputs: the leaf order, sphere_order[n_sph] / quad_order[n_quad] (allocated by the caller); the Node4 array
-// is allocated here (its size is only known at the end) with cudaMallocAsync and handed back through nodes_out.
+// Outputs: the leaf order, sphere_order[n_sph] / quad_order[n_quad] (allocated by the caller), which ends with the up to
+// max_hoisted scene-spanning primitives (spanning_key) the tree leaves out, and their references in
+// hoisted_ref_out[*n_hoisted_out]; the Node4 array is allocated here (its size is only known at the end) with
+// cudaMallocAsync and handed back through nodes_out.  *n_nodes_out = 0 with nothing allocated: the tree would hold fewer
+// than the two primitives a radix tree needs, so the caller builds on the host.
 cudaError_t build_lbvh_device(const B200rtSphere *d_sph, uint32_t n_sph, const B200rtQuad *d_quads, uint32_t n_quad,
-                              uint32_t *sphere_order, uint32_t *quad_order, float4 **nodes_out, uint32_t *n_nodes_out,
-                              uint32_t *depth_out) {
+                              uint32_t max_hoisted, uint32_t *sphere_order, uint32_t *quad_order, float4 **nodes_out,
+                              uint32_t *n_nodes_out, uint32_t *depth_out, uint32_t *n_hoisted_out, uint32_t hoisted_ref_out[kMaxHoisted]) {
     const uint32_t n = n_sph + n_quad;
+    *n_nodes_out = 0;
+    *n_hoisted_out = 0;
     // Encoding limits: a leaf reference holds a 26-bit index into its per-type array (bvh_builder.h), and the radix
     // tree's index arithmetic ((n - 1) + ~child, lmax * d) must stay inside int.  The host builder rejects the same
     // scenes (bvh_builder.cpp); api.cu checks before calling, this is the backstop.
@@ -309,24 +381,46 @@ cudaError_t build_lbvh_device(const B200rtSphere *d_sph, uint32_t n_sph, const B
     LB(tmp_alloc(owned, &pb.lox, n)); LB(tmp_alloc(owned, &pb.loy, n)); LB(tmp_alloc(owned, &pb.loz, n));
     LB(tmp_alloc(owned, &pb.hix, n)); LB(tmp_alloc(owned, &pb.hiy, n)); LB(tmp_alloc(owned, &pb.hiz, n));
     LB(tmp_alloc(owned, &pb.cx, n)); LB(tmp_alloc(owned, &pb.cy, n)); LB(tmp_alloc(owned, &pb.cz, n));
-    int *cbounds;
-    LB(tmp_alloc(owned, &cbounds, 6));
-    const int init[6] = {0x7fffffff, 0x7fffffff, 0x7fffffff, (int)0x80000000, (int)0x80000000, (int)0x80000000};
-    LB(cudaMemcpyAsync(cbounds, init, sizeof init, cudaMemcpyHostToDevice, 0));
-    prim_setup<<<gn, B>>>(d_sph, n_sph, d_quads, n_quad, pb, cbounds);
+    long long *sbounds;
+    LB(tmp_alloc(owned, &sbounds, 6));
+    const long long sinit[6] = {0x7fffffffffffffffll, 0x7fffffffffffffffll, 0x7fffffffffffffffll,
+                                (long long)0x8000000000000000ull, (long long)0x8000000000000000ull, (long long)0x8000000000000000ull};
+    LB(cudaMemcpyAsync(sbounds, sinit, sizeof sinit, cudaMemcpyHostToDevice, 0));
+    prim_setup<<<gn, B>>>(d_sph, n_sph, d_quads, n_quad, pb, sbounds);
     unsigned long long *keys, *keys_alt;
     uint32_t *vals, *vals_alt;
     LB(tmp_alloc(owned, &keys, n)); LB(tmp_alloc(owned, &keys_alt, n));
     LB(tmp_alloc(owned, &vals, n)); LB(tmp_alloc(owned, &vals_alt, n));
-    morton_codes<<<gn, B>>>(pb, n, cbounds, keys, vals);
+    // the scene-spanning primitives: one pass for the keys, then one pass per pick (largest key first)
+    Hoisted H{};
+    const uint32_t keep = std::min(std::min(max_hoisted, kMaxHoisted), n - 1);
+    if (keep) {
+        unsigned long long *picked, host_picked[kMaxHoisted];
+        LB(tmp_alloc(owned, &picked, kMaxHoisted));
+        LB(cudaMemsetAsync(picked, 0, kMaxHoisted * sizeof(unsigned long long), 0));
+        spanning_keys<<<gn, B>>>(d_sph, n_sph, d_quads, n, sbounds, keys);
+        for (uint32_t r = 0; r < keep; ++r) pick_spanning<<<gn, B>>>(keys, n, picked, (int)r);
+        LB(cudaMemcpyAsync(host_picked, picked, sizeof host_picked, cudaMemcpyDeviceToHost, 0));
+        LB(cudaStreamSynchronize(0));
+        for (uint32_t r = 0; r < keep && host_picked[r]; ++r) H.prim[H.n++] = 0xFFFFFFFFu - (uint32_t)host_picked[r];
+    }
+    const uint32_t n_tree = n - H.n;
+    if (n_tree < 2) { cleanup(); return cudaSuccess; }
+    int *cbounds;
+    LB(tmp_alloc(owned, &cbounds, 6));
+    const int init[6] = {0x7fffffff, 0x7fffffff, 0x7fffffff, (int)0x80000000, (int)0x80000000, (int)0x80000000};
+    LB(cudaMemcpyAsync(cbounds, init, sizeof init, cudaMemcpyHostToDevice, 0));
+    centroid_bounds<<<gn, B>>>(pb, n, H, cbounds);
+    morton_codes<<<gn, B>>>(pb, n, cbounds, H, keys, vals);
     {
         cub::DoubleBuffer<unsigned long long> dk(keys, keys_alt);
         cub::DoubleBuffer<uint32_t> dv(vals, vals_alt);
+        const int end_bit = H.n ? 64 : 63;
         size_t tmp_bytes = 0;
-        LB(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, dk, dv, (int)n, 0, 63));
+        LB(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, dk, dv, (int)n, 0, end_bit));
         char *tmp;
         LB(tmp_alloc(owned, &tmp, tmp_bytes));
-        LB(cub::DeviceRadixSort::SortPairs(tmp, tmp_bytes, dk, dv, (int)n, 0, 63));
+        LB(cub::DeviceRadixSort::SortPairs(tmp, tmp_bytes, dk, dv, (int)n, 0, end_bit));
         keys = dk.Current();
         vals = dv.Current();
     }
@@ -336,8 +430,8 @@ cudaError_t build_lbvh_device(const B200rtSphere *d_sph, uint32_t n_sph, const B
     LB(tmp_alloc(owned, &T.hix, n)); LB(tmp_alloc(owned, &T.hiy, n)); LB(tmp_alloc(owned, &T.hiz, n));
     LB(tmp_alloc(owned, &T.visits, n));
     LB(cudaMemsetAsync(T.visits, 0, n * sizeof(int), 0));
-    radix_tree<<<gn, B>>>(keys, (int)n, T);
-    fit_boxes<<<gn, B>>>(pb, vals, (int)n, T);
+    radix_tree<<<gn, B>>>(keys, (int)n_tree, T);
+    fit_boxes<<<gn, B>>>(pb, vals, (int)n_tree, T);
     // typed (per primitive kind) positions in leaf order
     uint32_t *flags, *quad_rank;
     LB(tmp_alloc(owned, &flags, n)); LB(tmp_alloc(owned, &quad_rank, n));
@@ -349,7 +443,9 @@ cudaError_t build_lbvh_device(const B200rtSphere *d_sph, uint32_t n_sph, const B
         LB(tmp_alloc(owned, &tmp, tmp_bytes));
         LB(cub::DeviceScan::ExclusiveSum(tmp, tmp_bytes, flags, quad_rank, (int)n));
     }
-    leaf_order<<<gn, B>>>(vals, quad_rank, n, n_sph, sphere_order, quad_order);
+    uint32_t *hoisted_ref;
+    LB(tmp_alloc(owned, &hoisted_ref, kMaxHoisted));
+    leaf_order<<<gn, B>>>(vals, quad_rank, n, n_tree, n_sph, sphere_order, quad_order, hoisted_ref);
     // breadth-first collapse to 4-wide nodes (at most n - 1 of them)
     LB(dev_alloc_async(&nodes4, (size_t)(n - 1) * sizeof(Node4), 0));
     CollapseTask *qa, *qb;
@@ -370,12 +466,14 @@ cudaError_t build_lbvh_device(const B200rtSphere *d_sph, uint32_t n_sph, const B
     }
     uint32_t n_nodes = 0;
     LB(cudaMemcpyAsync(&n_nodes, counters + 1, sizeof(uint32_t), cudaMemcpyDeviceToHost, 0));
+    LB(cudaMemcpyAsync(hoisted_ref_out, hoisted_ref, H.n * sizeof(uint32_t), cudaMemcpyDeviceToHost, 0));
     LB(cudaStreamSynchronize(0));
     LB(cudaGetLastError());
     cleanup();
     *nodes_out = reinterpret_cast<float4 *>(nodes4);
     *n_nodes_out = n_nodes;
     *depth_out = depth;
+    *n_hoisted_out = H.n;
     return cudaSuccess;
 #undef LB
 }

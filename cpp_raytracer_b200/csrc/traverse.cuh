@@ -47,6 +47,10 @@ struct DeviceScene {
     const double2 *quads;       // 8 x double2 per quad, leaf order: n^[3] V[3] w[3] s1[3] s2[3] pad
     const uint2 *quad_meta;
     const DeviceMaterial *materials;
+    // The scene-spanning primitives the tree leaves out (bvh_builder.h spanning_key), tested by every ray before the tree:
+    // references as in a leaf (kQuadFlagD | quad position, or sphere position), after the tree's in the leaf order.
+    uint32_t n_hoisted;
+    uint32_t hoisted_ref[4];
 #ifdef B200RT_DEBUG_BOUNDS
     DebugBounds dbg;
 #endif
@@ -331,37 +335,57 @@ __device__ __forceinline__ void trav_node_step(const DeviceScene &S, Trav &T, ui
 #undef B200RT_CHILD
 }
 
+// One primitive test in the reference's arithmetic (`ref` as in a leaf): a strictly closer hit becomes T.best, and an
+// exact tie goes to the lower canonical index (scene.h:59-75).
+__device__ __forceinline__ void trav_prim(const DeviceScene &S, Trav &T, uint32_t ref) {
+    double t;
+    bool hit;
+    const uint32_t i = ref & ~kQuadFlagD;
+    if (ref & kQuadFlagD) {
+        hit = quad_root(T.ray.ox, T.ray.oy, T.ray.oz, T.ray.dx, T.ray.dy, T.ray.dz, S.quads + (size_t)i * 8, T.tmin, T.best.t,
+                        T.best.ref != kNoHit, t);
+    } else {
+        const double2 s0 = __ldg(S.spheres + (size_t)i * 2);
+        const double2 s1 = __ldg(S.spheres + (size_t)i * 2 + 1);
+        hit = sphere_root(T.ray.ox, T.ray.oy, T.ray.oz, T.ray.dx, T.ray.dy, T.ray.dz, T.a, s0.x, s0.y, s1.x, s1.y, T.tmin, T.best.t,
+                          T.best.ref != kNoHit, t);
+    }
+    if (hit && (t < T.best.t || canonical_prim(S, ref) < canonical_prim(S, T.best.ref))) {
+        T.best.t = t;
+        T.best.ref = ref;
+        T.tmax32 = __double2float_ru(t);
+    }
+}
+
 // One leaf: FP64 primitive tests in the reference's arithmetic, then pop.
 __device__ __forceinline__ uint32_t trav_leaf_step(const DeviceScene &S, Trav &T, const uint2 *stack) {
     const uint32_t cnt = (T.cur >> 26) & 0xFu, first = T.cur & 0x03FFFFFFu;
-    const bool is_quad = T.cur & kQuadFlagD;
+    const uint32_t type = T.cur & kQuadFlagD;
 #ifdef B200RT_DEBUG_BOUNDS
-    if (!B200RT_CHECK(S, first + cnt <= (is_quad ? S.dbg.n_quads : S.dbg.n_spheres), 2)) { trav_pop(T, stack); return 0; }
+    if (!B200RT_CHECK(S, first + cnt <= (type ? S.dbg.n_quads : S.dbg.n_spheres), 2)) { trav_pop(T, stack); return 0; }
 #endif
-    for (uint32_t i = 0; i < cnt; ++i) {
-        double t;
-        bool hit;
-        uint32_t ref;
-        if (is_quad) {
-            ref = kQuadFlagD | (first + i);
-            hit = quad_root(T.ray.ox, T.ray.oy, T.ray.oz, T.ray.dx, T.ray.dy, T.ray.dz, S.quads + (size_t)(first + i) * 8, T.tmin, T.best.t,
-                            T.best.ref != kNoHit, t);
-        } else {
-            ref = first + i;
-            const double2 s0 = __ldg(S.spheres + (size_t)(first + i) * 2);
-            const double2 s1 = __ldg(S.spheres + (size_t)(first + i) * 2 + 1);
-            hit = sphere_root(T.ray.ox, T.ray.oy, T.ray.oz, T.ray.dx, T.ray.dy, T.ray.dz, T.a, s0.x, s0.y, s1.x, s1.y, T.tmin, T.best.t,
-                              T.best.ref != kNoHit, t);
-        }
-        // strictly closer wins; an exact tie goes to the lower canonical index (scene.h:59-75)
-        if (hit && (t < T.best.t || canonical_prim(S, ref) < canonical_prim(S, T.best.ref))) {
-            T.best.t = t;
-            T.best.ref = ref;
-            T.tmax32 = __double2float_ru(t);
-        }
-    }
+    for (uint32_t i = 0; i < cnt; ++i) trav_prim(S, T, type | (first + i));
     trav_pop(T, stack);
     return cnt;
+}
+
+// The scene-spanning primitives (DeviceScene::hoisted_ref), tested right after trav_setup / trav_init and before the
+// tree.  The count is the same for every lane, so the warp runs these tests converged -- a ground the rays would
+// otherwise reach in a leaf at a different iteration each tests with all of them -- and the tree traversal then starts
+// with tmax already at the ground hit, which culls the subtrees behind it from the first node on.  The closest hit does
+// not depend on the order of the tests: each test's answer is the primitive's first root above tmin whatever tmax was,
+// and exact ties go to the lower canonical index, so the result is the bits a leaf test gives.  With COUNT these
+// tests are counted as primitive tests.
+template <bool COUNT>
+__device__ __forceinline__ void trav_hoisted(const DeviceScene &S, Trav &T, TraversalCounters *ctr) {
+    for (uint32_t k = 0; k < S.n_hoisted; ++k) {
+        const uint32_t ref = S.hoisted_ref[k];
+#ifdef B200RT_DEBUG_BOUNDS
+        if (!B200RT_CHECK(S, (ref & kQuadFlagD) ? (ref & ~kQuadFlagD) < S.dbg.n_quads : ref < S.dbg.n_spheres, 2)) continue;
+#endif
+        trav_prim(S, T, ref);
+        if (COUNT) { ctr->prims++; if (ref & kQuadFlagD) ctr->quads++; }
+    }
 }
 
 // The traversal loop.  Every iteration offers a lane BOTH kinds of step, one after the other: with NODE-then-LEAF order
@@ -399,6 +423,7 @@ __device__ __forceinline__ Hit closest_hit(const DeviceScene &S, double ox, doub
     Trav T;
     uint2 stack[STACK];
     trav_init(T, ox, oy, oz, dx, dy, dz, tmin, tmax);
+    trav_hoisted<COUNT>(S, T, ctr);
     while (!trav_done(T)) trav_iteration<COUNT, LEAF_FIRST>(S, T, stack, ctr);
     return T.best;
 }

@@ -128,6 +128,7 @@ __global__ void __launch_bounds__(kPathBlock, kPathMinBlocks) wf_trace(const __g
                         Ray r;
                         slot_load_ray(s, r);
                         trav_init(T, r.ox, r.oy, r.oz, r.dx, r.dy, r.dz, kRayTmin, kRayTmax);
+                        trav_hoisted<COUNT>(P.scene, T, &ctr);
                         have = true;
                     }
                 }

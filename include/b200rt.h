@@ -107,6 +107,7 @@ typedef struct B200rtSceneInfo {
     uint32_t tree_depth;          /* depth of the 4-wide tree */
     uint32_t stack_entries;       /* traversal stack entries the kernels are instantiated with */
     double build_ms, upload_ms;
+    uint32_t n_hoisted;           /* scene-spanning primitives tested by every ray before the tree instead of in it */
 } B200rtSceneInfo;
 
 enum {
